@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- throughput of the ABC-Net hot path (batched U-Net forward + heat-map decode) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch 256]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch 256] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): v2 ABC-Net U-Net, 256 synthetic binary 1x512x512 images per GPU per step,
 bf16 activations / fp32 accumulation, followed by the fused peak-decode kernel. One "step" = one batch.
@@ -32,6 +32,10 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 HEADS = [1, 14, 3, 2, 1, 360, 60, 60]
+HEAD_NAMES = ("atom_target", "atom_type", "atom_charge", "atom_hs", "bond_target", "bond_type", "bond_rho", "bond_omega_type")
+# (image, y, x) positions whose logits --dump-outputs writes: 8192 x 501 channels x 4 B = 16 MB; with the records at the default
+# batch and capacities filled to the brim (256 x (1024 + 4096) x 24 B = 31 MB) the dump stays under 64 MB
+DUMP_PIXELS = 8192
 METRIC = "images_per_sec_unet_fwd_decode"
 UNIT = "images/s"
 FLOPS_PER_IMAGE = 93.98e9          # SURVEY.md section 6 (forward, v2 heads, 512x512)
@@ -233,22 +237,14 @@ def run_reference(args, rank, world):
     n = 8                                        # BASELINE.json configs[0]: batch of 8 images = one bounded sample of the 256-image step
     torch.set_num_threads(os.cpu_count() or 1)
     imgs = make_images(100, n)
-    # --steps / --warmup are honoured as given (about 1 s per 8-image step on 16 cores); only a wall-clock guard of ~4 minutes
-    # can end the run early, and the line then says how many steps were timed
-    t_guard = time.perf_counter()
-    warm = 0
-    for _ in range(max(args.warmup, 0)):
+    # --steps / --warmup are honoured as given (about 1 s per 8-image step on 16 cores)
+    warm = max(args.warmup, 0)
+    for _ in range(warm):
         cpu_path(sd, imgs, calib)
-        warm += 1
-        if time.perf_counter() - t_guard > 60:
-            break
+    steps = args.steps
     t0 = time.perf_counter()
-    steps = 0
-    for _ in range(max(args.steps, 1)):
+    for _ in range(steps):
         cpu_path(sd, imgs, calib)
-        steps += 1
-        if time.perf_counter() - t0 > 180:
-            break
     dt = time.perf_counter() - t0
     v = n * steps / dt
     cores = torch.get_num_threads()
@@ -492,6 +488,36 @@ def run_comparator(args, dev, pool, B):
 
 
 # ----------------------------------------------------------------------------------------- GPU arm
+def dump_outputs(out_dir, outs, recs):
+    """Write what one inference step hands its caller, as float32 .npy files (exact for every field below), so that two builds
+    can be compared output for output on the same inputs:
+      atoms.npy   [n, 6]  image, x, y, type, charge, hs of every decoded atom peak, in decoder order
+      bonds.npy   [n, 6]  image, x, y, omega, type, rho of every decoded bond record, in decoder order
+      counts.npy  [B, 3]  atom peaks, bond records and bond-centre peaks per image
+      logit_positions.npy [DUMP_PIXELS, 3]  (image, y, x), drawn with a fixed seed (the dense maps are 8.4 GB at batch 256)
+      logits_<head>.npy [DUMP_PIXELS, channels]  logits of every channel of the head at those positions"""
+    os.makedirs(out_dir, exist_ok=True)
+
+    def save(name, arr):
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+    img_a = np.concatenate([np.full(len(ra), i) for i, (ra, _, _) in enumerate(recs)])
+    img_b = np.concatenate([np.full(len(rb), i) for i, (_, rb, _) in enumerate(recs)])
+    a = np.concatenate([ra for ra, _, _ in recs])
+    b = np.concatenate([rb for _, rb, _ in recs])
+    save("atoms", np.stack([img_a, a["x"], a["y"], a["type"], a["charge"], a["hs"]], -1).astype(np.float32))
+    save("bonds", np.stack([img_b, b["x"], b["y"], b["omega"], b["type"], b["rho"]], -1).astype(np.float32))
+    save("counts", np.array([(len(ra), len(rb), nbp) for ra, rb, nbp in recs], np.float32).reshape(-1, 3))
+    B, H, W = outs[0].shape[0], outs[0].shape[2], outs[0].shape[3]
+    rng = np.random.default_rng(0)
+    pos = np.stack([rng.integers(0, n, DUMP_PIXELS) for n in (B, H, W)], -1)
+    save("logit_positions", pos.astype(np.float32))
+    n, y, x = (torch.from_numpy(pos[:, k:k + 1]).to(outs[0].device) for k in range(3))
+    for name, t, h in zip(HEAD_NAMES, outs, HEADS):
+        c = torch.arange(h, device=t.device)[None]
+        v = t[n, c // 8, y, x, c % 8] if t.dim() == 5 else t[n, c, y, x]           # planar-8 [B, ceil(h/8), H, W, 8] or NCHW
+        save("logits_" + name, v.float().cpu().numpy())
+
+
 def run_ours(args, rank, world, local_rank):
     import torch.distributed as dist
 
@@ -567,6 +593,8 @@ def run_ours(args, rank, world, local_rank):
     clocks = sampler.stop(t_host0, time.time())
     ms = e0.elapsed_time(e1)
     timing, model.timing = model.timing, None
+    if args.dump_outputs and rank == 0:                  # the last timed step's logits and records, before other legs reuse the buffers
+        dump_outputs(args.dump_outputs, out_bufs, dec.fetch(B))
     # ---- timed: end to end through the public API with HOST buffers. Every step copies its own images host -> device
     # (pinned memory, side stream, double-buffered so that the copy of step i+1 overlaps the kernels of step i) and reads
     # the decoded records back (one D2H + stream sync per step).
@@ -834,7 +862,11 @@ def _reserve_stdout():
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of every headline leg (device-resident, e2e, MOL-block, sparse heads, fp16, graph replay, "
+                         "training step, reference arm); the side measurements cpu_baseline (2 x 8 images), small_batch (50 "
+                         "iterations per size), gpu_comparator (3 iterations) and, with several GPUs, the all-reduce alone "
+                         "(20 repetitions) keep fixed counts")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=256)
@@ -846,7 +878,14 @@ def main():
     ap.add_argument("--no-comparator", action="store_true", help="skip the torch / cuDNN comparator leg ('gpu_comparator')")
     ap.add_argument("--train-batch", type=int, default=64, help="images per GPU per training step (train.py:44; multi_gpu_train2.py:20 uses 60)")
     ap.add_argument("--train-only", action="store_true", help="only the training-step leg: prints its object as the JSON line")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last step's decoded records and a fixed "
+                    "sample of its logits to DIR/<name>.npy (rank 0's images). Inference path only: the reference arm decodes a "
+                    "different 8-image sample with its own calibration, so its records are not comparable with these")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.train_only):
+        ap.error("--dump-outputs writes the outputs of the inference path (--impl ours without --train-only)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -56,6 +56,28 @@ def sample_positions(seed, n, H, W):
     return r[:, 0] % H, r[:, 1] % W
 
 
+UNET_SAMPLE_PIXELS = 32             # pixels per output set kept in unet_small.npz / unet_rgb.npz: the files stay far below 1 MB
+
+
+def pixel_sample(seed, B, H, W, n=UNET_SAMPLE_PIXELS):
+    """n distinct (image, y, x) positions of a [B, *, H, W] output, sorted, as int64 [n, 3]."""
+    r = np.sort(np.random.default_rng(seed).choice(B * H * W, n, replace=False))
+    return np.stack(np.unravel_index(r, (B, H, W)), -1).astype(np.int64)
+
+
+def reduce_logits(key, ys, pos):
+    """What the golden keeps of the 8 head outputs ys [B, C, H, W]: every channel at the pixels pos ({key}{i}, [n, C]) and
+    the float64 sum and absolute sum of the whole map ({key}_sum{i}, {key}_abssum{i})."""
+    out = {}
+    for i, y in enumerate(ys):
+        y = np.asarray(y)
+        y64 = y.astype(np.float64)
+        out[f"{key}{i}"] = y[pos[:, 0], :, pos[:, 1], pos[:, 2]]
+        out[f"{key}_sum{i}"] = np.array(y64.sum())
+        out[f"{key}_abssum{i}"] = np.array(np.abs(y64).sum())
+    return out
+
+
 # ----------------------------------------------------------------------------- U-Net
 def golden_unet():
     UNet = import_ref_unet()
@@ -67,18 +89,17 @@ def golden_unet():
         m.load_state_dict(sd)
         m.eval()
         x = torch.from_numpy(synth.binary_images(seed, B, H, W, 0.08))
+        pos = out[f"{tag}_pos"] = pixel_sample(seed, B, H // 4, W // 4)
         with torch.no_grad():
             ys = m(x)
-        for i, y in enumerate(ys):
-            out[f"{tag}_out{i}"] = y.numpy()
+        out.update(reduce_logits(f"{tag}_out", ys, pos))
         # train-mode forward (BN batch statistics; dropout disabled by p=0 so it is deterministic)
         m.train()
         for om in m.out_modules:
             om.drop.p = 0.0
         with torch.no_grad():
             ys = m(x)
-        for i, y in enumerate(ys):
-            out[f"{tag}_train_out{i}"] = y.numpy()
+        out.update(reduce_logits(f"{tag}_train_out", ys, pos))
     np.savez_compressed(os.path.join(HERE, "unet_small.npz"), **out)
 
     # full resolution: samples + checksums only (dense output is 32.8 MB / image)
@@ -111,16 +132,15 @@ def golden_unet_rgb():
     m.load_state_dict(sd)
     x = torch.from_numpy(detrand.uniform(77, (B, 3, H, W), 0.0, 1.0).astype(np.float32))       # torch.rand-like
     out = {}
+    pos = out["pos"] = pixel_sample(seed, B, H // 4, W // 4)
     m.eval()
     with torch.no_grad():
-        for i, y in enumerate(m(x)):
-            out[f"out{i}"] = y.numpy()
+        out.update(reduce_logits("out", m(x), pos))
     m.train()
     for om in m.out_modules:
         om.drop.p = 0.0
     with torch.no_grad():
-        for i, y in enumerate(m(x)):
-            out[f"train_out{i}"] = y.numpy()
+        out.update(reduce_logits("train_out", m(x), pos))
     np.savez_compressed(os.path.join(HERE, "unet_rgb.npz"), **out)
     print("3-channel unet golden written")
 

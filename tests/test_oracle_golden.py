@@ -18,6 +18,24 @@ def test_param_inventory():
     assert n == 10_698_575
 
 
+def at_pixels(y, pos):
+    """Every channel of the maps y [B, C, H, W] (numpy or torch) at the pixels pos [n, 3] = (image, y, x) -> [n, C]."""
+    return y[pos[:, 0], :, pos[:, 1], pos[:, 2]]
+
+
+def assert_matches_unet_golden(y, g, pos, key, i, tol):
+    """Head i of y against a U-Net golden (tests/golden/make_golden.py reduce_logits): allclose(rtol = atol = tol) on every
+    channel at the stored pixels pos, and on the sum and absolute sum of the whole map the bound that elementwise allclose
+    implies."""
+    y = y.numpy()
+    np.testing.assert_allclose(at_pixels(y, pos), g[f"{key}{i}"], rtol=tol, atol=tol)
+    abssum = float(g[f"{key}_abssum{i}"])
+    bound = tol * (y.size + abssum)
+    y64 = y.astype(np.float64)
+    assert abs(y64.sum() - float(g[f"{key}_sum{i}"])) <= bound, (key, i)
+    assert abs(np.abs(y64).sum() - abssum) <= bound, (key, i)
+
+
 @pytest.mark.parametrize("tag,B,H,W,seed", [("small", 2, 64, 96, 3), ("tiny", 2, 32, 32, 4)])
 def test_unet_oracle_matches_reference(golden_dir, tag, B, H, W, seed):
     g = np.load(os.path.join(golden_dir, "unet_small.npz"))
@@ -28,8 +46,8 @@ def test_unet_oracle_matches_reference(golden_dir, tag, B, H, W, seed):
         yt = unet_ref.forward(x, sd, training=True)
     for i, (y, t) in enumerate(zip(ys, yt)):
         # same ATen kernels as the reference module -> agreement to fp32 round-off
-        np.testing.assert_allclose(y.numpy(), g[f"{tag}_out{i}"], rtol=1e-5, atol=1e-5)
-        np.testing.assert_allclose(t.numpy(), g[f"{tag}_train_out{i}"], rtol=1e-4, atol=1e-4)
+        assert_matches_unet_golden(y, g, g[f"{tag}_pos"], f"{tag}_out", i, 1e-5)
+        assert_matches_unet_golden(t, g, g[f"{tag}_pos"], f"{tag}_train_out", i, 1e-4)
 
 
 def test_unet_oracle_matches_reference_three_channels(golden_dir):
@@ -43,8 +61,8 @@ def test_unet_oracle_matches_reference_three_channels(golden_dir):
         yt = unet_ref.forward(x, sd, training=True)
     assert [tuple(y.shape) for y in ys] == [(1, h, 24, 16) for h in unet_ref.V2_HEADS]
     for i, (y, t) in enumerate(zip(ys, yt)):
-        np.testing.assert_allclose(y.numpy(), g[f"out{i}"], rtol=1e-5, atol=1e-5)
-        np.testing.assert_allclose(t.numpy(), g[f"train_out{i}"], rtol=1e-4, atol=1e-4)
+        assert_matches_unet_golden(y, g, g["pos"], "out", i, 1e-5)
+        assert_matches_unet_golden(t, g, g["pos"], "train_out", i, 1e-4)
 
 
 def test_unet_crop_side_is_first_row_col():

@@ -8,6 +8,7 @@ import pytest
 import torch
 
 from oracle import assemble_ref, decode_ref, detrand, loss_ref, synth, unet_ref
+from test_oracle_golden import at_pixels
 
 pytestmark = pytest.mark.gpu
 
@@ -48,7 +49,8 @@ def test_unet_forward_vs_golden(golden_dir, tag, B, H, W, seed):
     x = torch.from_numpy(synth.binary_images(seed, B, H, W, 0.08)).cuda()
     outs = m(x)
     assert isinstance(outs, list) and len(outs) == 8
-    _check_logits(outs, [g[f"{tag}_out{i}"] for i in range(8)], f"golden[{tag}]")
+    pos = g[f"{tag}_pos"]                   # the golden keeps every channel at these pixels
+    _check_logits([at_pixels(o, pos) for o in outs], [g[f"{tag}_out{i}"] for i in range(8)], f"golden[{tag}]")
 
 
 def test_unet_layer_by_layer_vs_oracle():
