@@ -10,6 +10,7 @@
 #include <cstdlib>
 #include <cuda_bf16.h>
 
+#include "bn_launch.cuh"
 #include "common.cuh"
 #include "p8_device.cuh"
 
@@ -48,35 +49,43 @@ __device__ __forceinline__ void load8f(const float* __restrict__ src, float* dst
   dst[0] = a.x; dst[1] = a.y; dst[2] = a.z; dst[3] = a.w; dst[4] = b.x; dst[5] = b.y; dst[6] = b.z; dst[7] = b.w;
 }
 
+// Block-wide sums of K per-thread fp32 partials v(0) .. v(K-1): a warp shuffle tree in fp32, then the 8 warp totals in fp64
+// in warp order. Thread i < K returns the block total of partial i. Every thread of the block calls it.
+template <int K, typename F>
+__device__ __forceinline__ double block_sum(F v, double (*red)[8]) {
+  static_assert(kBnThreads == 8 * 32, "one red[][] slot per warp");
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int i = 0; i < K; ++i) {
+    float x = v(i);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
+    if (lane == 0) red[i][warp] = static_cast<double>(x);
+  }
+  __syncthreads();
+  double t = 0.0;
+  if (threadIdx.x < K)
+#pragma unroll
+    for (int w = 0; w < 8; ++w) t += red[threadIdx.x][w];
+  return t;
+}
+
 // block-wide sum of 16 per-thread fp32 partials (8 channels x 2 statistics) -> fp64 atomics
 __device__ __forceinline__ void block_reduce16(const float* a, const float* b, double* __restrict__ ga, double* __restrict__ gb,
                                                int c0, double (*red)[8]) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-  for (int i = 0; i < 16; ++i) {
-    float v = i < 8 ? a[i] : b[i - 8];
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    if (lane == 0) red[i][warp] = static_cast<double>(v);
-  }
-  __syncthreads();
-  if (threadIdx.x < 16) {
-    double v = 0.0;
-#pragma unroll
-    for (int w = 0; w < 8; ++w) v += red[threadIdx.x][w];
-    atomicAdd((threadIdx.x < 8 ? ga : gb) + c0 + (threadIdx.x & 7), v);
-  }
+  const double t = block_sum<16>([&](int i) { return i < 8 ? a[i] : b[i - 8]; }, red);
+  if (threadIdx.x < 16) atomicAdd((threadIdx.x < 8 ? ga : gb) + c0 + (threadIdx.x & 7), t);
 }
 
 // ------------------------------------------------------------------------------------------- statistics
-__global__ void __launch_bounds__(256) bn_stats_kernel(P8View z, int HW, double* __restrict__ sum, double* __restrict__ sumsq) {
+__global__ void __launch_bounds__(kBnThreads) bn_stats_kernel(P8View z, int HW, double* __restrict__ sum, double* __restrict__ sumsq) {
   const int plane = blockIdx.y, n = blockIdx.z;
   const uint4* __restrict__ zb = z.ptr + (static_cast<size_t>(n) * z.planes + z.plane_off + plane) * HW;
   float s[8], q[8];
 #pragma unroll
   for (int i = 0; i < 8; ++i) s[i] = q[i] = 0.f;
-  const int stride = gridDim.x * 256;
-  int e = blockIdx.x * 256 + threadIdx.x;
+  const int stride = gridDim.x * kBnThreads;
+  int e = blockIdx.x * kBnThreads + threadIdx.x;
   for (; e + stride < HW; e += 2 * stride) {          // two independent 16-byte loads in flight per thread
     const uint4 u0 = zb[e], u1 = zb[e + stride];
     float v[8], w[8];
@@ -142,7 +151,7 @@ struct BnActParams {
 };
 
 template <bool POOL>
-__global__ void __launch_bounds__(256) bn_act_kernel(const BnActParams p) {
+__global__ void __launch_bounds__(kBnThreads) bn_act_kernel(const BnActParams p) {
   const int plane = blockIdx.y, n = blockIdx.z;
   const int HW = p.H * p.W;
   float sc[8], sh[8];
@@ -150,11 +159,11 @@ __global__ void __launch_bounds__(256) bn_act_kernel(const BnActParams p) {
   load8f(p.shift + plane * 8, sh);
   const uint4* __restrict__ zb = p.z.ptr + (static_cast<size_t>(n) * p.z.planes + p.z.plane_off + plane) * HW;
   uint4* __restrict__ ob = p.out ? p.out + (static_cast<size_t>(n) * p.out_planes + p.out_plane_off + plane) * HW : nullptr;
-  const int stride = gridDim.x * 256;
+  const int stride = gridDim.x * kBnThreads;
   if (!POOL) {
     const unsigned long long seed = p.seed + (p.seed_dev ? *p.seed_dev : 0ull);
     const unsigned long long vbase = (static_cast<unsigned long long>(n) * p.planes + plane) * HW;   // index of the plane's first vector
-    for (int e = blockIdx.x * 256 + threadIdx.x; e < HW; e += stride) {
+    for (int e = blockIdx.x * kBnThreads + threadIdx.x; e < HW; e += stride) {
       float v[8], dm[8];
       unpack8u(zb[e], v);
       if (p.drop_p > 0.f) {
@@ -177,7 +186,7 @@ __global__ void __launch_bounds__(256) bn_act_kernel(const BnActParams p) {
   } else {
     const int bw = p.W >> 1, hw2 = (p.H >> 1) * bw;
     uint4* __restrict__ pb = p.pool + (static_cast<size_t>(n) * p.pool_planes + p.pool_plane_off + plane) * hw2;
-    for (int b = blockIdx.x * 256 + threadIdx.x; b < hw2; b += stride) {
+    for (int b = blockIdx.x * kBnThreads + threadIdx.x; b < hw2; b += stride) {
       const int by = b / bw, bx = b - by * bw;
       const int i00 = 2 * by * p.W + 2 * bx;
       const uint4 u[4] = {zb[i00], zb[i00 + 1], zb[i00 + p.W], zb[i00 + p.W + 1]};
@@ -271,7 +280,7 @@ __device__ __forceinline__ void bwd_block4(const BnActBwdParams& p, const float 
 
 // reduce: s1 = sum g, s2 = sum g * xhat (xhat = (z - mean) * invstd, accumulated as sum g*z and combined per block)
 template <bool POOL, int MINB = 2>
-__global__ void __launch_bounds__(256, MINB) bn_act_bwd_reduce_kernel(const BnActBwdParams p) {
+__global__ void __launch_bounds__(kBnThreads, MINB) bn_act_bwd_reduce_kernel(const BnActBwdParams p) {
   const int plane = blockIdx.y, n = blockIdx.z;
   const int HW = p.H * p.W;
   float sc[8], sh[8];
@@ -282,12 +291,12 @@ __global__ void __launch_bounds__(256, MINB) bn_act_bwd_reduce_kernel(const BnAc
   float s1[8], t2[8];
 #pragma unroll
   for (int i = 0; i < 8; ++i) s1[i] = t2[i] = 0.f;
-  const int stride = gridDim.x * 256;
+  const int stride = gridDim.x * kBnThreads;
   if (!POOL) {
     const unsigned long long seed = p.seed + (p.seed_dev ? *p.seed_dev : 0ull);
     const unsigned long long vbase = (static_cast<unsigned long long>(n) * p.planes + plane) * HW;
     const unsigned char* __restrict__ mk = (p.drop_p > 0.f && p.drop_mask != nullptr) ? p.drop_mask + vbase : nullptr;
-    int e = blockIdx.x * 256 + threadIdx.x;
+    int e = blockIdx.x * kBnThreads + threadIdx.x;
     for (; e + stride < HW; e += 2 * stride) {            // four independent 16-byte loads in flight per thread
       const uint4 zu0 = zb[e], du0 = db[e], zu1 = zb[e + stride], du1 = db[e + stride];
       const int m0 = mk ? mk[e] : -1, m1 = mk ? mk[e + stride] : -1;
@@ -320,7 +329,7 @@ __global__ void __launch_bounds__(256, MINB) bn_act_bwd_reduce_kernel(const BnAc
   } else {
     const int bw = p.W >> 1, hw2 = (p.H >> 1) * bw;
     const uint4* __restrict__ pb = p.dP.ptr + (static_cast<size_t>(n) * p.dP.planes + p.dP.plane_off + plane) * hw2;
-    for (int b = blockIdx.x * 256 + threadIdx.x; b < hw2; b += stride) {
+    for (int b = blockIdx.x * kBnThreads + threadIdx.x; b < hw2; b += stride) {
       const int by = b / bw, bx = b - by * bw;
       const int i00 = 2 * by * p.W + 2 * bx;
       float v[4][8], d[4][8], g[4][8], dp[8];
@@ -367,7 +376,7 @@ __global__ void __launch_bounds__(256, MINB) bn_act_bwd_reduce_kernel(const BnAc
 
 // apply: dz = scale * (g - s1/M - xhat * s2/M) = scale * g + cb * z + ca  with per-channel constants ca, cb
 template <bool POOL, int MINB = 2>
-__global__ void __launch_bounds__(256, MINB) bn_act_bwd_apply_kernel(const BnActBwdParams p) {
+__global__ void __launch_bounds__(kBnThreads, MINB) bn_act_bwd_apply_kernel(const BnActBwdParams p) {
   const int plane = blockIdx.y, n = blockIdx.z;
   const int HW = p.H * p.W;
   __shared__ float cst[2][8];
@@ -397,12 +406,12 @@ __global__ void __launch_bounds__(256, MINB) bn_act_bwd_apply_kernel(const BnAct
   const uint4* __restrict__ zb = p.z.ptr + (static_cast<size_t>(n) * p.z.planes + p.z.plane_off + plane) * HW;
   const uint4* __restrict__ db = p.dA.ptr ? p.dA.ptr + (static_cast<size_t>(n) * p.dA.planes + p.dA.plane_off + plane) * HW : nullptr;
   uint4* __restrict__ ob = p.dz + (static_cast<size_t>(n) * p.dz_planes + p.dz_plane_off + plane) * HW;
-  const int stride = gridDim.x * 256;
+  const int stride = gridDim.x * kBnThreads;
   if (!POOL) {
     const unsigned long long seed = p.seed + (p.seed_dev ? *p.seed_dev : 0ull);
     const unsigned long long vbase = (static_cast<unsigned long long>(n) * p.planes + plane) * HW;
     const unsigned char* __restrict__ mk = (p.drop_p > 0.f && p.drop_mask != nullptr) ? p.drop_mask + vbase : nullptr;
-    int e = blockIdx.x * 256 + threadIdx.x;
+    int e = blockIdx.x * kBnThreads + threadIdx.x;
     for (; e + stride < HW; e += 2 * stride) {            // four independent 16-byte loads in flight per thread
       const uint4 zu0 = zb[e], du0 = db[e], zu1 = zb[e + stride], du1 = db[e + stride];
       const int m0 = mk ? mk[e] : -1, m1 = mk ? mk[e + stride] : -1;
@@ -435,7 +444,7 @@ __global__ void __launch_bounds__(256, MINB) bn_act_bwd_apply_kernel(const BnAct
   } else {
     const int bw = p.W >> 1, hw2 = (p.H >> 1) * bw;
     const uint4* __restrict__ pb = p.dP.ptr + (static_cast<size_t>(n) * p.dP.planes + p.dP.plane_off + plane) * hw2;
-    for (int b = blockIdx.x * 256 + threadIdx.x; b < hw2; b += stride) {
+    for (int b = blockIdx.x * kBnThreads + threadIdx.x; b < hw2; b += stride) {
       const int by = b / bw, bx = b - by * bw;
       const int i00 = 2 * by * p.W + 2 * bx;
       float v[4][8], d[4][8], g[4][8], dp[8];
@@ -483,18 +492,18 @@ __global__ void __launch_bounds__(256) nchw_to_p8_kernel(const float* __restrict
 
 // fp32 NCHW -> bf16 P8 with an optional device-side scale, zero-filled padding planes and per-channel sums of the scaled
 // values (the bias gradient of the 1x1 head convolutions): one pass over the loss gradient instead of three.
-__global__ void __launch_bounds__(256) nchw_to_p8_ex_kernel(const float* __restrict__ src, uint4* __restrict__ dst, int C, int HW,
-                                                            int dst_planes, const float* __restrict__ scale,
-                                                            double* __restrict__ dbias) {
+__global__ void __launch_bounds__(kBnThreads) nchw_to_p8_ex_kernel(const float* __restrict__ src, uint4* __restrict__ dst, int C,
+                                                                   int HW, int dst_planes, const float* __restrict__ scale,
+                                                                   double* __restrict__ dbias) {
   const int plane = blockIdx.y, n = blockIdx.z;
   const float sc = scale ? *scale : 1.f;
   const float* __restrict__ sb = src + (static_cast<size_t>(n) * C + plane * 8) * HW;
   uint4* __restrict__ db = dst + (static_cast<size_t>(n) * dst_planes + plane) * HW;
   const int nvalid = min(8, max(0, C - plane * 8));
-  float s[8], zero[8];
+  float s[8];
 #pragma unroll
-  for (int i = 0; i < 8; ++i) s[i] = zero[i] = 0.f;
-  for (int e = blockIdx.x * 256 + threadIdx.x; e < HW; e += gridDim.x * 256) {
+  for (int i = 0; i < 8; ++i) s[i] = 0.f;
+  for (int e = blockIdx.x * kBnThreads + threadIdx.x; e < HW; e += gridDim.x * kBnThreads) {
     float v[8];
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
@@ -504,22 +513,9 @@ __global__ void __launch_bounds__(256) nchw_to_p8_ex_kernel(const float* __restr
     db[e] = pack8(v);
   }
   if (dbias != nullptr && nvalid > 0) {      // block-uniform condition
-    __shared__ double red[16][8];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-      float v = s[i];
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-      if (lane == 0) red[i][warp] = static_cast<double>(v);
-    }
-    __syncthreads();
-    if (threadIdx.x < nvalid) {
-      double v = 0.0;
-#pragma unroll
-      for (int w = 0; w < 8; ++w) v += red[threadIdx.x][w];
-      atomicAdd(dbias + plane * 8 + threadIdx.x, v);
-    }
+    __shared__ double red[8][8];
+    const double t = block_sum<8>([&](int i) { return s[i]; }, red);
+    if (threadIdx.x < nvalid) atomicAdd(dbias + plane * 8 + threadIdx.x, t);
   }
 }
 
@@ -651,17 +647,6 @@ static int p8_check(const void* ptr, int planes, int plane_off, int cplanes, con
   return ABC_OK;
 }
 
-// grid.x for the (pixels, plane, image) decomposition: enough blocks to fill the machine, few enough that every
-// thread streams several vectors and the per-block atomics stay negligible
-static int plane_grid_x(long long items, int planes, int N, int per_thread = 1) {
-  long long need = (items + 256ll * per_thread - 1) / (256ll * per_thread);
-  static const long long per_sm = [] { const char* e = getenv("ABCNET_BN_BLOCKS_PER_SM"); return e && atoi(e) > 0 ? atoi(e) : 12; }();
-  long long cap = (148ll * per_sm + static_cast<long long>(planes) * N - 1) / (static_cast<long long>(planes) * N);
-  if (cap < 1) cap = 1;
-  if (need > cap) need = cap;
-  return need < 1 ? 1 : static_cast<int>(need);
-}
-
 extern "C" int abc_bn_stats(const void* z, int N, int H, int W, int planes, int plane_off, int C, double* sum, double* sumsq,
                             void* stream) {
   if (int rc = device_check()) return rc;
@@ -672,7 +657,8 @@ extern "C" int abc_bn_stats(const void* z, int N, int H, int W, int planes, int 
   ABC_CUDA(cudaMemsetAsync(sum, 0, C * sizeof(double), st));
   ABC_CUDA(cudaMemsetAsync(sumsq, 0, C * sizeof(double), st));
   P8View v{static_cast<const uint4*>(z), planes, plane_off};
-  bn_stats_kernel<<<dim3(plane_grid_x(static_cast<long long>(H) * W, C / 8, N, 4), C / 8, N), 256, 0, st>>>(v, H * W, sum, sumsq);
+  const BnLaunch l = bn_launch_config(BnPass::kStats, N, C / 8, H, W);
+  bn_stats_kernel<<<l.grid, l.block, 0, st>>>(v, H * W, sum, sumsq);
   return launch_check("bn_stats_kernel");
 }
 
@@ -708,13 +694,9 @@ extern "C" int abc_bn_act(const AbcBnActDesc* d, void* stream) {
   p.seed_dev = reinterpret_cast<const unsigned long long*>(d->seed_dev);
   p.drop_mask = static_cast<unsigned char*>(d->drop_mask);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (d->pool) {
-    const long long items = static_cast<long long>(d->H / 2) * (d->W / 2);
-    bn_act_kernel<true><<<dim3(plane_grid_x(items, p.planes, d->N), p.planes, d->N), 256, 0, st>>>(p);
-  } else {
-    const long long items = static_cast<long long>(d->H) * d->W;
-    bn_act_kernel<false><<<dim3(plane_grid_x(items, p.planes, d->N, 2), p.planes, d->N), 256, 0, st>>>(p);
-  }
+  const BnLaunch l = bn_launch_config(d->pool ? BnPass::kPool : BnPass::kPixels, d->N, p.planes, d->H, d->W);
+  if (d->pool) bn_act_kernel<true><<<l.grid, l.block, 0, st>>>(p);
+  else bn_act_kernel<false><<<l.grid, l.block, 0, st>>>(p);
   return launch_check("bn_act_kernel");
 }
 
@@ -750,23 +732,20 @@ extern "C" int abc_bn_act_backward(const AbcBnActBwdDesc* d, void* stream) {
   ABC_REQUIRE((reinterpret_cast<uintptr_t>(d->gscale) & 15) == 0, "abc_bn_act_backward: gscale must be 16-byte aligned");
   ABC_CUDA(cudaMemsetAsync(d->s1, 0, d->C * sizeof(double), st));
   ABC_CUDA(cudaMemsetAsync(d->s2, 0, d->C * sizeof(double), st));
+  const BnLaunch l = bn_launch_config(d->dP ? BnPass::kPool : BnPass::kPixels, d->N, cp, d->H, d->W);
   if (d->dP) {
-    const long long items = static_cast<long long>(d->H / 2) * (d->W / 2);
-    const dim3 grid(plane_grid_x(items, cp, d->N), cp, d->N);
-    bn_act_bwd_reduce_kernel<true><<<grid, 256, 0, st>>>(p);
+    bn_act_bwd_reduce_kernel<true><<<l.grid, l.block, 0, st>>>(p);
     if (int rc = launch_check("bn_act_bwd_reduce_kernel")) return rc;
-    bn_act_bwd_apply_kernel<true><<<grid, 256, 0, st>>>(p);
+    bn_act_bwd_apply_kernel<true><<<l.grid, l.block, 0, st>>>(p);
   } else {
-    const long long items = static_cast<long long>(d->H) * d->W;
-    const dim3 grid(plane_grid_x(items, cp, d->N, 2), cp, d->N);
     // resident blocks per SM (register cap) of the two passes: ABCNET_BN_MINB = <reduce digit><apply digit>, read once
     static const int minb = [] { const char* e = getenv("ABCNET_BN_MINB"); return e ? atoi(e) : 34; }();
-    if (minb / 10 == 4) bn_act_bwd_reduce_kernel<false, 4><<<grid, 256, 0, st>>>(p);
-    else bn_act_bwd_reduce_kernel<false, 3><<<grid, 256, 0, st>>>(p);
+    if (minb / 10 == 4) bn_act_bwd_reduce_kernel<false, 4><<<l.grid, l.block, 0, st>>>(p);
+    else bn_act_bwd_reduce_kernel<false, 3><<<l.grid, l.block, 0, st>>>(p);
     if (int rc = launch_check("bn_act_bwd_reduce_kernel")) return rc;
-    if (minb % 10 == 4) bn_act_bwd_apply_kernel<false, 4><<<grid, 256, 0, st>>>(p);
-    else if (minb % 10 == 3) bn_act_bwd_apply_kernel<false, 3><<<grid, 256, 0, st>>>(p);
-    else bn_act_bwd_apply_kernel<false, 2><<<grid, 256, 0, st>>>(p);
+    if (minb % 10 == 4) bn_act_bwd_apply_kernel<false, 4><<<l.grid, l.block, 0, st>>>(p);
+    else if (minb % 10 == 3) bn_act_bwd_apply_kernel<false, 3><<<l.grid, l.block, 0, st>>>(p);
+    else bn_act_bwd_apply_kernel<false, 2><<<l.grid, l.block, 0, st>>>(p);
   }
   return launch_check("bn_act_bwd_apply_kernel");
 }
@@ -789,8 +768,8 @@ extern "C" int abc_nchw_to_p8_ex(const float* src, void* dst, int N, int C, int 
   ABC_REQUIRE((reinterpret_cast<uintptr_t>(dst) & 15) == 0, "abc_nchw_to_p8_ex: dst must be 16-byte aligned");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (dbias) ABC_CUDA(cudaMemsetAsync(dbias, 0, C * sizeof(double), st));
-  const dim3 grid(plane_grid_x(static_cast<long long>(H) * W, dst_planes, N, 2), dst_planes, N);
-  nchw_to_p8_ex_kernel<<<grid, 256, 0, st>>>(src, static_cast<uint4*>(dst), C, H * W, dst_planes, scale, dbias);
+  const BnLaunch l = bn_launch_config(BnPass::kPixels, N, dst_planes, H, W);
+  nchw_to_p8_ex_kernel<<<l.grid, l.block, 0, st>>>(src, static_cast<uint4*>(dst), C, H * W, dst_planes, scale, dbias);
   return launch_check("nchw_to_p8_ex_kernel");
 }
 
