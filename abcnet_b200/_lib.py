@@ -88,6 +88,7 @@ class AbcHeadsFusedDesc(C.Structure):
         ("w1pack", C.c_void_p), ("bias1", C.c_void_p), ("n_heads", C.c_int), ("cout", C.c_int * 16),
         ("w2pack", C.c_void_p), ("w2pack_bytes", C.c_int64), ("bias2", C.c_void_p), ("bias2_len", C.c_int),
         ("out", C.c_void_p * 16), ("out_mode", C.c_int * 16), ("out_planes", C.c_int * 16), ("item_slot", C.c_int * 6),
+        ("act_fp16", C.c_int),
     ]
 
 

@@ -1,21 +1,26 @@
 // Fused output heads for sm_100a: for every head of the U-Net, conv3x3(128 -> 128) + BatchNorm(eval, folded) +
 // LeakyReLU(0.01) + conv1x1(128 -> h) in ONE kernel -- OutConv of /root/reference/src/unet.py:63-74, applied to the shared
-// trunk at :116-118. The 128-channel hidden map of a head never leaves the SM:
+// trunk at :116-118. The 128-channel hidden map of a head never leaves tensor memory:
 //
 //   conv1 : implicit GEMM as in conv_igemm_sm100.cu (TMA halo tile, 9 shifted descriptors, tcgen05.mma M = 128 pixels,
-//           N = 256 = TWO heads per CTA column, K = 2 chunks x 9 taps x 64 channels), accumulators in TMEM;
-//   epilogue phase 1 : TMEM -> registers -> bias + LeakyReLU -> bf16 -> shared memory, written directly in the
-//           K-major core-matrix layout of a tcgen05 A operand (hidden[pixel][128 channels], 32 KB per head);
-//   conv2 : 8 more MMAs per chunk of <= 128 output channels (A = hidden from shared memory, B = the head's 1x1 weights
-//           streamed through the same weight ring), accumulating into the TMEM columns phase 1 has just drained;
+//           N = 256 = TWO heads per CTA, K = 2 chunks x 9 taps x 64 channels), accumulators in TMEM;
+//   epilogue phase 1 : TMEM -> registers -> bias + LeakyReLU -> 16-bit -> back to TMEM (tcgen05.st), two values per
+//           32-bit column, lane = pixel: the A-operand layout of tcgen05.mma kind::f16 with A in tensor memory;
+//   conv2 : 8 MMAs per chunk of <= 128 output channels (A = hidden map from TMEM, B = the head's 1x1 weights streamed
+//           through the conv1 weight ring), accumulating into the TMEM columns phase 1 has just drained;
 //   epilogue phase 2 : TMEM -> + bias -> fp32 logits (NCHW, or planar-8 for the fused inference + decode path).
+//
+// TMEM: two buffers of 256 columns (tile t uses buffer t & 1). In buffer b, conv1 accumulates head A in columns [0, 128) and
+// head B in [128, 256); phase 1 writes hidden A to [0, 64) and hidden B to [64, 128); the conv2 chunks then accumulate one
+// after another in [128, 256). The buffer returns to conv1 (tile t + 2) once its last chunk is drained.
 //
 // Compared with conv_igemm(conv1) + 8 x conv_igemm(conv2) this removes the write and re-read of the hidden maps
 // (2 x 8.6 GB per 256-image batch) and nine launches. The conv2 MMAs of tile t are issued by the MMA warp in the middle
 // of the conv1 MMAs of tile t + 1 (after a host-chosen "slot" of the 18 (chunk, tap) steps), so the tensor pipe never
-// waits for the epilogue.
+// waits for the epilogue. The hidden maps take no shared memory, so the weight ring is as deep as the stand-alone conv1's.
 //
-// Warp roles (384 threads, 1 CTA / SM, persistent over M tiles, blockIdx.y = head pair):
+// Warp roles (384 threads, 1 CTA / SM, persistent over M tiles; the CTAs are split among the head pairs by
+// hf_split_ctas in heads_split.cuh):
 //   warp 0 : TMA producer (activation halo tiles)      warp 3 : bulk-copy producer (conv1 + conv2 weight blocks)
 //   warp 1 : MMA issuer                                warp 2 : TMEM allocation
 //   warps 4-11 : epilogue (two per TMEM lane quarter)
@@ -23,36 +28,40 @@
 #include <cuda_bf16.h>
 
 #include "common.cuh"
+#include "heads_split.cuh"
+#include "p8_device.cuh"
 #include "ptx_sm100.cuh"
 
 namespace abc {
 
 constexpr int kHfThreads = 384;
-constexpr int kHfNA = 2, kHfNB = 3;
 constexpr int kHfMaxPairs = 8, kHfMaxItems = 6;
 constexpr uint32_t kHfHeader = 4096;
 constexpr uint32_t kHfARow = 10 * 16, kHfAPlane = 18 * kHfARow, kHfAStage = 8 * kHfAPlane;   // 64 channels = 8 planes
 constexpr uint32_t kHfBBlock = 256 * 64 * 2;
-constexpr uint32_t kHfHid = 128 * 128 * 2;          // hidden map of one head for one 128-pixel tile
-constexpr uint32_t kHfSmem = kHfHeader + kHfNA * kHfAStage + kHfNB * kHfBBlock + 2 * kHfHid;
-static_assert(kHfSmem <= 232448, "shared memory budget");
+constexpr uint32_t kHfSmemLimit = 232448;
+constexpr int kHfNA = 2;
+constexpr int kHfNB = static_cast<int>((kHfSmemLimit - kHfHeader - kHfNA * kHfAStage) / kHfBBlock);   // 5 weight blocks
+constexpr uint32_t kHfSmem = kHfHeader + kHfNA * kHfAStage + kHfNB * kHfBBlock;
+static_assert(kHfSmem <= kHfSmemLimit, "shared memory budget");
 
 struct HfItem {          // one conv2 chunk: <= 128 output channels of one head
   int head_slot;         // 0 / 1: first / second head of the pair
   int nc;                // GEMM N of this chunk (multiple of 16, <= 128)
   int ch0;               // first output channel of the head covered by this chunk
-  int w2_off;            // byte offset of the packed [16][nc][8] bf16 weight block in w2
+  int w2_off;            // byte offset of the packed [16][nc][8] 16-bit weight block in w2
   int bias_off;          // offset (floats) of the chunk's bias in the pair's bias2 block
   int slot;              // issued after this (chunk, tap) step of the NEXT tile's conv1 (0..17)
-  int first, last;       // first / last chunk of its head
 };
 
 struct HfParams {
   int N, H, W, tiles_x, tiles_y, num_tiles, in_plane_off;
-  const uint8_t* w1;     // packed conv1 weights [pair][chunk 2][tap 9][8][256][8] bf16
+  const uint8_t* w1;     // packed conv1 weights [pair][chunk 2][tap 9][8][256][8] 16-bit
   const float* bias1;    // [pairs * 256]
   const uint8_t* w2;
   const float* bias2;    // per pair: bias2_off[pair] .. (+ bias2_len[pair])
+  int pairs;
+  int cta0[kHfMaxPairs + 1];   // CTAs [cta0[p], cta0[p + 1]) work on pair p
   int bias2_off[kHfMaxPairs], bias2_len[kHfMaxPairs];
   int n_items[kHfMaxPairs];
   HfItem items[kHfMaxPairs][kHfMaxItems];
@@ -63,38 +72,28 @@ struct HfParams {
   uint32_t tap16[9];
 };
 
-__device__ __forceinline__ uint4 hf_pack8(const float* v) {
-  __nv_bfloat162 a = __floats2bfloat162_rn(v[0], v[1]);
-  __nv_bfloat162 b = __floats2bfloat162_rn(v[2], v[3]);
-  __nv_bfloat162 c = __floats2bfloat162_rn(v[4], v[5]);
-  __nv_bfloat162 d = __floats2bfloat162_rn(v[6], v[7]);
-  uint4 r;
-  r.x = *reinterpret_cast<uint32_t*>(&a);
-  r.y = *reinterpret_cast<uint32_t*>(&b);
-  r.z = *reinterpret_cast<uint32_t*>(&c);
-  r.w = *reinterpret_cast<uint32_t*>(&d);
-  return r;
-}
-
+// kF16: activations and weights are IEEE fp16 (UNet(act_dtype="fp16")), else bf16
+template <bool kF16>
 __global__ void __launch_bounds__(kHfThreads, 1)
 heads_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ HfParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   const uint32_t sbase = smem_u32(smem);
   const int warp = static_cast<int>(warp_id_uniform());
   const int lane = threadIdx.x & 31;
-  const int pair = blockIdx.y;
+  int pair = 0;
+  while (pair + 1 < p.pairs && static_cast<int>(blockIdx.x) >= p.cta0[pair + 1]) ++pair;
+  const int cta_rank = blockIdx.x - p.cta0[pair], cta_stride = p.cta0[pair + 1] - p.cta0[pair];
 
   // barrier slots (8 bytes each)
   const uint32_t bar_a_full = sbase, bar_a_empty = sbase + 8 * kHfNA;
   const uint32_t bar_b_full = sbase + 8 * 2 * kHfNA, bar_b_empty = bar_b_full + 8 * kHfNB;
-  const uint32_t bar_acc_full = bar_b_empty + 8 * kHfNB;       // [2] conv1 accumulators of a stage complete
-  const uint32_t bar_acc_empty = bar_acc_full + 16;            // [2] stage fully drained (after the conv2 logits)
-  const uint32_t bar_hid_full = bar_acc_empty + 16;            // [2 heads] hidden operand written to shared memory
-  const uint32_t bar_hid_empty = bar_hid_full + 16;            // [2 heads] conv2 MMAs have finished reading it
-  const uint32_t bar_c2_full = bar_hid_empty + 16;             // [2 heads] a conv2 chunk is complete in TMEM
-  const uint32_t bar_c2_empty = bar_c2_full + 16;              // [2 heads] ... and has been drained
+  const uint32_t bar_acc_full = bar_b_empty + 8 * kHfNB;       // [2] conv1 accumulators of a buffer complete
+  const uint32_t bar_acc_empty = bar_acc_full + 16;            // [2] buffer fully drained (after the conv2 logits)
+  const uint32_t bar_hid_full = bar_acc_empty + 16;            // both hidden operands of a tile written to TMEM
+  const uint32_t bar_c2_full = bar_hid_full + 8;               // a conv2 chunk is complete in TMEM
+  const uint32_t bar_c2_empty = bar_c2_full + 8;               // ... and has been drained
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + 512);
-  HfItem* items_s = reinterpret_cast<HfItem*>(smem + 576);     // [kHfMaxItems] (32 bytes each)
+  HfItem* items_s = reinterpret_cast<HfItem*>(smem + 576);     // [kHfMaxItems]
   float* bias1_s = reinterpret_cast<float*>(smem + 1024);      // [256]
   float* bias2_s = reinterpret_cast<float*>(smem + 2048);      // [512]
   const int n_items = p.n_items[pair];
@@ -111,11 +110,10 @@ heads_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
     for (int i = 0; i < 2; ++i) {
       mbar_init(bar_acc_full + 8 * i, 1);
       mbar_init(bar_acc_empty + 8 * i, 8);
-      mbar_init(bar_hid_full + 8 * i, 8);
-      mbar_init(bar_hid_empty + 8 * i, 1);
-      mbar_init(bar_c2_full + 8 * i, 1);
-      mbar_init(bar_c2_empty + 8 * i, 8);
     }
+    mbar_init(bar_hid_full, 8);
+    mbar_init(bar_c2_full, 1);
+    mbar_init(bar_c2_empty, 8);
     fence_mbar_init();
     tma_prefetch_desc(&tmap);
   }
@@ -130,17 +128,16 @@ heads_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
 
   const uint32_t a_region = sbase + kHfHeader;
   const uint32_t b_region = a_region + kHfNA * kHfAStage;
-  const uint32_t hid_region = b_region + kHfNB * kHfBBlock;
   const int tiles_per_img = p.tiles_x * p.tiles_y;
-  // tiles of this CTA: blockIdx.x, blockIdx.x + gridDim.x, ...
-  const int my_tiles = (p.num_tiles > static_cast<int>(blockIdx.x)) ? (p.num_tiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
+  // tiles of this CTA: cta_rank, cta_rank + cta_stride, ...
+  const int my_tiles = (p.num_tiles > cta_rank) ? (p.num_tiles - cta_rank + cta_stride - 1) / cta_stride : 0;
 
   if (warp == 0) {
     // ------------------------------------------------------------------ A producer
     int stage = 0;
     uint32_t phase = 0;
     for (int it = 0; it < my_tiles; ++it) {
-      const int g = blockIdx.x + it * gridDim.x;
+      const int g = cta_rank + it * cta_stride;
       const int n = g / tiles_per_img;
       const int rem = g - n * tiles_per_img;
       const int ty = rem / p.tiles_x, tx = rem - ty * p.tiles_x;
@@ -201,19 +198,16 @@ heads_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
     }
   } else if (warp == 1) {
     // ------------------------------------------------------------------ MMA issuer
-    const uint32_t idesc1 = umma_idesc_bf16(128, 256, 0, 0);
+    const uint32_t idesc1 = umma_idesc_16(128, 256, 0, 0, kF16);
     const uint64_t a_hi64 = umma_desc_hi(kHfAPlane, kHfARow);
     const uint64_t b_hi64 = umma_desc_hi(256 * 16, 128);
-    const uint64_t h_hi64 = umma_desc_hi(2048, 128);           // hidden operand: plane pitch 128 pixels x 16 B
     const uint32_t a_hi = static_cast<uint32_t>(a_hi64 >> 32), b_hi = static_cast<uint32_t>(b_hi64 >> 32);
-    const uint32_t h_hi = static_cast<uint32_t>(h_hi64 >> 32);
     const uint32_t a_lo0 = static_cast<uint32_t>(a_hi64) | (a_region >> 4);
     const uint32_t b_lo0 = static_cast<uint32_t>(b_hi64) | (b_region >> 4);
-    const uint32_t h_lo0 = static_cast<uint32_t>(h_hi64) | (hid_region >> 4);
     constexpr uint32_t a_kstep = (2 * kHfAPlane) >> 4, b_kstep = (2 * 256 * 16) >> 4;
     int a_stage = 0, b_stage = 0;
     uint32_t a_phase = 0, b_phase = 0;
-    uint32_t acc_empty_phase = 0, hid_full_phase = 0, c2_empty_phase = 0;   // one phase bit per barrier index
+    uint32_t acc_empty_phase = 0, hid_full_phase = 0, c2_empty_phase = 0;   // acc_empty: one phase bit per buffer
     for (int it = 0; it <= my_tiles; ++it) {
       const bool has_c1 = it < my_tiles, has_c2 = it >= 1;
       if (!has_c1 && !has_c2) break;
@@ -258,28 +252,26 @@ heads_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
         if (has_c2) {
           while (next_item < n_items && (items_s[next_item].slot <= slot || !has_c1)) {
             const HfItem item = items_s[next_item];
-            const int hs = item.head_slot;
-            if (item.first) {                                  // hidden operand of the previous tile is in shared memory
-              mbar_wait(bar_hid_full + 8 * hs, (hid_full_phase >> hs) & 1u);
-              hid_full_phase ^= 1u << hs;
+            if (next_item == 0) {                              // hidden operands of the previous tile are in TMEM
+              mbar_wait(bar_hid_full, hid_full_phase);
+              hid_full_phase ^= 1u;
             }
-            mbar_wait(bar_c2_empty + 8 * hs, ((c2_empty_phase >> hs) & 1u) ^ 1u);   // the head's TMEM columns have been drained
-            c2_empty_phase ^= 1u << hs;
+            mbar_wait(bar_c2_empty, c2_empty_phase ^ 1u);      // the previous chunk has been drained
+            c2_empty_phase ^= 1u;
             mbar_wait(bar_b_full + 8 * b_stage, b_phase);
             tc_fence_after();
-            const uint32_t idesc2 = umma_idesc_bf16(128, item.nc, 0, 0);
+            const uint32_t idesc2 = umma_idesc_16(128, item.nc, 0, 0, kF16);
             const uint64_t w_hi64 = umma_desc_hi(static_cast<uint32_t>(item.nc) * 16, 128);
             const uint32_t w_hi = static_cast<uint32_t>(w_hi64 >> 32);
             const uint32_t w_lo = static_cast<uint32_t>(w_hi64) | ((b_region + b_stage * kHfBBlock) >> 4);
-            const uint32_t h_lo = h_lo0 + hs * (kHfHid >> 4);
-            const uint32_t d2 = tmem_base + sp * 256 + hs * 128;
+            const uint32_t a2 = tmem_base + sp * 256 + item.head_slot * 64;
+            const uint32_t d2 = tmem_base + sp * 256 + 128;
             if (elect_one()) {
 #pragma unroll
               for (int k = 0; k < 8; ++k)
-                umma_bf16_lohi(d2, h_lo + k * (4096 >> 4), h_hi, w_lo + k * 2 * item.nc, w_hi, idesc2, k != 0 ? 1u : 0u);
+                umma_16_ts(d2, a2 + k * 8, w_lo + k * 2 * item.nc, w_hi, idesc2, k != 0 ? 1u : 0u);
               umma_commit(bar_b_empty + 8 * b_stage);
-              umma_commit(bar_c2_full + 8 * hs);
-              if (item.last) umma_commit(bar_hid_empty + 8 * hs);
+              umma_commit(bar_c2_full);
             }
             __syncwarp();
             if (++b_stage == kHfNB) {
@@ -304,9 +296,9 @@ heads_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
     const float4* bias1_4 = reinterpret_cast<const float4*>(bias1_s);
     const float4* bias2_4 = reinterpret_cast<const float4*>(bias2_s);
     const size_t plane_px = static_cast<size_t>(p.H) * p.W;
-    uint32_t acc_full_phase = 0, hid_empty_phase = 0, c2_full_phase = 0;      // one phase bit per barrier index
+    uint32_t acc_full_phase = 0, c2_full_phase = 0;        // acc_full: one phase bit per buffer
     for (int it = 0; it < my_tiles; ++it) {
-      const int g = blockIdx.x + it * gridDim.x;
+      const int g = cta_rank + it * cta_stride;
       const int n = g / tiles_per_img;
       const int rem = g - n * tiles_per_img;
       const int ty = rem / p.tiles_x, tx = rem - ty * p.tiles_x;
@@ -318,51 +310,53 @@ heads_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
       mbar_wait(bar_acc_full + 8 * s, (acc_full_phase >> s) & 1u);
       acc_full_phase ^= 1u << s;
       tc_fence_after();
-      // ---- phase 1: conv1 accumulators -> bias + LeakyReLU -> bf16 hidden operand in shared memory
+      // ---- phase 1: conv1 accumulators -> bias + LeakyReLU -> 16-bit hidden operand, back into TMEM. This warp takes
+      // channels [64 eh, 64 eh + 64) of each head: accumulator columns hs * 128 + 64 eh + [0, 64) -> packed columns
+      // hs * 64 + 32 eh + [0, 32). Hidden A and B overwrite head A's accumulators, which BOTH warps of the lane quarter
+      // must have loaded first (the named barrier); head B's accumulators are not overwritten in this phase.
 #pragma unroll 1
       for (int hs = 0; hs < 2; ++hs) {
-        mbar_wait(bar_hid_empty + 8 * hs, ((hid_empty_phase >> hs) & 1u) ^ 1u);
-        hid_empty_phase ^= 1u << hs;
-        uint8_t* hid = smem + (hid_region - sbase) + hs * kHfHid + m * 16;
-        uint32_t raw[2][16];
-        // this warp's units of the head: eh, eh + 2, eh + 4, eh + 6 (16 channels = 2 planes each), two per round
+        uint32_t raw[4][16];
 #pragma unroll
-        for (int round = 0; round < 2; ++round) {
-          const int u0 = eh + 4 * round, u1 = u0 + 2;
-          tmem_ld16(tstage + hs * 128 + u0 * 16, raw[0]);
-          tmem_ld16(tstage + hs * 128 + u1 * 16, raw[1]);
-          tmem_ld_wait();
-#pragma unroll
-          for (int h2 = 0; h2 < 2; ++h2) {
-            const int u = h2 ? u1 : u0;
-            float v[16];
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-              const float4 bb = bias1_4[hs * 32 + u * 4 + i];
-              const float t0 = __uint_as_float(raw[h2][4 * i + 0]) + bb.x, t1 = __uint_as_float(raw[h2][4 * i + 1]) + bb.y;
-              const float t2 = __uint_as_float(raw[h2][4 * i + 2]) + bb.z, t3 = __uint_as_float(raw[h2][4 * i + 3]) + bb.w;
-              v[4 * i + 0] = fmaxf(t0, 0.01f * t0);
-              v[4 * i + 1] = fmaxf(t1, 0.01f * t1);
-              v[4 * i + 2] = fmaxf(t2, 0.01f * t2);
-              v[4 * i + 3] = fmaxf(t3, 0.01f * t3);
-            }
-            *reinterpret_cast<uint4*>(hid + (2 * u) * 2048) = hf_pack8(v);
-            *reinterpret_cast<uint4*>(hid + (2 * u + 1) * 2048) = hf_pack8(v + 8);
-          }
+        for (int i = 0; i < 4; ++i) tmem_ld16(tstage + hs * 128 + eh * 64 + i * 16, raw[i]);
+        tmem_ld_wait();
+        if (hs == 0) {
+          tc_fence_before();
+          named_bar_sync(1 + q, 64);
+          tc_fence_after();
         }
-        fence_proxy_async();               // make the generic-proxy writes visible to the tensor core (async proxy)
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(bar_hid_full + 8 * hs);
+        uint32_t packed[32];
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+          float v[16];
+#pragma unroll
+          for (int j = 0; j < 4; ++j) {
+            const float4 bb = bias1_4[hs * 32 + eh * 16 + i * 4 + j];
+            const float t0 = __uint_as_float(raw[i][4 * j + 0]) + bb.x, t1 = __uint_as_float(raw[i][4 * j + 1]) + bb.y;
+            const float t2 = __uint_as_float(raw[i][4 * j + 2]) + bb.z, t3 = __uint_as_float(raw[i][4 * j + 3]) + bb.w;
+            v[4 * j + 0] = fmaxf(t0, 0.01f * t0);
+            v[4 * j + 1] = fmaxf(t1, 0.01f * t1);
+            v[4 * j + 2] = fmaxf(t2, 0.01f * t2);
+            v[4 * j + 3] = fmaxf(t3, 0.01f * t3);
+          }
+          const uint4 u0 = pack8_act16(v, kF16), u1 = pack8_act16(v + 8, kF16);
+          packed[8 * i + 0] = u0.x; packed[8 * i + 1] = u0.y; packed[8 * i + 2] = u0.z; packed[8 * i + 3] = u0.w;
+          packed[8 * i + 4] = u1.x; packed[8 * i + 5] = u1.y; packed[8 * i + 6] = u1.z; packed[8 * i + 7] = u1.w;
+        }
+        tmem_st16(tstage + hs * 64 + eh * 32, packed);
+        tmem_st16(tstage + hs * 64 + eh * 32 + 16, packed + 16);
       }
+      tmem_st_wait();
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(bar_hid_full);
       // ---- phase 2: conv2 accumulators of this tile (issued during the next tile's conv1) -> + bias -> fp32 logits
 #pragma unroll 1
       for (int ii = 0; ii < n_items; ++ii) {
         const HfItem item = items_s[ii];
-        const int hs = item.head_slot;
-        const int head = 2 * pair + hs;
-        mbar_wait(bar_c2_full + 8 * hs, (c2_full_phase >> hs) & 1u);
-        c2_full_phase ^= 1u << hs;
+        const int head = 2 * pair + item.head_slot;
+        mbar_wait(bar_c2_full, c2_full_phase);
+        c2_full_phase ^= 1u;
         tc_fence_after();
         const int units = item.nc >> 4;
         const int cout = p.cout[head];
@@ -370,7 +364,7 @@ heads_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
         uint32_t raw[16];
 #pragma unroll 1
         for (int u = eh; u < units; u += 2) {
-          tmem_ld16(tstage + hs * 128 + u * 16, raw);
+          tmem_ld16(tstage + 128 + u * 16, raw);
           tmem_ld_wait();
           const int ch0 = item.ch0 + u * 16;
           float v[16];
@@ -403,7 +397,7 @@ heads_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
         }
         tc_fence_before();
         __syncwarp();
-        if (lane == 0) mbar_arrive(bar_c2_empty + 8 * hs);
+        if (lane == 0) mbar_arrive(bar_c2_empty);
       }
       if (lane == 0) mbar_arrive(bar_acc_empty + 8 * s);
     }
@@ -478,18 +472,20 @@ extern "C" int abc_heads_fused(const AbcHeadsFusedDesc* d, void* stream_) {
         it.ch0 = 128 * cidx;
         it.w2_off = w2_off;
         it.bias_off = bias_len;
-        it.first = cidx == 0;
-        it.last = cidx == chunks - 1;
-        // issue points inside the next tile's conv1 stream: first chunks at the end of K chunk 0, further ones spread over chunk 1
-        int slot = d->item_slot[ni] >= 0 && d->item_slot[ni] < 18 ? d->item_slot[ni] : (cidx == 0 ? 8 : (cidx == 1 ? 12 : 16));
-        if (ni > 0 && slot < p.items[pr][ni - 1].slot) slot = p.items[pr][ni - 1].slot;
-        it.slot = slot;
         w2_off += it.nc * 256;
         bias_len += it.nc;
         ++ni;
       }
     }
     ABC_REQUIRE(bias_len <= 512, "abc_heads_fused: pair %d: %d conv2 output columns exceed the 512 supported", pr, bias_len);
+    // issue points inside the next tile's conv1 stream (18 (chunk, tap) steps). The chunks share one TMEM region, so each
+    // waits for the drain of the one before. Measured on B200 with the v2 heads (ABCNET_HF_SLOTS sweep): early and 4 steps
+    // apart (2, 6, 10, 14) beat later or more evenly spread points by 0.4 - 1 ms.
+    for (int i = 0; i < ni; ++i) {
+      int slot = d->item_slot[i] >= 0 && d->item_slot[i] < 18 ? d->item_slot[i] : (2 + 4 * i < 17 ? 2 + 4 * i : 17);
+      if (i > 0 && slot < p.items[pr][i - 1].slot) slot = p.items[pr][i - 1].slot;
+      p.items[pr][i].slot = slot;
+    }
     p.n_items[pr] = ni;
     p.bias2_len[pr] = bias_len;
     bias_off_total += bias_len;
@@ -510,7 +506,8 @@ extern "C" int abc_heads_fused(const AbcHeadsFusedDesc* d, void* stream_) {
                                  static_cast<cuuint64_t>(d->W) * d->H * 16 * d->in_planes};
   const cuuint32_t box[4] = {80, 18, 8, 1};
   const cuuint32_t estr[4] = {1, 1, 1, 1};
-  CUresult cr = encode(&tmap, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(d->in), gdim, gstride, box, estr,
+  const bool f16 = d->act_fp16 != 0;
+  CUresult cr = encode(&tmap, f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(d->in), gdim, gstride, box, estr,
                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (cr != CUDA_SUCCESS) {
@@ -518,14 +515,29 @@ extern "C" int abc_heads_fused(const AbcHeadsFusedDesc* d, void* stream_) {
     return ABC_ERR_CUDA;
   }
   static PerDeviceOnce attr_once;
-  ABC_CUDA(attr_once.run([] { return cudaFuncSetAttribute(heads_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kHfSmem); }));
+  ABC_CUDA(attr_once.run([] {
+    cudaError_t e = cudaFuncSetAttribute(heads_fused_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kHfSmem);
+    return e != cudaSuccess ? e : cudaFuncSetAttribute(heads_fused_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kHfSmem);
+  }));
   int sms = sm_count();
   if (sms <= 0) sms = 148;
-  int gx = sms / pairs;
-  if (gx < 1) gx = 1;
-  if (gx > p.num_tiles) gx = p.num_tiles;
-  dim3 grid(gx, pairs, 1);
-  heads_fused_kernel<<<grid, kHfThreads, kHfSmem, static_cast<cudaStream_t>(stream_)>>>(tmap, p);
+  int64_t cost[kHfMaxPairs];
+  for (int pr = 0; pr < pairs; ++pr) {
+    int nc[kHfMaxItems], channels = 0;
+    for (int i = 0; i < p.n_items[pr]; ++i) nc[i] = p.items[pr][i].nc;
+    for (int hs = 0; hs < 2 && 2 * pr + hs < d->n_heads; ++hs) channels += d->cout[2 * pr + hs];
+    cost[pr] = hf_pair_tile_cost(p.n_items[pr], nc, channels);
+  }
+  int ctas[kHfMaxPairs];
+  const int total = hf_split_ctas(pairs, cost, sms, p.num_tiles, ctas);
+  p.pairs = pairs;
+  p.cta0[0] = 0;
+  for (int pr = 0; pr < pairs; ++pr) p.cta0[pr + 1] = p.cta0[pr] + ctas[pr];
+  cudaStream_t st = static_cast<cudaStream_t>(stream_);
+  if (f16)
+    heads_fused_kernel<true><<<total, kHfThreads, kHfSmem, st>>>(tmap, p);
+  else
+    heads_fused_kernel<false><<<total, kHfThreads, kHfSmem, st>>>(tmap, p);
   return launch_check("heads_fused_kernel");
 }
 

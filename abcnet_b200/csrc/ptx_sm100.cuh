@@ -117,6 +117,18 @@ __device__ __forceinline__ void umma_bf16_lohi(uint32_t tmem_d, uint32_t a_lo, u
       ::"r"(tmem_d), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// D[tmem] (+)= A[tmem] * B[smem]: A is M = 128 lanes (one row each) x K / 2 columns, two 16-bit elements per 32-bit column
+// (the lower half holds the even K index), so a K step of 16 advances the A address by 8 columns.
+__device__ __forceinline__ void umma_16_ts(uint32_t tmem_d, uint32_t tmem_a, uint32_t b_lo, uint32_t b_hi, uint32_t idesc,
+                                           uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t.reg .b64 db;\n\t"
+      "mov.b64 db, {%2, %3};\n\t"
+      "setp.ne.b32 p, %5, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], db, %4, p;\n\t}"
+      ::"r"(tmem_d), "r"(tmem_a), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 // mbarrier arrive when all previously issued tcgen05 ops of this thread have completed
 // (implies tcgen05.fence::before_thread_sync).
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
@@ -132,6 +144,19 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
         "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
       : "r"(taddr)
       : "memory");
+}
+// the inverse: thread i -> TMEM lane (lane_base + i), columns [c, c+16); complete after tmem_st_wait()
+__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t* r) {
+  asm volatile(
+      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};"
+      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]),
+        "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
+      : "memory");
+}
+__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
+// barrier among `threads` threads (whole warps) of the CTA; id 0 is __syncthreads
+__device__ __forceinline__ void named_bar_sync(uint32_t id, uint32_t threads) {
+  asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(threads) : "memory");
 }
 
 // ----------------------------------------------------------------------------- CTA pair (cta_group::2)

@@ -397,7 +397,7 @@ class UNet(nn.Module):
             # 128 (4.36) and two of 256 (3.9): fewer re-reads of the hidden tile at the same padding.
             n_tile = 16 if h <= 16 else (64 if h <= 64 else (128 if h <= 128 else (192 if (h + 191) // 192 * 192 <= (h + 127) // 128 * 128 else 128)))
             P[f"heads.{i}.conv2"] = _Packed(w2.unsqueeze(0).contiguous(), om.conv2.bias.detach().float(), [(0, 0)], n_tile, h, dtype=adt)
-        P["heads.fused"] = self._pack_fused_heads(dev) if self.act_dtype == "bf16" else None      # abc_heads_fused is a bf16 kernel
+        P["heads.fused"] = self._pack_fused_heads(dev)
         self._packed = P
         self._packed_key = self._param_key()
         self._pack_gen += 1                  # consumers that derive their own packs (SparseHeadsPipeline) key on this
@@ -415,6 +415,7 @@ class UNet(nn.Module):
             cols = sum(sum(((min(h - c0, 128) + 15) // 16) * 16 for c0 in range(0, h, 128)) for h in pair)
             if chunks > 6 or cols > 512:
                 return None
+        adt = self._act_torch_dtype
         blocks, biases = [], []
         for om, h in zip(self.out_modules, heads):
             w2 = om.conv2.weight.detach().float().reshape(h, -1)
@@ -424,7 +425,8 @@ class UNet(nn.Module):
                 nc = (cnt + 15) // 16 * 16
                 wb = w2.new_zeros(nc, 128)
                 wb[:cnt] = w2[c0:c0 + cnt]
-                blocks.append(wb.view(nc, 16, 8).permute(1, 0, 2).contiguous().to(torch.bfloat16).reshape(-1))
+                wb = wb.view(nc, 16, 8).permute(1, 0, 2).contiguous()
+                blocks.append((wb.clamp(-65504.0, 65504.0) if adt == torch.float16 else wb).to(adt).reshape(-1))   # as _Packed
                 bb = b2.new_zeros(nc)
                 bb[:cnt] = b2[c0:c0 + cnt]
                 biases.append(bb)
@@ -623,8 +625,9 @@ class UNet(nn.Module):
         """Eval forward. layout="nchw": the reference's list of fp32 NCHW tensors. layout="p8f": a ``HeadMaps`` list in
         which heads with more than one channel are fp32 planar-8 [B, ceil(h/8), H/4, W/4, 8] (padding slots undefined);
         this is the format the fused inference + decode path uses (``PeakDecoder`` accepts both).
-        fused=True (or ABCNET_FUSED_HEADS=1): conv1 + LeakyReLU + conv2 of all heads in one kernel (abc_heads_fused);
-        default: conv1 and the per-head conv2 as separate launches (hidden maps materialised in HBM)."""
+        fused=None (default): conv1 + LeakyReLU + conv2 of all heads in one kernel (abc_heads_fused) whenever the head list is
+        within its limits, unless ABCNET_FUSED_HEADS=0; fused=True requires it; fused=False: conv1 and the per-head conv2 as
+        separate launches (hidden maps materialised in HBM)."""
         if layout not in ("nchw", "p8f"):
             raise ValueError("layout must be 'nchw' or 'p8f'")
         p8f = layout == "p8f"
@@ -638,18 +641,18 @@ class UNet(nn.Module):
                 outs.append(torch.empty(shape, dtype=torch.float32, device=k2.device))
         fpack = self._packed.get("heads.fused")
         if fused is None:
-            # measured on B200 (profiles/r01_bench_v8_fused_heads.json): 12.1 ms fused against 6.9 + 3.4 ms for the separate
-            # launches -- with two 32 KB hidden operands in shared memory the weight ring shrinks to 3 blocks and the
-            # L2 -> SM weight stream (64 B/clk/SM at the MMA rate) starves the tensor pipe. Opt-in until that is fixed.
-            fused = fpack is not None and os.environ.get("ABCNET_FUSED_HEADS", "0") == "1"
+            # the hidden maps stay in TMEM, so the fused kernel saves their 2 x 8.6 GB HBM round trip per 256-image batch
+            # (DESIGN.md 4.2); ABCNET_FUSED_HEADS=0 selects the separate launches for A/B runs
+            fused = fpack is not None and os.environ.get("ABCNET_FUSED_HEADS", "1") != "0"
         if fused:
             if fpack is None:
-                raise ValueError("abc_heads_fused is not available for this head list / act_dtype (see include/abcnet_b200.h); use fused=False")
+                raise ValueError("abc_heads_fused is not available for this head list (see include/abcnet_b200.h); use fused=False")
             w2pack, bias2 = fpack
             pk1 = self._packed["heads.conv1.plain"]
             if pk1 is None:
                 wt1, b1, c1 = self._heads_w1
-                pk1 = self._packed["heads.conv1.plain"] = _Packed(wt1, b1, [(dy, dx) for (dy, dx, _, _) in _TAPS3], 256, c1, pair=False)      # bf16 only
+                pk1 = self._packed["heads.conv1.plain"] = _Packed(wt1, b1, [(dy, dx) for (dy, dx, _, _) in _TAPS3], 256, c1, pair=False,
+                                                                  dtype=self._act_torch_dtype)
             d = AbcHeadsFusedDesc()
             d.in_, d.N, d.H, d.W, d.in_planes, d.in_plane_off = k2.data_ptr(), B, H4, W4, k2.shape[1], 0
             d.w1pack, d.bias1, d.n_heads = pk1.w.data_ptr(), pk1.bias.data_ptr(), len(self.heads)
@@ -657,6 +660,7 @@ class UNet(nn.Module):
             slots = [int(v) for v in os.environ.get("ABCNET_HF_SLOTS", "").split(",") if v.strip()]
             for i in range(6):
                 d.item_slot[i] = slots[i] if i < len(slots) else -1
+            d.act_fp16 = int(pk1.fp16)
             for i, h in enumerate(self.heads):
                 d.cout[i], d.out[i] = h, outs[i].data_ptr()
                 d.out_mode[i] = 2 if outs[i].dim() == 5 else 1

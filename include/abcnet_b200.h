@@ -172,15 +172,17 @@ ABC_API int64_t abc_conv_wpack_bytes(int cin, int cout, int ntaps, int n_tile);
 /* ---------------------------------------------------------------------------------------------------
  * Fused output heads (inference): for every head conv3x3(128 -> 128) + BatchNorm (folded) + LeakyReLU(0.01) +
  * conv1x1(128 -> cout[h]) in one kernel -- OutConv, src/unet.py:63-74, applied to the shared trunk at :116-118. The hidden
- * 128-channel maps stay in shared memory / TMEM (csrc/heads_fused_sm100.cu). Two heads share one CTA column.
+ * 128-channel maps stay in tensor memory (csrc/heads_fused_sm100.cu). Two heads share one CTA; the CTAs are split among
+ * the head pairs in proportion to their work (csrc/heads_split.cuh).
  *   w1pack / bias1 : conv1 of all heads concatenated on the output-channel axis, packed as for abc_conv_igemm with
  *                    n_tile = 256 and the 3x3 taps in (ky, kx) order (zero-padded to a multiple of 256 channels)
  *   w2pack / bias2 : conv2 in (head, chunk) order, chunk c = output channels [128 c, 128 (c + 1)) of the head with
- *                    nc = count rounded up to 16: bf16 [16 (K planes)][nc][8] (zero rows past the count), bias fp32 [nc];
+ *                    nc = count rounded up to 16: 16-bit [16 (K planes)][nc][8] (zero rows past the count), bias fp32 [nc];
  *                    total sizes from abc_heads_fused_pack_sizes
  *   out[h]         : fp32 logits, out_mode[h] = 1: NCHW [N][cout][H][W]; 2: planar-8 [N][out_planes][H][W][8]
- *   item_slot[i]   : tuning knob, -1 = default: the i-th conv2 chunk of a CTA column is issued after this (K chunk, tap)
+ *   item_slot[i]   : tuning knob, -1 = default: the i-th conv2 chunk of a head pair is issued after this (K chunk, tap)
  *                    step (0..17) of the next tile's conv1
+ *   act_fp16       : 0: bf16 trunk and weights; 1: IEEE fp16 (AbcConvDesc.act_fp16), hidden maps rounded to fp16
  * Limits: n_heads <= 16, at most 6 chunks and 512 padded conv2 channels per pair of heads.
  */
 typedef struct AbcHeadsFusedDesc {
@@ -199,6 +201,7 @@ typedef struct AbcHeadsFusedDesc {
   int out_mode[16];
   int out_planes[16];
   int item_slot[6];
+  int act_fp16;
 } AbcHeadsFusedDesc;
 ABC_API int abc_heads_fused(const AbcHeadsFusedDesc* desc, void* stream);
 ABC_API int abc_heads_fused_pack_sizes(int n_heads, const int* cout, int64_t* w2pack_bytes, int* bias2_len);
