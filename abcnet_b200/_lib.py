@@ -18,7 +18,7 @@ EXPORTS = (
     "abc_loss_partials", "abc_loss_backward", "abc_loss_partials_p8",
     "abc_bn_stats", "abc_bn_finalize", "abc_bn_act", "abc_bn_act_backward", "abc_nchw_to_p8", "abc_channel_sum",
     "abc_nchw_to_p8_ex", "abc_deinterleave2", "abc_conv_wgrad", "abc_conv3x3_c1_wgrad", "abc_conv3x3_c1_raw",
-    "abc_heads_fused", "abc_heads_fused_pack_sizes", "abc_gather_pack", "abc_adam_step", "abc_adam_chunk_elems", "abc_assemble_molblocks", "abc_gather_patches", "abc_rasterise_targets",
+    "abc_heads_fused", "abc_heads_fused_pack_sizes", "abc_gather_pack", "abc_adam_step", "abc_adam_chunk_elems", "abc_assemble_molblocks", "abc_gather_patches", "abc_gather_patches_pooled", "abc_rasterise_targets",
     "abc_unet_wpack_bytes", "abc_unet_workspace_bytes", "abc_unet_create", "abc_unet_forward_infer", "abc_unet_destroy", "abc_unet_pack_host",
 )
 
@@ -68,6 +68,7 @@ class AbcDecodeDesc(C.Structure):
         ("bonds", C.c_void_p), ("bond_cap", C.c_int),
         ("counts", C.c_void_p), ("p8f_mask", C.c_int), ("centre_prob", C.c_int), ("thr_omega", C.c_float),
         ("peak_pix", C.c_void_p), ("peak_cnt", C.c_void_p), ("peak_cap", C.c_int), ("sparse_mode", C.c_int),
+        ("peak_off", C.c_void_p), ("pool_slots", C.c_int),
     ]
 
 
@@ -185,6 +186,7 @@ def _load():
     lib.abc_adam_step.argtypes = [vp, vp, vp, vp, vp, vp, ci, vp, vp, vp]
     lib.abc_rasterise_targets.argtypes = [C.POINTER(AbcTargetsDesc), vp]
     lib.abc_gather_patches.argtypes = [vp, ci, ci, ci, ci, vp, vp, ci, vp, vp]
+    lib.abc_gather_patches_pooled.argtypes = [vp, ci, ci, ci, ci, vp, vp, vp, ci, vp, vp]
     lib.abc_unet_wpack_bytes.restype = C.c_int64
     lib.abc_unet_wpack_bytes.argtypes = [C.POINTER(AbcUNetConfig)]
     lib.abc_unet_workspace_bytes.restype = C.c_int64

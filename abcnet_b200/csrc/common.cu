@@ -75,7 +75,7 @@ int sm_count() {
 
 extern "C" {
 const char* abc_last_error(void) { return abc::g_err; }
-int abc_version(void) { return 100; }
+int abc_version(void) { return 101; }
 int abc_device_ok(void) { return abc::device_check() == ABC_OK ? 1 : 0; }
 int abc_sm_count(void) {
   int n = abc::sm_count();

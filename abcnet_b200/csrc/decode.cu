@@ -2,7 +2,7 @@
 // per-peak class arg-max, circular omega NMS + half-circle test, rho / bond-type gather.
 // Kernels: decode_split_kernel (default: one CTA for the atoms and one for the bonds of every image; also the peak-list
 // step of the sparse-heads path), decode_kernel (v1: one CTA per image, ABCNET_DECODE_V1=1), gather_patches_kernel and
-// decode_finish_kernel (sparse heads).
+// decode_finish_kernel (sparse heads, with peak_offsets_kernel in the pooled slot layout of peak_slots.cuh).
 //
 // Replaces, bit-exactly, the dense tensor statements and the per-scalar .cpu().item() loop of
 // /root/reference/src/img2smiles.py:62-80, :115-124 and the gather part of :134-182 (see include/abcnet_b200.h).
@@ -10,6 +10,7 @@
 #include <cstdlib>
 
 #include "common.cuh"
+#include "peak_slots.cuh"
 
 namespace abc {
 
@@ -30,11 +31,11 @@ struct DecParams {
   int p8f_mask;
   int centre_prob;
   float thr_omega;
-  // sparse-heads path (AbcDecodeDesc.sparse_mode): peak lists [N][2][peak_cap] / raw counts [N][2]; hw_gather = pixels per
-  // "image" of the maps the gathers read: H * W, or the number of compact slots N * 2 * peak_cap in finish mode
+  // sparse-heads path (AbcDecodeDesc.sparse_mode): peak lists [N][2][slots.list_stride] / raw counts [N][2]; hw_gather =
+  // pixels per "image" of the maps the gathers read: H * W, or the number of compact slots in finish mode
   int32_t* peak_pix;
   int32_t* peak_cnt;
-  int peak_cap;
+  SlotLayout slots;
   int mode;
   int hw_gather;
 };
@@ -358,14 +359,15 @@ __global__ void __launch_bounds__(kDec2Threads) decode_split_kernel(const DecPar
 
   if (p.mode == 1) {
     // ---------------------------------------------------------------- sparse heads, step 1: ordered peak lists only
-    int32_t* list = p.peak_pix + static_cast<size_t>(n * 2 + bonds) * p.peak_cap;
+    const int stride = p.slots.list_stride;
+    int32_t* list = p.peak_pix + static_cast<size_t>(n * 2 + bonds) * stride;
 #pragma unroll 1
     for (int h = 0; h < 2; ++h) {
       uint32_t fl = h ? hi : lo;
       int idx = warp_off + (h ? tot_lo + inc_hi - cnt_hi : inc_lo - cnt_lo);
       const int base = wbase + (lane + 32 * h) * 32;
       while (fl) {
-        if (idx < p.peak_cap) list[idx] = base + __ffs(fl) - 1;
+        if (idx < stride) list[idx] = base + __ffs(fl) - 1;
         fl &= fl - 1;
         ++idx;
       }
@@ -460,22 +462,23 @@ __global__ void __launch_bounds__(kDec2Threads) decode_split_kernel(const DecPar
 
 // ---------------------------------------------------------------------------------------------------------------
 // Sparse heads (SURVEY.md section 8f, N4): the class / offset heads are only read at peaks, so the fused inference + decode
-// path evaluates them only there. Slot s = (n * 2 + which) * peak_cap + i holds peak i (row-major order) of image n
-// (which = 0 atoms, 1 bond centres). gather_patches_kernel writes, for every valid slot, the 3x3 neighbourhood of the trunk
-// (zero outside the image = the conv padding) as one "pixel" of a compact P8 tensor [1][9 * planes][P / 8][8][8] whose
-// plane order (64-channel chunk, tap, plane) is the K order of the dense 3x3 implicit GEMM: a 1x1 abc_conv_igemm over it
-// with the SAME packed conv1 weights performs, per output element, the same MMA sequence as the dense layer -> identical
-// bits. One warp per slot.
+// path evaluates them only there. Peak i (row-major order) of group g = n * 2 + which (which = 0 atoms, 1 bond centres) of
+// image n owns slot slot_base(g) + i of the compact tensors (peak_slots.cuh: g * peak_cap, or a batch-wide pool through
+// exclusive offsets). gather_patches_kernel writes, for every valid slot, the 3x3 neighbourhood of the trunk (zero outside
+// the image = the conv padding) as one "pixel" of a compact P8 tensor [1][9 * planes][P / 8][8][8] whose plane order
+// (64-channel chunk, tap, plane) is the K order of the dense 3x3 implicit GEMM: a 1x1 abc_conv_igemm over it with the SAME
+// packed conv1 weights performs, per output element, the same MMA sequence as the dense layer -> identical bits. One warp
+// per slot; in the pooled layout its group comes from a binary search over the offsets (2N + 1 ints, served from L1).
 __global__ void __launch_bounds__(256) gather_patches_kernel(const uint4* __restrict__ trunk, int H, int W, int planes,
                                                             const int32_t* __restrict__ peak_pix, const int32_t* __restrict__ peak_cnt,
-                                                            int cap, uint4* __restrict__ out, int P) {
+                                                            SlotLayout sl, int groups, uint4* __restrict__ out, int P) {
   const int slot = blockIdx.x * 8 + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   if (slot >= P) return;
-  const int g = slot / cap, i = slot - g * cap;
-  if (i >= min(peak_cnt[g], cap)) return;                      // unused slot: keeps its (finite) old contents
+  const int g = slot_group(sl, slot, groups), i = slot - slot_base(sl, g);
+  if (i >= slot_count(sl, g, peak_cnt[g])) return;             // unused slot: keeps its (finite) old contents
   const int n = g >> 1;
-  const int pix = peak_pix[slot];
+  const int pix = peak_pix[static_cast<size_t>(g) * sl.list_stride + i];
   const int y = pix / W, x = pix - y * W;
   const int nq = 9 * planes;
   const size_t rows = static_cast<size_t>(P >> 3);
@@ -490,22 +493,40 @@ __global__ void __launch_bounds__(256) gather_patches_kernel(const uint4* __rest
   }
 }
 
+// Pooled layout: off[g] = exclusive prefix sum of the untruncated counts cnt[0 .. g), off[groups] = total. One CTA; thread t
+// owns a run of consecutive groups, so the slot order is the group order whatever the launch (no atomics).
+__global__ void __launch_bounds__(kDecThreads) peak_offsets_kernel(const int32_t* __restrict__ cnt, int groups, int32_t* __restrict__ off) {
+  __shared__ int warp_sums[33];
+  const int per = (groups + kDecThreads - 1) / kDecThreads;
+  const int b0 = min(static_cast<int>(threadIdx.x) * per, groups), b1 = min(b0 + per, groups);
+  int s = 0;
+  for (int b = b0; b < b1; ++b) s += cnt[b];
+  int total;
+  const int base = block_exscan(s, warp_sums, &total);
+  slot_offsets(cnt + b0, b1 - b0, base, off + b0);
+  if (threadIdx.x == 0) off[groups] = total;
+}
+
+// Fixed layout: at most 1024 slots per group (the documented peak_cap limit).
 constexpr int kMaxPeakCap = 1024;
+// Bond-centre peaks per round of decode_finish_kernel; a group with more peaks (pooled layout) takes several rounds.
+constexpr int kFinishChunk = 1024;
 
 // Step 3: records from the peak lists and the COMPACT class / offset logits (maps[1..3, 5..7] are [1][C][P] or planar-8
-// [1][ceil(C/8)][P][8] with P = N * 2 * peak_cap slots; ldmap is called with n = 0, pix = slot). Same record logic as
-// decode_split_kernel; grid (N, 2).
+// [1][ceil(C/8)][P][8] over the P compact slots; ldmap is called with n = 0, pix = slot). Same record logic as
+// decode_split_kernel; grid (N, 2). Peaks without a slot (beyond peak_cap, or past the pool) are skipped; the counts stay
+// the untruncated ones so that the caller can tell.
 __global__ void __launch_bounds__(kDec2Threads) decode_finish_kernel(const DecParams p) {
   __shared__ int warp_cnt[kDec2Warps];
   __shared__ float wz[kDec2Warps][64];
-  __shared__ uint8_t bcnt[kMaxPeakCap];
-  __shared__ int boff[kMaxPeakCap];
-  const int n = blockIdx.x, bonds = blockIdx.y;
+  __shared__ uint8_t bcnt[kFinishChunk];
+  __shared__ int boff[kFinishChunk];
+  const int n = blockIdx.x, bonds = blockIdx.y, g = n * 2 + bonds;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int raw = p.peak_cnt[n * 2 + bonds];
-  const int cnt = min(raw, p.peak_cap);
-  const int slot0 = (n * 2 + bonds) * p.peak_cap;
-  const int32_t* list = p.peak_pix + slot0;
+  const int raw = p.peak_cnt[g];
+  const int cnt = slot_count(p.slots, g, raw);
+  const int slot0 = slot_base(p.slots, g);
+  const int32_t* list = p.peak_pix + static_cast<size_t>(g) * p.slots.list_stride;
   if (!bonds) {
     for (int i = tid; i < cnt; i += kDec2Threads) {
       if (i >= p.atom_cap) break;
@@ -522,71 +543,77 @@ __global__ void __launch_bounds__(kDec2Threads) decode_finish_kernel(const DecPa
     if (tid == 0) p.counts[n * 4 + 0] = raw;
     return;
   }
-  // pass A: surviving omega bins per bond-centre peak
-  for (int b = warp; b < cnt; b += kDec2Warps) {
-    const int slot = slot0 + b;
-    if (lane < p.n_omega) wz[warp][lane] = ldmap(p, 7, 0, lane, slot, p.n_omega);
-    if (lane + 32 < p.n_omega) wz[warp][lane + 32] = ldmap(p, 7, 0, lane + 32, slot, p.n_omega);
-    __syncwarp();
-    uint32_t slo, shi;
-    omega_survivors(wz[warp], p.n_omega, p.thr_omega, p.omega_mode, &slo, &shi);
-    if (lane == 0) bcnt[b] = static_cast<uint8_t>(__popc(slo) + __popc(shi));
-    __syncwarp();
-  }
-  __syncthreads();
-  // exclusive offsets over the peaks (each thread owns `per` consecutive peaks)
-  const int per = (cnt + kDec2Threads - 1) / kDec2Threads;
-  const int b0 = min(tid * per, cnt), b1 = min(b0 + per, cnt);
-  int c = 0;
-  for (int b = b0; b < b1; ++b) c += bcnt[b];
-  int inc = c;
+  int total_bonds = 0;                                           // records of the earlier rounds (block-uniform)
+  for (int c0 = 0; c0 < cnt; c0 += kFinishChunk) {
+    const int cc = min(cnt - c0, kFinishChunk);
+    // pass A: surviving omega bins per bond-centre peak
+    for (int b = warp; b < cc; b += kDec2Warps) {
+      const int slot = slot0 + c0 + b;
+      if (lane < p.n_omega) wz[warp][lane] = ldmap(p, 7, 0, lane, slot, p.n_omega);
+      if (lane + 32 < p.n_omega) wz[warp][lane + 32] = ldmap(p, 7, 0, lane + 32, slot, p.n_omega);
+      __syncwarp();
+      uint32_t slo, shi;
+      omega_survivors(wz[warp], p.n_omega, p.thr_omega, p.omega_mode, &slo, &shi);
+      if (lane == 0) bcnt[b] = static_cast<uint8_t>(__popc(slo) + __popc(shi));
+      __syncwarp();
+    }
+    __syncthreads();
+    // exclusive offsets over the peaks of this round (each thread owns `per` consecutive peaks)
+    const int per = (cc + kDec2Threads - 1) / kDec2Threads;
+    const int b0 = min(tid * per, cc), b1 = min(b0 + per, cc);
+    int c = 0;
+    for (int b = b0; b < b1; ++b) c += bcnt[b];
+    int inc = c;
 #pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    const int t = __shfl_up_sync(0xffffffffu, inc, o);
-    if (lane >= o) inc += t;
-  }
-  if (lane == 31) warp_cnt[warp] = inc;
-  __syncthreads();
-  int woff = 0, total_bonds = 0;
-  for (int w = 0; w < kDec2Warps; ++w) {
-    const int v = warp_cnt[w];
-    if (w < warp) woff += v;
-    total_bonds += v;
-  }
-  int off = woff + inc - c;
-  for (int b = b0; b < b1; ++b) {
-    boff[b] = off;
-    off += bcnt[b];
-  }
-  __syncthreads();
-  // pass B: emit
-  for (int b = warp; b < cnt; b += kDec2Warps) {
-    if (bcnt[b] == 0) continue;
-    const int slot = slot0 + b, pix = list[b];
-    if (lane < p.n_omega) wz[warp][lane] = ldmap(p, 7, 0, lane, slot, p.n_omega);
-    if (lane + 32 < p.n_omega) wz[warp][lane + 32] = ldmap(p, 7, 0, lane + 32, slot, p.n_omega);
-    __syncwarp();
-    uint32_t slo, shi;
-    omega_survivors(wz[warp], p.n_omega, p.thr_omega, p.omega_mode, &slo, &shi);
+    for (int o = 1; o < 32; o <<= 1) {
+      const int t = __shfl_up_sync(0xffffffffu, inc, o);
+      if (lane >= o) inc += t;
+    }
+    if (lane == 31) warp_cnt[warp] = inc;
+    __syncthreads();
+    int woff = 0, round_bonds = 0;
+    for (int w = 0; w < kDec2Warps; ++w) {
+      const int v = warp_cnt[w];
+      if (w < warp) woff += v;
+      round_bonds += v;
+    }
+    int off = total_bonds + woff + inc - c;
+    for (int b = b0; b < b1; ++b) {
+      boff[b] = off;
+      off += bcnt[b];
+    }
+    __syncthreads();
+    // pass B: emit
+    for (int b = warp; b < cc; b += kDec2Warps) {
+      if (bcnt[b] == 0) continue;
+      const int slot = slot0 + c0 + b, pix = list[c0 + b];
+      if (lane < p.n_omega) wz[warp][lane] = ldmap(p, 7, 0, lane, slot, p.n_omega);
+      if (lane + 32 < p.n_omega) wz[warp][lane + 32] = ldmap(p, 7, 0, lane + 32, slot, p.n_omega);
+      __syncwarp();
+      uint32_t slo, shi;
+      omega_survivors(wz[warp], p.n_omega, p.thr_omega, p.omega_mode, &slo, &shi);
 #pragma unroll
-    for (int h = 0; h < 2; ++h) {
-      const uint32_t mine = h == 0 ? slo : shi;
-      if ((mine >> lane) & 1u) {
-        const int w = lane + 32 * h;
-        const int o = boff[b] + __popc(mine & ((1u << lane) - 1u)) + (h == 1 ? __popc(slo) : 0);
-        if (o < p.bond_cap) {
-          AbcBondRec r;
-          r.x = static_cast<uint16_t>(pix / p.W);
-          r.y = static_cast<uint16_t>(pix % p.W);
-          r.omega = static_cast<uint8_t>(w);
-          r.type = static_cast<uint8_t>(argmax_map(p, 5, 0, w, p.n_omega, p.n_btype, p.n_btype * p.n_omega, slot));
-          r.pad = 0;
-          r.rho = fabsf(ldmap(p, 6, 0, w, slot, p.n_omega));
-          p.bonds[static_cast<size_t>(n) * p.bond_cap + o] = r;
+      for (int h = 0; h < 2; ++h) {
+        const uint32_t mine = h == 0 ? slo : shi;
+        if ((mine >> lane) & 1u) {
+          const int w = lane + 32 * h;
+          const int o = boff[b] + __popc(mine & ((1u << lane) - 1u)) + (h == 1 ? __popc(slo) : 0);
+          if (o < p.bond_cap) {
+            AbcBondRec r;
+            r.x = static_cast<uint16_t>(pix / p.W);
+            r.y = static_cast<uint16_t>(pix % p.W);
+            r.omega = static_cast<uint8_t>(w);
+            r.type = static_cast<uint8_t>(argmax_map(p, 5, 0, w, p.n_omega, p.n_btype, p.n_btype * p.n_omega, slot));
+            r.pad = 0;
+            r.rho = fabsf(ldmap(p, 6, 0, w, slot, p.n_omega));
+            p.bonds[static_cast<size_t>(n) * p.bond_cap + o] = r;
+          }
         }
       }
+      __syncwarp();
     }
-    __syncwarp();
+    total_bonds += round_bonds;
+    __syncthreads();                                             // bcnt / boff / warp_cnt are rewritten by the next round
   }
   if (tid == 0) {
     p.counts[n * 4 + 1] = total_bonds;
@@ -597,18 +624,37 @@ __global__ void __launch_bounds__(kDec2Threads) decode_finish_kernel(const DecPa
 
 }  // namespace abc
 
+namespace {
+int gather_patches(const void* trunk, int N, int H, int W, int planes, const int32_t* peak_pix, const int32_t* peak_cnt,
+                   const abc::SlotLayout& sl, long long P, void* out, void* stream, const char* what) {
+  using namespace abc;
+  ABC_REQUIRE(trunk && peak_pix && peak_cnt && out, "%s: null pointer", what);
+  ABC_REQUIRE(N > 0 && H > 0 && W > 0 && planes > 0 && planes % 8 == 0, "%s: planes=%d must be a multiple of 8 (64-channel chunks)", what, planes);
+  ABC_REQUIRE(P < (1LL << 30), "%s: too many slots", what);
+  gather_patches_kernel<<<static_cast<int>((P + 7) / 8), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      static_cast<const uint4*>(trunk), H, W, planes, peak_pix, peak_cnt, sl, 2 * N, static_cast<uint4*>(out), static_cast<int>(P));
+  return launch_check("gather_patches_kernel");
+}
+}  // namespace
+
 extern "C" int abc_gather_patches(const void* trunk, int N, int H, int W, int planes, const int32_t* peak_pix, const int32_t* peak_cnt,
                                   int peak_cap, void* out, void* stream) {
   using namespace abc;
   if (int rc = device_check()) return rc;
-  ABC_REQUIRE(trunk && peak_pix && peak_cnt && out, "abc_gather_patches: null pointer");
-  ABC_REQUIRE(N > 0 && H > 0 && W > 0 && planes > 0 && planes % 8 == 0, "abc_gather_patches: planes=%d must be a multiple of 8 (64-channel chunks)", planes);
   ABC_REQUIRE(peak_cap >= 64 && peak_cap % 64 == 0 && peak_cap <= kMaxPeakCap, "abc_gather_patches: peak_cap=%d (multiple of 64, <= %d)", peak_cap, kMaxPeakCap);
-  const long long P = 2LL * N * peak_cap;
-  ABC_REQUIRE(P < (1LL << 30), "abc_gather_patches: too many slots");
-  gather_patches_kernel<<<static_cast<int>((P + 7) / 8), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-      static_cast<const uint4*>(trunk), H, W, planes, peak_pix, peak_cnt, peak_cap, static_cast<uint4*>(out), static_cast<int>(P));
-  return launch_check("gather_patches_kernel");
+  const SlotLayout sl{nullptr, peak_cap, 0, peak_cap};
+  return gather_patches(trunk, N, H, W, planes, peak_pix, peak_cnt, sl, 2LL * N * peak_cap, out, stream, "abc_gather_patches");
+}
+
+extern "C" int abc_gather_patches_pooled(const void* trunk, int N, int H, int W, int planes, const int32_t* peak_pix,
+                                         const int32_t* peak_cnt, const int32_t* peak_off, int pool_slots, void* out, void* stream) {
+  using namespace abc;
+  if (int rc = device_check()) return rc;
+  ABC_REQUIRE(peak_off != nullptr, "abc_gather_patches_pooled: null peak_off");
+  ABC_REQUIRE(pool_slots >= 64 && pool_slots % 64 == 0, "abc_gather_patches_pooled: pool_slots=%d (positive multiple of 64)", pool_slots);
+  ABC_REQUIRE(2LL * N * H * W < (1LL << 31), "abc_gather_patches_pooled: 2 * N * H * W peak-list entries exceed the int32 range");
+  const SlotLayout sl{peak_off, 0, pool_slots, H * W};
+  return gather_patches(trunk, N, H, W, planes, peak_pix, peak_cnt, sl, pool_slots, out, stream, "abc_gather_patches_pooled");
 }
 
 extern "C" int abc_decode_peaks(const AbcDecodeDesc* d, void* stream) {
@@ -623,9 +669,15 @@ extern "C" int abc_decode_peaks(const AbcDecodeDesc* d, void* stream) {
     ABC_REQUIRE(!needed || d->maps[i] != nullptr, "abc_decode_peaks: map %d is null", i);
   }
   ABC_REQUIRE(mode == 1 || (d->atoms && d->bonds && d->counts), "abc_decode_peaks: null output");
-  if (mode != 0)
+  const bool pooled = mode != 0 && d->pool_slots != 0;
+  if (mode != 0 && !pooled)
     ABC_REQUIRE(d->peak_pix && d->peak_cnt && d->peak_cap >= 64 && d->peak_cap % 64 == 0 && d->peak_cap <= kMaxPeakCap,
                 "abc_decode_peaks: sparse modes need peak_pix / peak_cnt and peak_cap (multiple of 64, <= %d)", kMaxPeakCap);
+  if (pooled)
+    ABC_REQUIRE(d->peak_pix && d->peak_cnt && d->peak_off && d->pool_slots >= 64 && d->pool_slots % 64 == 0 &&
+                    d->pool_slots < (1 << 30) && 2LL * d->N * d->H * d->W < (1LL << 31),
+                "abc_decode_peaks: the pooled layout needs peak_pix / peak_cnt / peak_off, pool_slots=%d (positive multiple of 64, "
+                "< 2^30) and 2 * N * H * W < 2^31", d->pool_slots);
   ABC_REQUIRE(d->N > 0 && d->H > 0 && d->W > 0, "abc_decode_peaks: bad geometry");
   ABC_REQUIRE(static_cast<int64_t>(d->H) * d->W <= 32768 && d->H <= 65535 && d->W <= 65535,
               "abc_decode_peaks: H*W=%lld exceeds the 32768-pixel per-image limit of the shared-memory decoder",
@@ -645,8 +697,9 @@ extern "C" int abc_decode_peaks(const AbcDecodeDesc* d, void* stream) {
   p.centre_prob = d->centre_prob ? 1 : 0;
   p.thr_omega = p.centre_prob ? d->thr_omega : d->thr;
   p.atoms = d->atoms; p.atom_cap = d->atom_cap; p.bonds = d->bonds; p.bond_cap = d->bond_cap; p.counts = d->counts;
-  p.peak_pix = d->peak_pix; p.peak_cnt = d->peak_cnt; p.peak_cap = d->peak_cap; p.mode = mode;
-  p.hw_gather = mode == 2 ? 2 * d->N * d->peak_cap : d->H * d->W;
+  p.peak_pix = d->peak_pix; p.peak_cnt = d->peak_cnt; p.mode = mode;
+  p.slots = pooled ? SlotLayout{d->peak_off, 0, d->pool_slots, d->H * d->W} : SlotLayout{nullptr, d->peak_cap, 0, d->peak_cap};
+  p.hw_gather = mode != 2 ? d->H * d->W : pooled ? d->pool_slots : 2 * d->N * d->peak_cap;
   if (mode == 2) {
     decode_finish_kernel<<<dim3(d->N, 2, 1), kDec2Threads, 0, static_cast<cudaStream_t>(stream)>>>(p);
     return launch_check("decode_finish_kernel");
@@ -660,7 +713,10 @@ extern "C" int abc_decode_peaks(const AbcDecodeDesc* d, void* stream) {
       smem2_set = smem2;
     }
     decode_split_kernel<<<dim3(d->N, 2, 1), kDec2Threads, smem2, static_cast<cudaStream_t>(stream)>>>(p);
-    return launch_check("decode_split_kernel");
+    if (int rc = launch_check("decode_split_kernel")) return rc;
+    if (!pooled) return ABC_OK;
+    peak_offsets_kernel<<<1, kDecThreads, 0, static_cast<cudaStream_t>(stream)>>>(d->peak_cnt, 2 * d->N, d->peak_off);
+    return launch_check("peak_offsets_kernel");
   }
   const size_t smem = static_cast<size_t>(d->H) * d->W * 7;       // 4 B map + 2 B pixel list + 1 B survivor counts
   static size_t smem_set = 0;

@@ -90,15 +90,19 @@ class PeakDecoder:
         self._done.record(torch.cuda.current_stream())
         return N
 
+    def wait_copy(self):
+        """Wait for the copy enqueued by ``fetch_async``; no capacity check (``h_counts`` is then valid)."""
+        self._done.synchronize()
+
     def collect(self, N):
         """Wait for the copy enqueued by ``fetch_async`` and return per-image numpy record arrays."""
-        self._done.synchronize()
+        self.wait_copy()
         return self._parse(N)
 
     def wait(self, N):
         """Wait for the copy enqueued by ``fetch_async`` and check the capacities, without building per-image arrays (for
         callers that go straight to ``molblocks``). Returns the [N, 4] counts."""
-        self._done.synchronize()
+        self.wait_copy()
         counts = self.h_counts[:N].numpy()
         if (counts[:, 0] > self.atom_cap).any() or (counts[:, 1] > self.bond_cap).any():
             raise RuntimeError(f"decode capacity exceeded: max atoms {counts[:, 0].max()} (cap {self.atom_cap}), "

@@ -29,24 +29,44 @@ _CLASS_HEADS = (1, 2, 3, 5, 6, 7)
 
 
 class SparseHeadsPipeline:
-    """pipe = SparseHeadsPipeline(model, batch, peak_cap=128, bond_cap=2048)
-    n = pipe.launch(x)            # enqueue everything on the current stream (no synchronisation)
+    """pipe = SparseHeadsPipeline(model, batch, peak_cap=128, bond_cap=2048, peak_pool=None, atom_cap=None)
+    n = pipe.launch(x)            # enqueue everything on the current stream (no synchronisation); x holds 1 .. batch images
     recs = pipe.fetch(n)          # same per-image (atoms, bonds, n_bond_peaks) records as PeakDecoder.fetch
 
-    ``peak_cap``: slots per image and peak kind (multiple of 64, <= 1024). An image with more atom or bond-centre peaks
-    than that makes ``fetch`` raise (the dense path has no such limit)."""
+    Slot layouts of the compact tensors the class / offset heads run on:
 
-    def __init__(self, model, batch, peak_cap=128, bond_cap=2048, device=None):
+    * ``peak_pool=None`` (fixed): ``peak_cap`` slots per image and peak kind (multiple of 64, <= 1024). An image with more
+      atom or bond-centre peaks than that makes ``fetch`` raise (the dense path has no such limit).
+    * ``peak_pool=S`` (pooled, a multiple of 64): the batch shares S slots, handed out on the device in image order. An image
+      may have any number of peaks; ``fetch`` / ``collect`` / ``wait`` raise only when the batch's atom plus bond-centre
+      peaks exceed S. The per-step work is that of S slots whatever the peaks, so S = 2 * batch * peak_cap costs what the
+      fixed layout costs. ``peak_cap`` is not used.
+
+    ``atom_cap`` sizes the atom record arrays: ``peak_cap`` by default in the fixed layout, 1024 in the pooled one."""
+
+    def __init__(self, model, batch, peak_cap=128, bond_cap=2048, device=None, peak_pool=None, atom_cap=None):
         if list(model.heads) != V2_HEADS:
             raise NotImplementedError("SparseHeadsPipeline: the v2 head list [1, 14, 3, 2, 1, 360, 60, 60] only")
-        if peak_cap % 64 or not (64 <= peak_cap <= 1024):
-            raise ValueError("peak_cap must be a multiple of 64 in [64, 1024]")
-        self.m, self.batch, self.cap = model, batch, peak_cap
+        if peak_pool is None:
+            if peak_cap % 64 or not (64 <= peak_cap <= 1024):
+                raise ValueError("peak_cap must be a multiple of 64 in [64, 1024]")
+            P = 2 * batch * peak_cap
+        else:
+            if peak_pool % 64 or not (64 <= peak_pool < 1 << 30):
+                raise ValueError("peak_pool must be a positive multiple of 64 (below 2^30)")
+            P = peak_pool
+        self.m, self.batch, self.cap, self.pool = model, batch, peak_cap, peak_pool
         self.dev = device or model.s.device
-        self.dec = PeakDecoder(batch, atom_cap=peak_cap, bond_cap=bond_cap, device=self.dev)
-        self.P = 2 * batch * peak_cap
+        if atom_cap is None:
+            atom_cap = peak_cap if peak_pool is None else 1024
+        self.dec = PeakDecoder(batch, atom_cap=atom_cap, bond_cap=bond_cap, device=self.dev)
+        self.P = P
         dev = self.dev
-        self.peak_pix = torch.zeros((batch, 2, peak_cap), dtype=torch.int32, device=dev)
+        if peak_pool is None:
+            self.peak_pix = torch.zeros((batch, 2, peak_cap), dtype=torch.int32, device=dev)
+        else:
+            self.peak_pix = None                                          # untruncated lists [batch][2][H * W], sized at launch
+            self.peak_off = torch.zeros(2 * batch + 1, dtype=torch.int32, device=dev)
         self.peak_cnt = torch.zeros((batch, 2), dtype=torch.int32, device=dev)
         rows = self.P // 8
         adt = model._act_torch_dtype                                                              # 16-bit storage format of the model
@@ -69,8 +89,8 @@ class SparseHeadsPipeline:
         m = self.m
         k2 = m.trunk(x)                                                  # also (re)packs the weights when they changed
         B, _, H4, W4, _ = k2.shape
-        if B != self.batch:
-            raise ValueError(f"SparseHeadsPipeline was built for batches of {self.batch} images, got {B}")
+        if not 1 <= B <= self.batch:
+            raise ValueError(f"SparseHeadsPipeline was built for batches of up to {self.batch} images, got {B}")
         st = _lib.current_stream_ptr()
         P_ = m._packed
         if self._centre_pack is None or self._centre_key != m._pack_gen:
@@ -86,22 +106,32 @@ class SparseHeadsPipeline:
         zb = self._buf("zb", (B, 1, H4, W4), torch.float32)
         m._conv(P_["heads.0.conv2"], hid2, 0, za, act=0, out_mode=1, stream=st)
         m._conv(P_["heads.4.conv2"], hid2, 16, zb, act=0, out_mode=1, stream=st)
-        # peak lists
-        d = self._desc(B, H4, W4, thr, omega_mode, apply_sigmoid, thr_omega)
+        # peak lists (pooled: untruncated, plus the slot offsets of every image and peak kind)
+        if self.pool is None:
+            plist, P = self.peak_pix, 2 * B * self.cap
+        else:
+            plist, P = self._buf("plist", (self.batch, 2, H4 * W4), torch.int32), self.pool
+        d = self._desc(B, H4, W4, thr, omega_mode, apply_sigmoid, thr_omega, plist)
         d.maps[0], d.maps[4] = za.data_ptr(), zb.data_ptr()
         d.sparse_mode = 1
         check(lib.abc_decode_peaks(C.byref(d), st), "abc_decode_peaks[find]")
         # 3x3 trunk patches of the peaks -> compact K-ordered tensor -> conv1 (all heads' weights, same pack as the dense layer)
-        check(lib.abc_gather_patches(k2.data_ptr(), B, H4, W4, 16, self.peak_pix.data_ptr(), self.peak_cnt.data_ptr(), self.cap,
-                                     self.patches.data_ptr(), st), "abc_gather_patches")
+        patches = _slots(self.patches, P)
+        if self.pool is None:
+            check(lib.abc_gather_patches(k2.data_ptr(), B, H4, W4, 16, plist.data_ptr(), self.peak_cnt.data_ptr(), self.cap,
+                                         patches.data_ptr(), st), "abc_gather_patches")
+        else:
+            check(lib.abc_gather_patches_pooled(k2.data_ptr(), B, H4, W4, 16, plist.data_ptr(), self.peak_cnt.data_ptr(),
+                                                self.peak_off.data_ptr(), self.pool, patches.data_ptr(), st), "abc_gather_patches_pooled")
         pk1 = P_["heads.conv1"]
         if pk1.pair:
             raise RuntimeError("SparseHeadsPipeline does not support the CTA-pair weight pack (ABCNET_PAIR=1)")
-        self._conv1x1_k(pk1, self.patches, self.hid_c, st)
+        hid_c = _slots(self.hid_c, P)
+        self._conv1x1_k(pk1, patches, hid_c, st)
         for k in _CLASS_HEADS:
-            m._conv(P_[f"heads.{k}.conv2"], self.hid_c, 16 * k, self.logits_c[k], act=0, out_mode=2, stream=st)
+            m._conv(P_[f"heads.{k}.conv2"], hid_c, 16 * k, _slots(self.logits_c[k], P), act=0, out_mode=2, stream=st)
         # records
-        d = self._desc(B, H4, W4, thr, omega_mode, apply_sigmoid, thr_omega)
+        d = self._desc(B, H4, W4, thr, omega_mode, apply_sigmoid, thr_omega, plist)
         for k in _CLASS_HEADS:
             d.maps[k] = self.logits_c[k].data_ptr()
         d.p8f_mask = sum(1 << k for k in _CLASS_HEADS)
@@ -114,7 +144,7 @@ class SparseHeadsPipeline:
         view = _PackView(pk)
         self.m._conv(view, src, 0, dst, act=2, stream=st)
 
-    def _desc(self, B, H4, W4, thr, omega_mode, apply_sigmoid=False, thr_omega=-1.0):
+    def _desc(self, B, H4, W4, thr, omega_mode, apply_sigmoid, thr_omega, plist):
         d = AbcDecodeDesc()
         d.N, d.H, d.W = B, H4, W4
         d.c_type, d.c_charge, d.c_hs, d.n_omega, d.n_btype = 14, 3, 2, 60, 6
@@ -124,34 +154,51 @@ class SparseHeadsPipeline:
         d.atoms, d.atom_cap = self.dec.d_atoms.data_ptr(), self.dec.atom_cap
         d.bonds, d.bond_cap = self.dec.d_bonds.data_ptr(), self.dec.bond_cap
         d.counts = self.dec.d_counts.data_ptr()
-        d.peak_pix, d.peak_cnt, d.peak_cap = self.peak_pix.data_ptr(), self.peak_cnt.data_ptr(), self.cap
+        d.peak_pix, d.peak_cnt, d.peak_cap = plist.data_ptr(), self.peak_cnt.data_ptr(), self.cap
+        if self.pool is not None:
+            d.peak_off, d.pool_slots = self.peak_off.data_ptr(), self.pool
         return d
 
-    def fetch(self, N):
-        recs = self.dec.fetch(N)                                         # raises when a count exceeds peak_cap / bond_cap
+    def _check_slots(self, N):
+        """Every peak of the batch had a slot, so the records are complete (from the counts already copied back): in the
+        fixed layout no image has more than peak_cap atom or bond-centre peaks, in the pooled one the batch fits the pool.
+        Checked before the record capacities, which may be larger than peak_cap."""
         counts = self.dec.h_counts[:N].numpy()
-        if (counts[:, 2] > self.cap).any():
-            raise RuntimeError(f"sparse heads: {int(counts[:, 2].max())} bond-centre peaks in one image exceed peak_cap {self.cap}; "
-                               "use a larger peak_cap or the dense path")
-        return recs
+        if self.pool is None:
+            for col, kind in ((2, "bond-centre"), (0, "atom")):
+                if (counts[:, col] > self.cap).any():
+                    raise RuntimeError(f"sparse heads: {int(counts[:, col].max())} {kind} peaks in one image exceed peak_cap "
+                                       f"{self.cap}; use a larger peak_cap, a peak_pool or the dense path")
+            return
+        total = int(counts[:, 0].sum(dtype="int64") + counts[:, 2].sum(dtype="int64"))
+        if total > self.pool:
+            raise RuntimeError(f"sparse heads: {total} atom + bond-centre peaks in the batch exceed peak_pool {self.pool}; "
+                               "use a larger peak_pool or the dense path")
+
+    def fetch(self, N):
+        self.dec.fetch_async(N)
+        return self.collect(N)
 
     def fetch_async(self, N):
         return self.dec.fetch_async(N)
 
     def collect(self, N):
-        recs = self.dec.collect(N)
-        if (self.dec.h_counts[:N, 2] > self.cap).any():
-            raise RuntimeError("sparse heads: bond-centre peaks exceed peak_cap; use a larger peak_cap or the dense path")
-        return recs
+        self.dec.wait_copy()
+        self._check_slots(N)
+        return self.dec.collect(N)                                       # raises when a count exceeds atom_cap / bond_cap
 
     def wait(self, N):
-        counts = self.dec.wait(N)
-        if (counts[:, 2] > self.cap).any():
-            raise RuntimeError("sparse heads: bond-centre peaks exceed peak_cap; use a larger peak_cap or the dense path")
-        return counts
+        self.dec.wait_copy()
+        self._check_slots(N)
+        return self.dec.wait(N)
 
     def molblocks(self, N, n_threads=0):
         return self.dec.molblocks(N, n_threads)
+
+
+def _slots(t, P):
+    """The first P slots of a compact tensor [1][planes][rows][8][8]: the layout a convolution over P slots reads / writes."""
+    return t.view(-1)[: t.shape[1] * P * 8].view(1, t.shape[1], P // 8, 8, 8)
 
 
 class _PackView:

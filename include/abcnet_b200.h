@@ -263,11 +263,22 @@ typedef struct AbcDecodeDesc {
    *   sparse_mode 2 ("finish"): maps[1..3] and maps[5..7] are COMPACT logits over the slots -- [1][C][P] fp32, or planar-8
    *                             [1][ceil(C/8)][P][8] where p8f_mask says so -- as produced by running the heads on the
    *                             output of abc_gather_patches; records and counts as in mode 0 (counts[0] / counts[2] are
-   *                             the untruncated peak counts: the caller checks them against peak_cap). */
+   *                             the untruncated peak counts: the caller checks them against peak_cap).
+   * Pooled slot layout (pool_slots > 0; peak_cap is then ignored): the whole batch shares one pool of P = pool_slots slots.
+   * Slot s = peak_off[n * 2 + which] + i is peak i of image n, where peak_off[2N + 1] holds the exclusive prefix sums of the
+   * untruncated counts peak_cnt[N][2] in (n, which) order and peak_off[2N] is their total. An image may have any number of
+   * peaks; a peak whose slot would be >= pool_slots gets none, so the records are complete exactly when the total
+   * (counts[0] + counts[2] summed over the batch) is <= pool_slots.
+   *   sparse_mode 1 writes the UNTRUNCATED lists peak_pix[N][2][H * W], peak_cnt and peak_off (a deterministic scan,
+   *                 no atomics: the same counts always give the same slots);
+   *   sparse_mode 2 reads the slots through peak_off; the compact logits are [1][C][pool_slots] (or planar-8), as produced
+   *                 from the output of abc_gather_patches_pooled. */
   int32_t* peak_pix;
   int32_t* peak_cnt;
   int peak_cap;            /* multiple of 64, <= 1024 */
   int sparse_mode;
+  int32_t* peak_off;       /* pooled layout: [2N + 1] slot offsets (written by sparse_mode 1, read by sparse_mode 2) */
+  int pool_slots;          /* 0: the fixed layout above; > 0: the pooled layout, a multiple of 64 (2 * N * H * W < 2^31) */
 } AbcDecodeDesc;
 ABC_API int abc_decode_peaks(const AbcDecodeDesc* desc, void* stream);
 /* Sparse heads, step 2: for every valid slot the 3x3 neighbourhood of the trunk (P8 bf16 [N][planes][H][W][8], zero outside the
@@ -276,6 +287,11 @@ ABC_API int abc_decode_peaks(const AbcDecodeDesc* desc, void* stream);
  * with the packed weights of the dense 3x3 layer then reproduces that layer's outputs at the peaks bit for bit. */
 ABC_API int abc_gather_patches(const void* trunk, int N, int H, int W, int planes, const int32_t* peak_pix, const int32_t* peak_cnt,
                                int peak_cap, void* out, void* stream);
+/* The same gather in the pooled slot layout (AbcDecodeDesc.pool_slots): peak_pix [N][2][H * W], peak_cnt [N][2] and peak_off
+ * [2N + 1] as written by sparse_mode 1, out = [1][9 * planes][pool_slots / 8][8][8]. Slots past the batch's total keep their
+ * old contents; no slot at or past pool_slots is written. */
+ABC_API int abc_gather_patches_pooled(const void* trunk, int N, int H, int W, int planes, const int32_t* peak_pix,
+                                      const int32_t* peak_cnt, const int32_t* peak_off, int pool_slots, void* out, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------
  * Host-side assembly of the decoded records into V2000 MOL-block text (HOST memory in, HOST memory out, no GPU work):
