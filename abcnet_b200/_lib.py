@@ -88,8 +88,8 @@ class AbcHeadsFusedDesc(C.Structure):
         ("in_", C.c_void_p), ("N", C.c_int), ("H", C.c_int), ("W", C.c_int), ("in_planes", C.c_int), ("in_plane_off", C.c_int),
         ("w1pack", C.c_void_p), ("bias1", C.c_void_p), ("n_heads", C.c_int), ("cout", C.c_int * 16),
         ("w2pack", C.c_void_p), ("w2pack_bytes", C.c_int64), ("bias2", C.c_void_p), ("bias2_len", C.c_int),
-        ("out", C.c_void_p * 16), ("out_mode", C.c_int * 16), ("out_planes", C.c_int * 16), ("item_slot", C.c_int * 6),
-        ("act_fp16", C.c_int),
+        ("out", C.c_void_p * 16), ("out_mode", C.c_int * 16), ("out_planes", C.c_int * 16),
+        ("act_fp16", C.c_int), ("trace", C.c_void_p),
     ]
 
 

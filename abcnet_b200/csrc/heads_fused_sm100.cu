@@ -6,8 +6,8 @@
 //           N = 256 = TWO heads per CTA, K = 2 chunks x 9 taps x 64 channels), accumulators in TMEM;
 //   epilogue phase 1 : TMEM -> registers -> bias + LeakyReLU -> 16-bit -> back to TMEM (tcgen05.st), two values per
 //           32-bit column, lane = pixel: the A-operand layout of tcgen05.mma kind::f16 with A in tensor memory;
-//   conv2 : 8 MMAs per chunk of <= 128 output channels (A = hidden map from TMEM, B = the head's 1x1 weights streamed
-//           through the conv1 weight ring), accumulating into the TMEM columns phase 1 has just drained;
+//   conv2 : 8 MMAs per chunk of <= 128 output channels (A = hidden map from TMEM, B = the head's 1x1 weights, one chunk
+//           at a time in a shared-memory slot of their own), accumulating into the TMEM columns phase 1 has just drained;
 //   epilogue phase 2 : TMEM -> + bias -> fp32 logits (NCHW, or planar-8 for the fused inference + decode path).
 //
 // TMEM: two buffers of 256 columns (tile t uses buffer t & 1). In buffer b, conv1 accumulates head A in columns [0, 128) and
@@ -15,14 +15,15 @@
 // after another in [128, 256). The buffer returns to conv1 (tile t + 2) once its last chunk is drained.
 //
 // Compared with conv_igemm(conv1) + 8 x conv_igemm(conv2) this removes the write and re-read of the hidden maps
-// (2 x 8.6 GB per 256-image batch) and nine launches. The conv2 MMAs of tile t are issued by the MMA warp in the middle
-// of the conv1 MMAs of tile t + 1 (after a host-chosen "slot" of the 18 (chunk, tap) steps), so the tensor pipe never
-// waits for the epilogue. The hidden maps take no shared memory, so the weight ring is as deep as the stand-alone conv1's.
+// (2 x 8.6 GB per 256-image batch) and nine launches. conv1 and conv2 have an issuing warp each, so the conv1 MMA stream
+// waits on the epilogue only for a free TMEM buffer (the one of tile t - 2), never for a logit drain: each conv2 chunk
+// waits for the drain of the one before, and with one issuer that wait stalled conv1 too. The hidden maps take no shared
+// memory, which leaves room for a 4-block conv1 weight ring next to the conv2 slot.
 //
 // Warp roles (384 threads, 1 CTA / SM, persistent over M tiles; the CTAs are split among the head pairs by
 // hf_split_ctas in heads_split.cuh):
-//   warp 0 : TMA producer (activation halo tiles)      warp 3 : bulk-copy producer (conv1 + conv2 weight blocks)
-//   warp 1 : MMA issuer                                warp 2 : TMEM allocation
+//   warp 0 : TMA producer (activation halo tiles)      warp 3 : bulk-copy producer (conv1 weight blocks)
+//   warp 1 : conv1 MMA issuer                          warp 2 : TMEM allocation, then conv2 weight loads + MMA issuer
 //   warps 4-11 : epilogue (two per TMEM lane quarter)
 #include <cuda.h>
 #include <cuda_bf16.h>
@@ -40,9 +41,10 @@ constexpr uint32_t kHfHeader = 4096;
 constexpr uint32_t kHfARow = 10 * 16, kHfAPlane = 18 * kHfARow, kHfAStage = 8 * kHfAPlane;   // 64 channels = 8 planes
 constexpr uint32_t kHfBBlock = 256 * 64 * 2;
 constexpr uint32_t kHfSmemLimit = 232448;
+constexpr uint32_t kHfW2Slot = 128 * 16 * 8 * 2;   // one conv2 chunk: [16 K planes][<= 128 channels][8] 16-bit
 constexpr int kHfNA = 2;
-constexpr int kHfNB = static_cast<int>((kHfSmemLimit - kHfHeader - kHfNA * kHfAStage) / kHfBBlock);   // 5 weight blocks
-constexpr uint32_t kHfSmem = kHfHeader + kHfNA * kHfAStage + kHfNB * kHfBBlock;
+constexpr int kHfNB = static_cast<int>((kHfSmemLimit - kHfHeader - kHfNA * kHfAStage - kHfW2Slot) / kHfBBlock);   // 4 conv1 blocks
+constexpr uint32_t kHfSmem = kHfHeader + kHfNA * kHfAStage + kHfNB * kHfBBlock + kHfW2Slot;
 static_assert(kHfSmem <= kHfSmemLimit, "shared memory budget");
 
 struct HfItem {          // one conv2 chunk: <= 128 output channels of one head
@@ -51,7 +53,6 @@ struct HfItem {          // one conv2 chunk: <= 128 output channels of one head
   int ch0;               // first output channel of the head covered by this chunk
   int w2_off;            // byte offset of the packed [16][nc][8] 16-bit weight block in w2
   int bias_off;          // offset (floats) of the chunk's bias in the pair's bias2 block
-  int slot;              // issued after this (chunk, tap) step of the NEXT tile's conv1 (0..17)
 };
 
 struct HfParams {
@@ -70,10 +71,38 @@ struct HfParams {
   int cout[2 * kHfMaxPairs];
   int out_planes[2 * kHfMaxPairs];
   uint32_t tap16[9];
+  unsigned long long* trace;       // kHfTraceWords per CTA (kTrace instantiation only)
 };
 
-// kF16: activations and weights are IEEE fp16 (UNet(act_dtype="fp16")), else bf16
-template <bool kF16>
+// Per-CTA timeline record of the kTrace instantiation (tools/heads_trace.py reads it): clock64 cycles spent in each wait.
+enum HfTraceWord {
+  kHtPair, kHtTiles, kHtStartNs, kHtEndNs, kHtCycles,
+  kHtC1BFull, kHtC1AFull, kHtC1AccEmpty,                    // conv1 issuer
+  kHtC2HidFull, kHtC2C2Empty, kHtC2WFull, kHtC2WEmpty,      // conv2 issuer
+  kHtEpAccFull, kHtEpPhase1, kHtEpC2Full, kHtEpPhase2,      // epilogue warp 4: waits and busy cycles of the two phases
+  kHfTraceWords
+};
+
+__device__ __forceinline__ unsigned long long global_ns() {
+  unsigned long long t;
+  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+  return t;
+}
+
+// mbar_wait that, in the kTrace instantiation, adds the cycles it waited to `acc`
+template <bool kTrace>
+__device__ __forceinline__ void mbar_wait_t(uint32_t bar, uint32_t parity, unsigned long long& acc) {
+  if constexpr (kTrace) {
+    const long long t0 = clock64();
+    mbar_wait(bar, parity);
+    acc += static_cast<unsigned long long>(clock64() - t0);
+  } else {
+    mbar_wait(bar, parity);
+  }
+}
+
+// kF16: activations and weights are IEEE fp16 (UNet(act_dtype="fp16")), else bf16. kTrace: write p.trace (HfTraceWord)
+template <bool kF16, bool kTrace>
 __global__ void __launch_bounds__(kHfThreads, 1)
 heads_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ HfParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -92,6 +121,8 @@ heads_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
   const uint32_t bar_hid_full = bar_acc_empty + 16;            // both hidden operands of a tile written to TMEM
   const uint32_t bar_c2_full = bar_hid_full + 8;               // a conv2 chunk is complete in TMEM
   const uint32_t bar_c2_empty = bar_c2_full + 8;               // ... and has been drained
+  const uint32_t bar_w2_full = bar_c2_empty + 8;               // a conv2 chunk's weights are in the conv2 slot
+  const uint32_t bar_w2_empty = bar_w2_full + 8;               // ... and its MMAs have read them
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + 512);
   HfItem* items_s = reinterpret_cast<HfItem*>(smem + 576);     // [kHfMaxItems]
   float* bias1_s = reinterpret_cast<float*>(smem + 1024);      // [256]
@@ -114,6 +145,8 @@ heads_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
     mbar_init(bar_hid_full, 8);
     mbar_init(bar_c2_full, 1);
     mbar_init(bar_c2_empty, 8);
+    mbar_init(bar_w2_full, 1);
+    mbar_init(bar_w2_empty, 1);
     fence_mbar_init();
     tma_prefetch_desc(&tmap);
   }
@@ -125,9 +158,17 @@ heads_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(tmem_slot);
+  unsigned long long* const trace = kTrace ? p.trace + static_cast<size_t>(blockIdx.x) * kHfTraceWords : nullptr;
+  unsigned long long t_start_ns = 0;
+  long long t_start_clk = 0;
+  if constexpr (kTrace) {
+    t_start_ns = global_ns();
+    t_start_clk = clock64();
+  }
 
   const uint32_t a_region = sbase + kHfHeader;
   const uint32_t b_region = a_region + kHfNA * kHfAStage;
+  const uint32_t w2_region = b_region + kHfNB * kHfBBlock;
   const int tiles_per_img = p.tiles_x * p.tiles_y;
   // tiles of this CTA: cta_rank, cta_rank + cta_stride, ...
   const int my_tiles = (p.num_tiles > cta_rank) ? (p.num_tiles - cta_rank + cta_stride - 1) / cta_stride : 0;
@@ -156,48 +197,26 @@ heads_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
       }
     }
   } else if (warp == 3) {
-    // ------------------------------------------------------------------ B producer: conv1 blocks with the conv2 weight
-    // blocks of the previous tile interleaved at the same points at which the MMA warp consumes them
+    // ------------------------------------------------------------------ B producer: conv1 weight blocks
     const uint8_t* w1 = p.w1 + static_cast<size_t>(pair) * 18 * kHfBBlock;
     int stage = 0;
     uint32_t phase = 0;
-    for (int it = 0; it <= my_tiles; ++it) {
-      const bool has_c1 = it < my_tiles, has_c2 = it >= 1;
-      if (!has_c1 && !has_c2) break;
-      int next_item = 0;
-      for (int slot = 0; slot < 18; ++slot) {
-        if (has_c1) {
-          mbar_wait(bar_b_empty + 8 * stage, phase ^ 1);
-          if (elect_one()) {
-            mbar_arrive_expect_tx(bar_b_full + 8 * stage, kHfBBlock);
-            bulk_load_1d(b_region + stage * kHfBBlock, w1 + static_cast<size_t>(slot) * kHfBBlock, kHfBBlock, bar_b_full + 8 * stage);
-          }
-          __syncwarp();
-          if (++stage == kHfNB) {
-            stage = 0;
-            phase ^= 1;
-          }
+    for (int it = 0; it < my_tiles; ++it) {
+      for (int step = 0; step < 18; ++step) {
+        mbar_wait(bar_b_empty + 8 * stage, phase ^ 1);
+        if (elect_one()) {
+          mbar_arrive_expect_tx(bar_b_full + 8 * stage, kHfBBlock);
+          bulk_load_1d(b_region + stage * kHfBBlock, w1 + static_cast<size_t>(step) * kHfBBlock, kHfBBlock, bar_b_full + 8 * stage);
         }
-        if (has_c2) {
-          while (next_item < n_items && (items_s[next_item].slot <= slot || !has_c1)) {
-            const uint32_t bytes = static_cast<uint32_t>(items_s[next_item].nc) * 256u;
-            mbar_wait(bar_b_empty + 8 * stage, phase ^ 1);
-            if (elect_one()) {
-              mbar_arrive_expect_tx(bar_b_full + 8 * stage, bytes);
-              bulk_load_1d(b_region + stage * kHfBBlock, p.w2 + items_s[next_item].w2_off, bytes, bar_b_full + 8 * stage);
-            }
-            __syncwarp();
-            if (++stage == kHfNB) {
-              stage = 0;
-              phase ^= 1;
-            }
-            ++next_item;
-          }
+        __syncwarp();
+        if (++stage == kHfNB) {
+          stage = 0;
+          phase ^= 1;
         }
       }
     }
   } else if (warp == 1) {
-    // ------------------------------------------------------------------ MMA issuer
+    // ------------------------------------------------------------------ conv1 MMA issuer
     const uint32_t idesc1 = umma_idesc_16(128, 256, 0, 0, kF16);
     const uint64_t a_hi64 = umma_desc_hi(kHfAPlane, kHfARow);
     const uint64_t b_hi64 = umma_desc_hi(256 * 16, 128);
@@ -207,84 +226,103 @@ heads_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
     constexpr uint32_t a_kstep = (2 * kHfAPlane) >> 4, b_kstep = (2 * 256 * 16) >> 4;
     int a_stage = 0, b_stage = 0;
     uint32_t a_phase = 0, b_phase = 0;
-    uint32_t acc_empty_phase = 0, hid_full_phase = 0, c2_empty_phase = 0;   // acc_empty: one phase bit per buffer
-    for (int it = 0; it <= my_tiles; ++it) {
-      const bool has_c1 = it < my_tiles, has_c2 = it >= 1;
-      if (!has_c1 && !has_c2) break;
-      const int s = it & 1, sp = s ^ 1;
+    uint32_t acc_empty_phase = 0;   // one phase bit per buffer
+    unsigned long long w_b = 0, w_a = 0, w_acc = 0;
+    for (int it = 0; it < my_tiles; ++it) {
+      const int s = it & 1;
       const uint32_t tmem_d = tmem_base + s * 256;
-      if (has_c1) {
-        mbar_wait(bar_acc_empty + 8 * s, ((acc_empty_phase >> s) & 1u) ^ 1u);
-        acc_empty_phase ^= 1u << s;
-        tc_fence_after();
-      }
-      int next_item = 0;
+      // the only wait on the epilogue: buffer s is free once tile it - 2's last conv2 chunk has been drained
+      mbar_wait_t<kTrace>(bar_acc_empty + 8 * s, ((acc_empty_phase >> s) & 1u) ^ 1u, w_acc);
+      acc_empty_phase ^= 1u << s;
+      tc_fence_after();
       uint32_t a_base = 0;
-      for (int slot = 0; slot < 18; ++slot) {
-        if (has_c1) {
-          const int t = slot >= 9 ? slot - 9 : slot;
-          if (t == 0) {
-            mbar_wait(bar_a_full + 8 * a_stage, a_phase);
-            tc_fence_after();
-            a_base = a_lo0 + a_stage * (kHfAStage >> 4);
-          }
-          mbar_wait(bar_b_full + 8 * b_stage, b_phase);
+      for (int step = 0; step < 18; ++step) {
+        const int t = step >= 9 ? step - 9 : step;
+        if (t == 0) {
+          mbar_wait_t<kTrace>(bar_a_full + 8 * a_stage, a_phase, w_a);
           tc_fence_after();
-          const uint32_t b_base = b_lo0 + b_stage * (kHfBBlock >> 4);
-          const uint32_t a_tap = a_base + p.tap16[t];
-          if (elect_one()) {
-#pragma unroll
-            for (int j = 0; j < 4; ++j)
-              umma_bf16_lohi(tmem_d, a_tap + j * a_kstep, a_hi, b_base + j * b_kstep, b_hi, idesc1, (slot | j) != 0 ? 1u : 0u);
-            umma_commit(bar_b_empty + 8 * b_stage);
-            if (t == 8) umma_commit(bar_a_empty + 8 * a_stage);
-          }
-          __syncwarp();
-          if (++b_stage == kHfNB) {
-            b_stage = 0;
-            b_phase ^= 1;
-          }
-          if (t == 8 && ++a_stage == kHfNA) {
-            a_stage = 0;
-            a_phase ^= 1;
-          }
+          a_base = a_lo0 + a_stage * (kHfAStage >> 4);
         }
-        if (has_c2) {
-          while (next_item < n_items && (items_s[next_item].slot <= slot || !has_c1)) {
-            const HfItem item = items_s[next_item];
-            if (next_item == 0) {                              // hidden operands of the previous tile are in TMEM
-              mbar_wait(bar_hid_full, hid_full_phase);
-              hid_full_phase ^= 1u;
-            }
-            mbar_wait(bar_c2_empty, c2_empty_phase ^ 1u);      // the previous chunk has been drained
-            c2_empty_phase ^= 1u;
-            mbar_wait(bar_b_full + 8 * b_stage, b_phase);
-            tc_fence_after();
-            const uint32_t idesc2 = umma_idesc_16(128, item.nc, 0, 0, kF16);
-            const uint64_t w_hi64 = umma_desc_hi(static_cast<uint32_t>(item.nc) * 16, 128);
-            const uint32_t w_hi = static_cast<uint32_t>(w_hi64 >> 32);
-            const uint32_t w_lo = static_cast<uint32_t>(w_hi64) | ((b_region + b_stage * kHfBBlock) >> 4);
-            const uint32_t a2 = tmem_base + sp * 256 + item.head_slot * 64;
-            const uint32_t d2 = tmem_base + sp * 256 + 128;
-            if (elect_one()) {
+        mbar_wait_t<kTrace>(bar_b_full + 8 * b_stage, b_phase, w_b);
+        tc_fence_after();
+        const uint32_t b_base = b_lo0 + b_stage * (kHfBBlock >> 4);
+        const uint32_t a_tap = a_base + p.tap16[t];
+        if (elect_one()) {
 #pragma unroll
-              for (int k = 0; k < 8; ++k)
-                umma_16_ts(d2, a2 + k * 8, w_lo + k * 2 * item.nc, w_hi, idesc2, k != 0 ? 1u : 0u);
-              umma_commit(bar_b_empty + 8 * b_stage);
-              umma_commit(bar_c2_full);
-            }
-            __syncwarp();
-            if (++b_stage == kHfNB) {
-              b_stage = 0;
-              b_phase ^= 1;
-            }
-            ++next_item;
-          }
+          for (int j = 0; j < 4; ++j)
+            umma_bf16_lohi(tmem_d, a_tap + j * a_kstep, a_hi, b_base + j * b_kstep, b_hi, idesc1, (step | j) != 0 ? 1u : 0u);
+          umma_commit(bar_b_empty + 8 * b_stage);
+          if (t == 8) umma_commit(bar_a_empty + 8 * a_stage);
+        }
+        __syncwarp();
+        if (++b_stage == kHfNB) {
+          b_stage = 0;
+          b_phase ^= 1;
+        }
+        if (t == 8 && ++a_stage == kHfNA) {
+          a_stage = 0;
+          a_phase ^= 1;
         }
       }
-      if (has_c1) {
-        if (elect_one()) umma_commit(bar_acc_full + 8 * s);
+      if (elect_one()) umma_commit(bar_acc_full + 8 * s);
+      __syncwarp();
+    }
+    if constexpr (kTrace) {
+      if (lane == 0) {
+        trace[kHtC1BFull] = w_b;
+        trace[kHtC1AFull] = w_a;
+        trace[kHtC1AccEmpty] = w_acc;
+      }
+    }
+  } else if (warp == 2) {
+    // ------------------------------------------------------------------ conv2 MMA issuer (after the TMEM allocation)
+    // Per chunk: load its weights into the conv2 slot once the previous chunk's MMAs have read it (this overlaps the
+    // previous chunk's drain), wait for the drain, issue. tcgen05.commit tracks only this thread's MMAs, so the conv1
+    // warp's commits are independent of these.
+    uint32_t hid_full_phase = 0, c2_empty_phase = 0, w2_phase = 0;
+    unsigned long long w_hid = 0, w_c2e = 0, w_wf = 0, w_we = 0;
+    for (int it = 0; it < my_tiles; ++it) {
+      const uint32_t tbuf = tmem_base + (it & 1) * 256;
+      for (int i = 0; i < n_items; ++i) {
+        const HfItem item = items_s[i];
+        const uint32_t bytes = static_cast<uint32_t>(item.nc) * 256u;
+        mbar_wait_t<kTrace>(bar_w2_empty, w2_phase ^ 1u, w_we);
+        if (elect_one()) {
+          mbar_arrive_expect_tx(bar_w2_full, bytes);
+          bulk_load_1d(w2_region, p.w2 + item.w2_off, bytes, bar_w2_full);
+        }
         __syncwarp();
+        if (i == 0) {                                          // both hidden operands of this tile are in TMEM
+          mbar_wait_t<kTrace>(bar_hid_full, hid_full_phase, w_hid);
+          hid_full_phase ^= 1u;
+        }
+        mbar_wait_t<kTrace>(bar_c2_empty, c2_empty_phase ^ 1u, w_c2e);   // the previous chunk has been drained
+        c2_empty_phase ^= 1u;
+        mbar_wait_t<kTrace>(bar_w2_full, w2_phase, w_wf);
+        w2_phase ^= 1u;
+        tc_fence_after();
+        const uint32_t idesc2 = umma_idesc_16(128, item.nc, 0, 0, kF16);
+        const uint64_t w_hi64 = umma_desc_hi(static_cast<uint32_t>(item.nc) * 16, 128);
+        const uint32_t w_hi = static_cast<uint32_t>(w_hi64 >> 32);
+        const uint32_t w_lo = static_cast<uint32_t>(w_hi64) | (w2_region >> 4);
+        const uint32_t a2 = tbuf + item.head_slot * 64;
+        const uint32_t d2 = tbuf + 128;
+        if (elect_one()) {
+#pragma unroll
+          for (int k = 0; k < 8; ++k)
+            umma_16_ts(d2, a2 + k * 8, w_lo + k * 2 * item.nc, w_hi, idesc2, k != 0 ? 1u : 0u);
+          umma_commit(bar_w2_empty);
+          umma_commit(bar_c2_full);
+        }
+        __syncwarp();
+      }
+    }
+    if constexpr (kTrace) {
+      if (lane == 0) {
+        trace[kHtC2HidFull] = w_hid;
+        trace[kHtC2C2Empty] = w_c2e;
+        trace[kHtC2WFull] = w_wf;
+        trace[kHtC2WEmpty] = w_we;
       }
     }
   } else if (warp >= 4) {
@@ -297,6 +335,8 @@ heads_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
     const float4* bias2_4 = reinterpret_cast<const float4*>(bias2_s);
     const size_t plane_px = static_cast<size_t>(p.H) * p.W;
     uint32_t acc_full_phase = 0, c2_full_phase = 0;        // acc_full: one phase bit per buffer
+    unsigned long long w_acc = 0, w_c2 = 0, busy1 = 0, busy2 = 0;
+    long long t_mark = 0;
     for (int it = 0; it < my_tiles; ++it) {
       const int g = cta_rank + it * cta_stride;
       const int n = g / tiles_per_img;
@@ -307,9 +347,10 @@ heads_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
       const size_t px = static_cast<size_t>(y) * p.W + x;
       const int s = it & 1;
       const uint32_t tstage = tmem_base + s * 256 + (static_cast<uint32_t>(q * 32) << 16);
-      mbar_wait(bar_acc_full + 8 * s, (acc_full_phase >> s) & 1u);
+      mbar_wait_t<kTrace>(bar_acc_full + 8 * s, (acc_full_phase >> s) & 1u, w_acc);
       acc_full_phase ^= 1u << s;
       tc_fence_after();
+      if constexpr (kTrace) t_mark = clock64();
       // ---- phase 1: conv1 accumulators -> bias + LeakyReLU -> 16-bit hidden operand, back into TMEM. This warp takes
       // channels [64 eh, 64 eh + 64) of each head: accumulator columns hs * 128 + 64 eh + [0, 64) -> packed columns
       // hs * 64 + 32 eh + [0, 32). Hidden A and B overwrite head A's accumulators, which BOTH warps of the lane quarter
@@ -350,12 +391,16 @@ heads_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(bar_hid_full);
-      // ---- phase 2: conv2 accumulators of this tile (issued during the next tile's conv1) -> + bias -> fp32 logits
+      if constexpr (kTrace) {
+        busy1 += static_cast<unsigned long long>(clock64() - t_mark);
+        t_mark = clock64();
+      }
+      // ---- phase 2: conv2 accumulators of this tile, chunk by chunk -> + bias -> fp32 logits
 #pragma unroll 1
       for (int ii = 0; ii < n_items; ++ii) {
         const HfItem item = items_s[ii];
         const int head = 2 * pair + item.head_slot;
-        mbar_wait(bar_c2_full, c2_full_phase);
+        mbar_wait_t<kTrace>(bar_c2_full, c2_full_phase, w_c2);
         c2_full_phase ^= 1u;
         tc_fence_after();
         const int units = item.nc >> 4;
@@ -400,6 +445,15 @@ heads_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
         if (lane == 0) mbar_arrive(bar_c2_empty);
       }
       if (lane == 0) mbar_arrive(bar_acc_empty + 8 * s);
+      if constexpr (kTrace) busy2 += static_cast<unsigned long long>(clock64() - t_mark);
+    }
+    if constexpr (kTrace) {
+      if (warp == 4 && lane == 0) {
+        trace[kHtEpAccFull] = w_acc;
+        trace[kHtEpPhase1] = busy1;
+        trace[kHtEpC2Full] = w_c2;
+        trace[kHtEpPhase2] = busy2 - w_c2;
+      }
     }
   }
 
@@ -408,6 +462,15 @@ heads_fused_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_consta
   if (warp == 2) {
     tc_fence_after();
     tmem_dealloc<512>(tmem_base);
+  }
+  if constexpr (kTrace) {
+    if (threadIdx.x == 0) {
+      trace[kHtPair] = pair;
+      trace[kHtTiles] = my_tiles;
+      trace[kHtStartNs] = t_start_ns;
+      trace[kHtEndNs] = global_ns();
+      trace[kHtCycles] = static_cast<unsigned long long>(clock64() - t_start_clk);
+    }
   }
 }
 
@@ -478,14 +541,6 @@ extern "C" int abc_heads_fused(const AbcHeadsFusedDesc* d, void* stream_) {
       }
     }
     ABC_REQUIRE(bias_len <= 512, "abc_heads_fused: pair %d: %d conv2 output columns exceed the 512 supported", pr, bias_len);
-    // issue points inside the next tile's conv1 stream (18 (chunk, tap) steps). The chunks share one TMEM region, so each
-    // waits for the drain of the one before. Measured on B200 with the v2 heads (ABCNET_HF_SLOTS sweep): early and 4 steps
-    // apart (2, 6, 10, 14) beat later or more evenly spread points by 0.4 - 1 ms.
-    for (int i = 0; i < ni; ++i) {
-      int slot = d->item_slot[i] >= 0 && d->item_slot[i] < 18 ? d->item_slot[i] : (2 + 4 * i < 17 ? 2 + 4 * i : 17);
-      if (i > 0 && slot < p.items[pr][i - 1].slot) slot = p.items[pr][i - 1].slot;
-      p.items[pr][i].slot = slot;
-    }
     p.n_items[pr] = ni;
     p.bias2_len[pr] = bias_len;
     bias_off_total += bias_len;
@@ -516,8 +571,11 @@ extern "C" int abc_heads_fused(const AbcHeadsFusedDesc* d, void* stream_) {
   }
   static PerDeviceOnce attr_once;
   ABC_CUDA(attr_once.run([] {
-    cudaError_t e = cudaFuncSetAttribute(heads_fused_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kHfSmem);
-    return e != cudaSuccess ? e : cudaFuncSetAttribute(heads_fused_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kHfSmem);
+    void (*const kernels[4])(const CUtensorMap, const HfParams) = {heads_fused_kernel<false, false>, heads_fused_kernel<true, false>,
+                                                                   heads_fused_kernel<false, true>, heads_fused_kernel<true, true>};
+    for (auto k : kernels)
+      if (cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, kHfSmem); e != cudaSuccess) return e;
+    return cudaSuccess;
   }));
   int sms = sm_count();
   if (sms <= 0) sms = 148;
@@ -533,11 +591,14 @@ extern "C" int abc_heads_fused(const AbcHeadsFusedDesc* d, void* stream_) {
   p.pairs = pairs;
   p.cta0[0] = 0;
   for (int pr = 0; pr < pairs; ++pr) p.cta0[pr + 1] = p.cta0[pr] + ctas[pr];
+  p.trace = static_cast<unsigned long long*>(d->trace);
   cudaStream_t st = static_cast<cudaStream_t>(stream_);
-  if (f16)
-    heads_fused_kernel<true><<<total, kHfThreads, kHfSmem, st>>>(tmap, p);
+  if (d->trace)
+    (f16 ? heads_fused_kernel<true, true> : heads_fused_kernel<false, true>)<<<total, kHfThreads, kHfSmem, st>>>(tmap, p);
+  else if (f16)
+    heads_fused_kernel<true, false><<<total, kHfThreads, kHfSmem, st>>>(tmap, p);
   else
-    heads_fused_kernel<false><<<total, kHfThreads, kHfSmem, st>>>(tmap, p);
+    heads_fused_kernel<false, false><<<total, kHfThreads, kHfSmem, st>>>(tmap, p);
   return launch_check("heads_fused_kernel");
 }
 

@@ -7,15 +7,23 @@
 
 namespace abc {
 
-// Cost of one 128-pixel tile of a pair in tensor-pipe cycles of one SM, a model rather than a measurement:
-//   conv1      : 2 x 9 x 4 MMAs of 128 x 256 x 16 at 8192 bf16 FLOP/clk = 128 clk each;
-//   conv2      : 8 MMAs of 128 x nc x 16 per chunk, nc / 2 clk each plus the fixed per-MMA cost of ~60 clk (DESIGN.md 4.1);
-//   logits     : 128 pixels x channels x 4 bytes at 64 B/clk -- the stores overlap the MMAs of the next tile only in part,
-//                because the next chunk waits for the drain of the previous one.
+// Cost of one 128-pixel tile of a pair in SM cycles. conv1 and conv2 have an issuing warp each, so a tile costs the longer
+// of two streams that overlap:
+//   tensor pipe : conv1 = 2 x 9 x 4 MMAs of 128 x 256 x 16 at 8192 bf16 FLOP/clk = 128 clk each; conv2 = 8 MMAs of
+//                 128 x nc x 16 per chunk, nc / 2 clk each plus ~60 clk fixed (DESIGN.md 4.1); plus ~19 clk per logit
+//                 channel of weight-ring stalls, which grow with the pair's logit stores;
+//   conv2 chain : epilogue phase 1 (~2000 clk), then per chunk the MMA latency behind the queued conv1 MMAs (~1350 clk)
+//                 and its drain (~1000 clk per 32 channels: each of the two epilogue warps of a lane quarter stores 16).
+//                 The chunks share one TMEM region, so each waits for the drain of the one before.
+// The constants are fitted to the per-tile cycles that tools/heads_trace.py measured on B200 with the v2 heads
+// (profiles/r05_heads_trace_after.json): the 1 + 360-channel pair is bound by its chain, the others by the tensor pipe.
 inline int64_t hf_pair_tile_cost(int n_chunks, const int* nc, int logit_channels) {
-  int64_t c = 72 * 128;
-  for (int i = 0; i < n_chunks; ++i) c += 8 * (nc[i] / 2 + 60);
-  return c + static_cast<int64_t>(128) * 4 * logit_channels / 64;
+  int64_t pipe = 72 * 128 + static_cast<int64_t>(19) * logit_channels, chain = 2000;
+  for (int i = 0; i < n_chunks; ++i) {
+    pipe += 8 * (nc[i] / 2 + 60);
+    chain += 1350 + 1000 * ((nc[i] + 31) / 32);
+  }
+  return pipe > chain ? pipe : chain;
 }
 
 // ctas[p] for pairs p = 0 .. pairs-1: at least one each, then every further CTA (up to `sms` in total) to the pair with the

@@ -620,6 +620,27 @@ class UNet(nn.Module):
         cv("dconv2.3", k1, 0, k2)                                           # trunk
         return k2
 
+    def _heads_fused_desc(self, k2, outs):
+        """AbcHeadsFusedDesc of abc_heads_fused for trunk output k2 and the head outputs outs (tools/heads_trace.py adds a
+        trace buffer to it)."""
+        w2pack, bias2 = self._packed["heads.fused"]
+        pk1 = self._packed["heads.conv1.plain"]
+        if pk1 is None:
+            wt1, b1, c1 = self._heads_w1
+            pk1 = self._packed["heads.conv1.plain"] = _Packed(wt1, b1, [(dy, dx) for (dy, dx, _, _) in _TAPS3], 256, c1, pair=False,
+                                                              dtype=self._act_torch_dtype)
+        B, _, H4, W4, _ = k2.shape
+        d = AbcHeadsFusedDesc()
+        d.in_, d.N, d.H, d.W, d.in_planes, d.in_plane_off = k2.data_ptr(), B, H4, W4, k2.shape[1], 0
+        d.w1pack, d.bias1, d.n_heads = pk1.w.data_ptr(), pk1.bias.data_ptr(), len(self.heads)
+        d.w2pack, d.w2pack_bytes, d.bias2, d.bias2_len = w2pack.data_ptr(), w2pack.numel() * 2, bias2.data_ptr(), bias2.numel()
+        d.act_fp16 = int(pk1.fp16)
+        for i, h in enumerate(self.heads):
+            d.cout[i], d.out[i] = h, outs[i].data_ptr()
+            d.out_mode[i] = 2 if outs[i].dim() == 5 else 1
+            d.out_planes[i] = outs[i].shape[1] if outs[i].dim() == 5 else 0
+        return d
+
     @torch.no_grad()
     def infer(self, x, outs=None, layout="nchw", fused=None):
         """Eval forward. layout="nchw": the reference's list of fp32 NCHW tensors. layout="p8f": a ``HeadMaps`` list in
@@ -647,24 +668,7 @@ class UNet(nn.Module):
         if fused:
             if fpack is None:
                 raise ValueError("abc_heads_fused is not available for this head list (see include/abcnet_b200.h); use fused=False")
-            w2pack, bias2 = fpack
-            pk1 = self._packed["heads.conv1.plain"]
-            if pk1 is None:
-                wt1, b1, c1 = self._heads_w1
-                pk1 = self._packed["heads.conv1.plain"] = _Packed(wt1, b1, [(dy, dx) for (dy, dx, _, _) in _TAPS3], 256, c1, pair=False,
-                                                                  dtype=self._act_torch_dtype)
-            d = AbcHeadsFusedDesc()
-            d.in_, d.N, d.H, d.W, d.in_planes, d.in_plane_off = k2.data_ptr(), B, H4, W4, k2.shape[1], 0
-            d.w1pack, d.bias1, d.n_heads = pk1.w.data_ptr(), pk1.bias.data_ptr(), len(self.heads)
-            d.w2pack, d.w2pack_bytes, d.bias2, d.bias2_len = w2pack.data_ptr(), w2pack.numel() * 2, bias2.data_ptr(), bias2.numel()
-            slots = [int(v) for v in os.environ.get("ABCNET_HF_SLOTS", "").split(",") if v.strip()]
-            for i in range(6):
-                d.item_slot[i] = slots[i] if i < len(slots) else -1
-            d.act_fp16 = int(pk1.fp16)
-            for i, h in enumerate(self.heads):
-                d.cout[i], d.out[i] = h, outs[i].data_ptr()
-                d.out_mode[i] = 2 if outs[i].dim() == 5 else 1
-                d.out_planes[i] = outs[i].shape[1] if outs[i].dim() == 5 else 0
+            d = self._heads_fused_desc(k2, outs)
             with self._timed("heads.fused"):
                 check(lib.abc_heads_fused(C.byref(d), st), "abc_heads_fused")
             return outs

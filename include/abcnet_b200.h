@@ -180,9 +180,10 @@ ABC_API int64_t abc_conv_wpack_bytes(int cin, int cout, int ntaps, int n_tile);
  *                    nc = count rounded up to 16: 16-bit [16 (K planes)][nc][8] (zero rows past the count), bias fp32 [nc];
  *                    total sizes from abc_heads_fused_pack_sizes
  *   out[h]         : fp32 logits, out_mode[h] = 1: NCHW [N][cout][H][W]; 2: planar-8 [N][out_planes][H][W][8]
- *   item_slot[i]   : tuning knob, -1 = default: the i-th conv2 chunk of a head pair is issued after this (K chunk, tap)
- *                    step (0..17) of the next tile's conv1
  *   act_fp16       : 0: bf16 trunk and weights; 1: IEEE fp16 (AbcConvDesc.act_fp16), hidden maps rounded to fp16
+ *   trace          : NULL, or a device buffer of 16 uint64 per CTA: the kernel then records, per CTA, its head pair, tile
+ *                    count, start / end %globaltimer and the clock64 cycles each issuing warp and the epilogue spent
+ *                    waiting on each barrier (tools/heads_trace.py). For profiling; the logits are unchanged.
  * Limits: n_heads <= 16, at most 6 chunks and 512 padded conv2 channels per pair of heads.
  */
 typedef struct AbcHeadsFusedDesc {
@@ -200,8 +201,8 @@ typedef struct AbcHeadsFusedDesc {
   void* out[16];
   int out_mode[16];
   int out_planes[16];
-  int item_slot[6];
   int act_fp16;
+  void* trace;
 } AbcHeadsFusedDesc;
 ABC_API int abc_heads_fused(const AbcHeadsFusedDesc* desc, void* stream);
 ABC_API int abc_heads_fused_pack_sizes(int n_heads, const int* cout, int64_t* w2pack_bytes, int* bias2_len);
