@@ -20,6 +20,10 @@ EXPORTS = (
     "abc_nchw_to_p8_ex", "abc_deinterleave2", "abc_conv_wgrad", "abc_conv3x3_c1_wgrad", "abc_conv3x3_c1_raw",
     "abc_heads_fused", "abc_heads_fused_pack_sizes", "abc_gather_pack", "abc_adam_step", "abc_adam_chunk_elems", "abc_assemble_molblocks", "abc_gather_patches", "abc_gather_patches_pooled", "abc_rasterise_targets",
     "abc_unet_wpack_bytes", "abc_unet_workspace_bytes", "abc_unet_create", "abc_unet_forward_infer", "abc_unet_destroy", "abc_unet_pack_host",
+    # deterministic reductions (torch.use_deterministic_algorithms)
+    "abc_bn_stats_det", "abc_channel_sum_det", "abc_bn_stats_workspace_bytes", "abc_bn_act_backward_workspace_bytes",
+    "abc_nchw_to_p8_ex_det", "abc_nchw_to_p8_ex_workspace_bytes", "abc_conv3x3_c1_wgrad_det", "abc_conv3x3_cn_wgrad_det",
+    "abc_conv3x3_wgrad_workspace_bytes", "abc_conv_wgrad_workspace_bytes", "abc_conv_stat_workspace_bytes", "abc_loss_workspace_bytes",
 )
 
 
@@ -38,6 +42,7 @@ class AbcConvDesc(C.Structure):
         ("k_segments", C.c_int), ("seg_tap0", C.c_int * 4), ("seg_ntaps", C.c_int * 4),
         ("row_fold", C.c_int), ("cta_pair", C.c_int), ("swap_mn", C.c_int),
         ("stat_sum", C.c_void_p), ("stat_sq", C.c_void_p), ("subpixel", C.c_int), ("k_chunk", C.c_int), ("act_fp16", C.c_int),
+        ("stat_ws", C.c_void_p),
     ]
 
 
@@ -114,6 +119,7 @@ class AbcBnActBwdDesc(C.Structure):
         ("scale", C.c_void_p), ("shift", C.c_void_p), ("mean", C.c_void_p), ("invstd", C.c_void_p),
         ("act", C.c_int), ("drop_p", C.c_float), ("seed", C.c_uint64),
         ("s1", C.c_void_p), ("s2", C.c_void_p), ("seed_dev", C.c_void_p), ("gscale", C.c_void_p), ("drop_mask", C.c_void_p),
+        ("ws", C.c_void_p),
     ]
 
 
@@ -123,7 +129,7 @@ class AbcWgradDesc(C.Structure):
         ("in_", C.c_void_p), ("in_planes", C.c_int), ("in_plane_off", C.c_int), ("cin", C.c_int),
         ("N", C.c_int), ("H", C.c_int), ("W", C.c_int),
         ("ntaps", C.c_int), ("tap_dy", C.c_int * 9), ("tap_dx", C.c_int * 9),
-        ("dw", C.c_void_p), ("row_boxes", C.c_int),
+        ("dw", C.c_void_p), ("row_boxes", C.c_int), ("ws", C.c_void_p),
     ]
 
 
@@ -133,7 +139,7 @@ class AbcLossDesc(C.Structure):
         ("N", C.c_int), ("H", C.c_int), ("W", C.c_int),
         ("c_type", C.c_int), ("c_charge", C.c_int), ("c_hs", C.c_int), ("n_omega", C.c_int), ("n_btype", C.c_int),
         ("type_weights", C.c_void_p), ("sums", C.c_void_p), ("scale", C.c_void_p),
-        ("dlogits", C.c_void_p * 8),
+        ("dlogits", C.c_void_p * 8), ("ws", C.c_void_p),
     ]
 
 
@@ -196,6 +202,19 @@ def _load():
     lib.abc_unet_destroy.argtypes = [vp]
     lib.abc_unet_pack_host.argtypes = [C.POINTER(AbcUNetConfig), C.POINTER(AbcNamedTensor), ci, vp, C.c_int64, C.POINTER(C.c_int64)]
     lib.abc_assemble_molblocks.argtypes = [vp, ci, vp, ci, vp, ci, vp, vp, ci, ci, vp, C.c_int64, vp]
+    lib.abc_bn_stats_det.argtypes = [vp, ci, ci, ci, ci, ci, ci, vp, vp, vp, vp]
+    lib.abc_channel_sum_det.argtypes = lib.abc_bn_stats_det.argtypes
+    lib.abc_nchw_to_p8_ex_det.argtypes = [vp, vp, ci, ci, ci, ci, ci, vp, vp, vp, vp]
+    lib.abc_conv3x3_c1_wgrad_det.argtypes = [vp, ci, vp, ci, ci, ci, ci, ci, vp, vp, vp]
+    lib.abc_conv3x3_cn_wgrad_det.argtypes = [vp, ci, vp, ci, ci, ci, ci, ci, vp, vp, vp]
+    sz = C.c_size_t
+    for name, args in (("abc_bn_stats_workspace_bytes", [ci] * 4), ("abc_bn_act_backward_workspace_bytes", [C.POINTER(AbcBnActBwdDesc)]),
+                       ("abc_nchw_to_p8_ex_workspace_bytes", [ci] * 5), ("abc_conv3x3_wgrad_workspace_bytes", [ci]),
+                       ("abc_conv_wgrad_workspace_bytes", [C.POINTER(AbcWgradDesc)]),
+                       ("abc_conv_stat_workspace_bytes", [C.POINTER(AbcConvDesc)]),
+                       ("abc_loss_workspace_bytes", [C.POINTER(AbcLossDesc), ci])):
+        getattr(lib, name).restype = sz
+        getattr(lib, name).argtypes = args
     return lib
 
 

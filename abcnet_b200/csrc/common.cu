@@ -71,11 +71,48 @@ int sm_count() {
   return n;
 }
 
+// One block per 32 consecutive elements: lane = element, warp w sums the contiguous slot range [w S / 8, (w + 1) S / 8) in
+// order, thread w == 0 then adds the 8 warp totals in warp order.
+template <typename T>
+__global__ void __launch_bounds__(256) det_reduce_kernel(const T* __restrict__ ws, int slots, int n, const DetOut out, int add) {
+  __shared__ T part[8][32];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int e = blockIdx.x * 32 + lane;
+  const int s0 = static_cast<int>(static_cast<long long>(slots) * warp / 8), s1 = static_cast<int>(static_cast<long long>(slots) * (warp + 1) / 8);
+  T t = 0;
+  if (e < n)
+    for (int s = s0; s < s1; ++s) t += ws[static_cast<size_t>(s) * n + e];
+  part[warp][lane] = t;
+  __syncthreads();
+  if (warp != 0 || e >= n) return;
+  T r = part[0][lane];
+#pragma unroll
+  for (int w = 1; w < 8; ++w) r += part[w][lane];
+  int k = 0, start = 0;
+  while (e >= out.end[k]) start = out.end[k++];
+  T* dst = static_cast<T*>(out.ptr[k]) + (e - start);
+  *dst = add ? *dst + r : r;
+}
+
+template <typename T>
+static int det_reduce_t(const T* ws, int slots, int n, const DetOut& out, int add, cudaStream_t st) {
+  ABC_REQUIRE(ws && slots > 0 && n > 0 && out.count >= 1 && out.count <= kDetMaxOut && out.end[out.count - 1] == n,
+              "det_reduce: bad workspace / output segments");
+  det_reduce_kernel<T><<<(n + 31) / 32, 256, 0, st>>>(ws, slots, n, out, add);
+  return launch_check("det_reduce_kernel");
+}
+int det_reduce(const float* ws, int slots, int n, const DetOut& out, int add, cudaStream_t st) {
+  return det_reduce_t(ws, slots, n, out, add, st);
+}
+int det_reduce(const double* ws, int slots, int n, const DetOut& out, int add, cudaStream_t st) {
+  return det_reduce_t(ws, slots, n, out, add, st);
+}
+
 }  // namespace abc
 
 extern "C" {
 const char* abc_last_error(void) { return abc::g_err; }
-int abc_version(void) { return 102; }
+int abc_version(void) { return 103; }
 int abc_device_ok(void) { return abc::device_check() == ABC_OK ? 1 : 0; }
 int abc_sm_count(void) {
   int n = abc::sm_count();

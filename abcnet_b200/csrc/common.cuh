@@ -53,6 +53,21 @@ struct PerDeviceOnce {
     }                                 \
   } while (0)
 
+// Fixed-order reduction of the deterministic mode (det_slots.cuh): for e < n, r = sum over s < slots of ws[s * n + e], added in
+// slot-index order (contiguous slot ranges per warp, then the warp totals in warp order -- fixed for given slots and n). The
+// element range is cut into consecutive output segments (ends ascending, the last one == n): element e of segment k goes to
+// out[k][e - start of k]; add != 0 adds r to the value there instead of overwriting it.
+constexpr int kDetMaxOut = 10;
+struct DetOut {
+  void* ptr[kDetMaxOut];
+  int end[kDetMaxOut];
+  int count;
+};
+int det_reduce(const float* ws, int slots, int n, const DetOut& out, int add, cudaStream_t st);
+int det_reduce(const double* ws, int slots, int n, const DetOut& out, int add, cudaStream_t st);
+inline DetOut det_out1(void* a, int n) { DetOut o{}; o.ptr[0] = a; o.end[0] = n; o.count = 1; return o; }
+inline DetOut det_out2(void* a, void* b, int n) { DetOut o{}; o.ptr[0] = a; o.end[0] = n; o.ptr[1] = b; o.end[1] = 2 * n; o.count = 2; return o; }
+
 inline int launch_check(const char* what) {
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) {

@@ -25,6 +25,7 @@
 #include <cuda_bf16.h>
 
 #include "common.cuh"
+#include "det_slots.cuh"
 #include "p8_device.cuh"
 #include "ptx_sm100.cuh"
 
@@ -67,6 +68,9 @@ struct ConvKParams {
   // bf16-rounded outputs, accumulated per thread over the CTA's whole tile loop, one fp64 atomic per thread at the end
   double* stat_sum;
   double* stat_sq;
+  // DET: the same per-thread / per-warp sums stored to slot blockIdx.x * 8 + owner of [slots][2 cout] (sums, then squares)
+  // instead of the atomics (det_slots.cuh)
+  double* stat_ws;
 };
 
 __device__ __forceinline__ float apply_act(float v, int act) {
@@ -128,7 +132,8 @@ __device__ __forceinline__ uint4 pool_max_bf16x8(uint4 q, bool f16) {
 // operand), N = 256 pixels (one 32 x 8 tile per pipeline stage is the B operand); accumulator = [channel][pixel].
 // STATS: the non-swap epilogue of the row-folded 16-channel layers also accumulates the fused BatchNorm statistics (32 extra
 // registers per epilogue thread, hence its own instantiation); the operand-swap epilogue does so behind a runtime flag.
-template <int KSTEPS, bool RESIDENT, bool CG2, bool SWAP = false, bool STATS = false>
+// DET: the fused statistics go to the deterministic slots of p.stat_ws instead of fp64 atomics.
+template <int KSTEPS, bool RESIDENT, bool CG2, bool SWAP = false, bool STATS = false, bool DET = false>
 __global__ void __launch_bounds__(kThreads, 1)
 conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap, const ConvKParams p) {
   static_assert(!(CG2 && RESIDENT), "the CTA-pair variant streams its weights");
@@ -533,8 +538,14 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap, const ConvKParams p)
     if (do_stats) {
       const int ch = n0 + (m_own - fj_own * cpj);
       if (ch < p.cout) {
-        atomicAdd(p.stat_sum + ch, static_cast<double>(st_s));
-        atomicAdd(p.stat_sq + ch, static_cast<double>(st_q));
+        if constexpr (DET) {            // owner = (epilogue half, folded row)
+          const int slot = blockIdx.x * kConvStatOwners + eh * J + fj_own;
+          p.stat_ws[det_slot_index(slot, 2 * p.cout, ch)] = static_cast<double>(st_s);
+          p.stat_ws[det_slot_index(slot, 2 * p.cout, p.cout + ch)] = static_cast<double>(st_q);
+        } else {
+          atomicAdd(p.stat_sum + ch, static_cast<double>(st_s));
+          atomicAdd(p.stat_sq + ch, static_cast<double>(st_q));
+        }
       }
     }
   } else if (warp >= 4) {
@@ -725,8 +736,14 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap, const ConvKParams p)
           b += __shfl_xor_sync(0xffffffffu, b, o);
         }
         if (lane == 0 && n0 + i < p.cout) {
-          atomicAdd(p.stat_sum + n0 + i, static_cast<double>(a));
-          atomicAdd(p.stat_sq + n0 + i, static_cast<double>(b));
+          if constexpr (DET) {          // owner = epilogue warp
+            const int slot = blockIdx.x * kConvStatOwners + (warp - 4);
+            p.stat_ws[det_slot_index(slot, 2 * p.cout, n0 + i)] = static_cast<double>(a);
+            p.stat_ws[det_slot_index(slot, 2 * p.cout, p.cout + n0 + i)] = static_cast<double>(b);
+          } else {
+            atomicAdd(p.stat_sum + n0 + i, static_cast<double>(a));
+            atomicAdd(p.stat_sq + n0 + i, static_cast<double>(b));
+          }
         }
       }
     }
@@ -969,10 +986,15 @@ extern "C" int abc_conv_igemm(const AbcConvDesc* d, void* stream_) {
     ABC_REQUIRE(swap || (fold == 4 && d->cout == 16 && d->n_tile == 64 && d->cin == 16),
                 "abc_conv_igemm: fused statistics are built for operand-swap launches and the row-folded 16 -> 16 layers "
                 "(use abc_bn_stats otherwise)");
-    ABC_CUDA(cudaMemsetAsync(d->stat_sum, 0, d->cout * sizeof(double), st_));
-    ABC_CUDA(cudaMemsetAsync(d->stat_sq, 0, d->cout * sizeof(double), st_));
     p.stat_sum = d->stat_sum;
     p.stat_sq = d->stat_sq;
+    p.stat_ws = d->stat_ws;
+    if (d->stat_ws)            // slots no owner writes (unused folded rows) must read as zero in the ordered sum
+      ABC_CUDA(cudaMemsetAsync(d->stat_ws, 0, abc_conv_stat_workspace_bytes(d), st_));
+    else {
+      ABC_CUDA(cudaMemsetAsync(d->stat_sum, 0, d->cout * sizeof(double), st_));
+      ABC_CUDA(cudaMemsetAsync(d->stat_sq, 0, d->cout * sizeof(double), st_));
+    }
   }
 
   EncodeTiledFn encode = get_encode_fn();
@@ -1006,16 +1028,25 @@ extern "C" int abc_conv_igemm(const AbcConvDesc* d, void* stream_) {
                                   conv_igemm_kernel<3, false, false, true>, conv_igemm_kernel<4, false, false, true>},
                                  {nullptr, conv_igemm_kernel<1, true, false, true>, conv_igemm_kernel<2, true, false, true>,
                                   conv_igemm_kernel<3, true, false, true>, conv_igemm_kernel<4, true, false, true>}};
+  KernelFn swap_det_kernels[2][5] = {{nullptr, conv_igemm_kernel<1, false, false, true, false, true>,
+                                      conv_igemm_kernel<2, false, false, true, false, true>, conv_igemm_kernel<3, false, false, true, false, true>,
+                                      conv_igemm_kernel<4, false, false, true, false, true>},
+                                     {nullptr, conv_igemm_kernel<1, true, false, true, false, true>,
+                                      conv_igemm_kernel<2, true, false, true, false, true>, conv_igemm_kernel<3, true, false, true, false, true>,
+                                      conv_igemm_kernel<4, true, false, true, false, true>}};
   KernelFn pair_kernel = conv_igemm_kernel<4, false, true>;
   KernelFn stats_kernel = conv_igemm_kernel<1, true, false, false, true>;      // row-folded 16 -> 16 with fused statistics
+  KernelFn stats_det_kernel = conv_igemm_kernel<1, true, false, false, true, true>;
   static PerDeviceOnce attr_once;
   ABC_CUDA(attr_once.run([&]() -> cudaError_t {
     for (int r = 0; r < 2; ++r)
       for (int k = 1; k <= 4; ++k) {
         if (cudaError_t e = cudaFuncSetAttribute(kernels[r][k], cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget)) return e;
         if (cudaError_t e = cudaFuncSetAttribute(swap_kernels[r][k], cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget)) return e;
+        if (cudaError_t e = cudaFuncSetAttribute(swap_det_kernels[r][k], cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget)) return e;
       }
     if (cudaError_t e = cudaFuncSetAttribute(stats_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget)) return e;
+    if (cudaError_t e = cudaFuncSetAttribute(stats_det_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget)) return e;
     return cudaFuncSetAttribute(pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget);
   }));
   const int ksteps = p.kp / 2;
@@ -1049,11 +1080,24 @@ extern "C" int abc_conv_igemm(const AbcConvDesc* d, void* stream_) {
   }
   if (gx > p.num_groups) gx = p.num_groups;
   dim3 grid(gx, n_tiles, 1);
-  KernelFn fn = (swap ? swap_kernels : kernels)[p.resident_b ? 1 : 0][ksteps];
+  const bool det = stats && p.stat_ws;
+  KernelFn fn = (swap ? (det ? swap_det_kernels : swap_kernels) : kernels)[p.resident_b ? 1 : 0][ksteps];
   if (stats && !swap) {
     ABC_REQUIRE(p.resident_b && ksteps == 1, "abc_conv_igemm: internal: fused statistics variant");
-    fn = stats_kernel;
+    fn = det ? stats_det_kernel : stats_kernel;
   }
   fn<<<grid, kThreads, smem_bytes, st_>>>(tmap, p);
-  return launch_check(swap ? "conv_igemm_kernel<swap>" : "conv_igemm_kernel");
+  if (int rc = launch_check(swap ? "conv_igemm_kernel<swap>" : "conv_igemm_kernel")) return rc;
+  return det ? det_reduce(p.stat_ws, conv_stat_slots(gx), 2 * d->cout, det_out2(d->stat_sum, d->stat_sq, d->cout), 0, st_) : ABC_OK;
+}
+
+// Workspace of the deterministic fused statistics (AbcConvDesc.stat_ws): the grid.x of the launch above, 8 owners per CTA.
+extern "C" size_t abc_conv_stat_workspace_bytes(const AbcConvDesc* d) {
+  using namespace abc;
+  if (!d || d->cout <= 0 || d->n_tile <= 0) return 0;
+  const int n_tiles = (d->cout + d->n_tile - 1) / d->n_tile;
+  int sms = sm_count();
+  if (sms <= 0) sms = 148;
+  const int gx = sms / n_tiles < 1 ? 1 : sms / n_tiles;      // an upper bound of the launch's grid.x (it is capped by the groups)
+  return det_ws_bytes(conv_stat_slots(gx), 2ll * d->cout, sizeof(double));
 }

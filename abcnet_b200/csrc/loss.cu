@@ -11,6 +11,7 @@
 #include <cuda_bf16.h>
 
 #include "common.cuh"
+#include "det_slots.cuh"
 
 namespace abc {
 
@@ -95,8 +96,9 @@ __device__ __forceinline__ float ld_tgt(const void* base, size_t i, int f64) {
   return f64 ? static_cast<float>(static_cast<const double*>(base)[i]) : static_cast<const float*>(base)[i];
 }
 
-template <bool BWD, bool SUMS>
-__global__ void __launch_bounds__(kLossThreads) loss_kernel(const LossParams p) {
+// DET: the block totals go to slot blockIdx.x of ws [blocks][16] (det_slots.cuh) instead of fp64 atomics.
+template <bool BWD, bool SUMS, bool DET = false>
+__global__ void __launch_bounds__(kLossThreads) loss_kernel(const LossParams p, double* __restrict__ ws) {
   const long long gid = static_cast<long long>(blockIdx.x) * kLossThreads + threadIdx.x;
   const long long total = static_cast<long long>(p.N) * p.HW;
   float acc[16];
@@ -173,7 +175,8 @@ __global__ void __launch_bounds__(kLossThreads) loss_kernel(const LossParams p) 
     if (threadIdx.x < 16) {
       double v = 0.0;
       for (int w = 0; w < kLossThreads / 32; ++w) v += red[threadIdx.x][w];
-      if (v != 0.0) atomicAdd(p.sums + threadIdx.x, v);
+      if constexpr (DET) ws[det_slot_index(blockIdx.x, 16, threadIdx.x)] = v;
+      else if (v != 0.0) atomicAdd(p.sums + threadIdx.x, v);
     }
   }
 }
@@ -261,8 +264,8 @@ __device__ __forceinline__ float focal_softmax_c(const float* __restrict__ z, co
   return num;
 }
 
-template <bool BWD, bool SUMS>
-__global__ void __launch_bounds__(256) loss_kernel_v2(const LossParams p) {
+template <bool BWD, bool SUMS, bool DET = false>
+__global__ void __launch_bounds__(256) loss_kernel_v2(const LossParams p, double* __restrict__ ws) {
   constexpr int CT = 14, CC = 3, CH = 2, NB = 6;
   __shared__ float osum[4][kPx];
   __shared__ double red[16][8];
@@ -367,7 +370,8 @@ __global__ void __launch_bounds__(256) loss_kernel_v2(const LossParams p) {
     if (threadIdx.x < 16) {
       double v = 0.0;
       for (int w = 0; w < 8; ++w) v += red[threadIdx.x][w];
-      if (v != 0.0) atomicAdd(p.sums + threadIdx.x, v);
+      if constexpr (DET) ws[det_slot_index(blockIdx.x, 16, threadIdx.x)] = v;
+      else if (v != 0.0) atomicAdd(p.sums + threadIdx.x, v);
     }
   }
 }
@@ -384,6 +388,7 @@ struct LossP8Params {
   uint4* dz[8];
   int planes[8];
   double* dbias[8];
+  double* ws;         // DET: per-block slots [blocks][loss_elems(true, n_omega)] (det_slots.cuh)
 };
 
 __device__ __forceinline__ uint2 pack4_bf16(const float* v) {
@@ -415,10 +420,43 @@ __device__ __forceinline__ void store_small_head(uint4* __restrict__ base, int p
   }
 }
 
+// Deterministic form of the sparse bias-gradient atomics: the live lanes `lm` of a warp add their values of one channel in lane
+// order (usually none is non-zero, one ballot), and lane 0 adds the total to the warp's own shared accumulator.
+__device__ __forceinline__ void det_bias_add(double* acc, float v, unsigned lm) {
+  unsigned nz = __ballot_sync(lm, v != 0.f);
+  if (nz == 0u) return;
+  double t = 0.0;
+  while (nz) {
+    const int b = __ffs(nz) - 1;
+    nz &= nz - 1;
+    t += static_cast<double>(__shfl_sync(lm, v, b));
+  }
+  if ((threadIdx.x & 31) == 0) *acc += t;
+}
+
+// Shared memory that only the instantiations which call this declare (the default kernels keep their shared-memory layout).
+template <typename T, int N>
+__device__ __forceinline__ T* shared_array() {
+  __shared__ T a[N];
+  return a;
+}
+
+// DET: the bias gradients of heads 1-3 and 5-7 are summed per warp in shared memory (a thread group = two warps sees every
+// pixel of its channels), the block writes its slot of p.ws ([blocks][loss_elems(true, n_omega)], det_slots.cuh).
+template <bool DET = false>
 __global__ void __launch_bounds__(256) loss_kernel_v2_p8(const LossParams p, const LossP8Params o) {
   constexpr int CT = 14, CC = 3, CH = 2, NB = 6;
+  constexpr int kBiasCh = 19 + 8 * kLossMaxOmegaDet;            // heads 1, 2, 3 (14 + 3 + 2), then 5, 6, 7 (8 n_omega)
   __shared__ float osum[4][kPx];
   __shared__ double red[18][8];
+  double* bacc = nullptr;                                        // [2][kBiasCh]: one accumulator row per warp of a thread group
+  if constexpr (DET) {
+    bacc = shared_array<double, 2 * kBiasCh>();
+    for (int i = threadIdx.x; i < 2 * kBiasCh; i += 256) bacc[i] = 0.0;
+    __syncthreads();
+  }
+  double* wacc = bacc + ((threadIdx.x >> 5) & 1) * kBiasCh;
+  const int b5 = 19, b6 = 19 + NB * p.n_omega, b7 = b6 + p.n_omega;
   const int px = threadIdx.x & (kPx - 1), wg = threadIdx.x >> 6;
   const long long total = static_cast<long long>(p.N) * p.HW;
   const size_t hw = static_cast<size_t>(p.HW);
@@ -444,6 +482,7 @@ __global__ void __launch_bounds__(256) loss_kernel_v2_p8(const LossParams p, con
     __syncthreads();
     const float omega_tsum = osum[0][px] + osum[1][px] + osum[2][px] + osum[3][px];
     __syncthreads();
+    const unsigned lm = DET ? __ballot_sync(0xffffffffu, live) : 0u;    // live lanes: a prefix of the warp
     if (!live) continue;
     float d;
     if (wg == 0) {          // centre maps (dense terms): bias gradients through the block reduction
@@ -464,17 +503,26 @@ __global__ void __launch_bounds__(256) loss_kernel_v2_p8(const LossParams p, con
       const size_t oc = (n * CT) * hw + pix;
       acc[ABC_L_TYPE] += focal_softmax_core<CT, true>(p.z[1] + oc, static_cast<const float*>(p.t[1]) + oc, hw, p.type_w, &ts, 1.f, dzv);
       acc[8 + ABC_L_TYPE] += ts;
-      store_small_head<CT>(o.dz[1], o.planes[1], n, hw, pix, dzv, o.dbias[1], true);
+      store_small_head<CT>(o.dz[1], o.planes[1], n, hw, pix, dzv, o.dbias[1], !DET);
+      if constexpr (DET)
+#pragma unroll
+        for (int c = 0; c < CT; ++c) det_bias_add(wacc + c, dzv[c], lm);
     } else if (wg == 2) {   // charges, H counts
       float ts, dzc[CC], dzh[CH];
       size_t oc = (n * CC) * hw + pix;
       acc[ABC_L_CHARGE] += focal_softmax_core<CC, true>(p.z[2] + oc, static_cast<const float*>(p.t[2]) + oc, hw, nullptr, &ts, 1.f, dzc);
       acc[8 + ABC_L_CHARGE] += ts;
-      store_small_head<CC>(o.dz[2], o.planes[2], n, hw, pix, dzc, o.dbias[2], true);
+      store_small_head<CC>(o.dz[2], o.planes[2], n, hw, pix, dzc, o.dbias[2], !DET);
       oc = (n * CH) * hw + pix;
       acc[ABC_L_HS] += focal_softmax_core<CH, true>(p.z[3] + oc, static_cast<const float*>(p.t[3]) + oc, hw, nullptr, &ts, 1.f, dzh);
       acc[8 + ABC_L_HS] += ts;
-      store_small_head<CH>(o.dz[3], o.planes[3], n, hw, pix, dzh, o.dbias[3], true);
+      store_small_head<CH>(o.dz[3], o.planes[3], n, hw, pix, dzh, o.dbias[3], !DET);
+      if constexpr (DET) {
+#pragma unroll
+        for (int c = 0; c < CC; ++c) det_bias_add(wacc + CT + c, dzc[c], lm);
+#pragma unroll
+        for (int c = 0; c < CH; ++c) det_bias_add(wacc + CT + CC + c, dzh[c], lm);
+      }
     } else {                // the least loaded group writes the channel padding of the omega-indexed heads
       const uint2 zero2 = make_uint2(0, 0);
       for (int c0 = NB * p.n_omega; c0 < o.planes[5] * 8; c0 += 4)
@@ -500,7 +548,7 @@ __global__ void __launch_bounds__(256) loss_kernel_v2_p8(const LossParams p, con
         if (tsum != 0.f) {
 #pragma unroll
           for (int t = 0; t < NB; ++t)
-            if (dzv[t] != 0.f) atomicAdd(o.dbias[5] + t * p.n_omega + w + k, static_cast<double>(dzv[t]));
+            if (!DET && dzv[t] != 0.f) atomicAdd(o.dbias[5] + t * p.n_omega + w + k, static_cast<double>(dzv[t]));
           const float zr = p.z[6][ow + wo];
           const float tr = ld_tgt(p.t[6], ow + wo, p.tgt_f64);
           const float diff = fabsf(zr) - tr;
@@ -508,14 +556,20 @@ __global__ void __launch_bounds__(256) loss_kernel_v2_p8(const LossParams p, con
           const float sd = diff > 0.f ? 1.f : (diff < 0.f ? -1.f : 0.f);
           const float sz = zr > 0.f ? 1.f : (zr < 0.f ? -1.f : 0.f);
           rr[k] = sd * sz * tsum;
-          if (rr[k] != 0.f) atomicAdd(o.dbias[6] + w + k, static_cast<double>(rr[k]));
+          if (!DET && rr[k] != 0.f) atomicAdd(o.dbias[6] + w + k, static_cast<double>(rr[k]));
         }
         oo[k] = 0.f;
         if (omega_tsum != 0.f) {
           const float tw = ld_tgt(p.t[7], ow + wo, p.tgt_f64);
           acc[ABC_L_OMEGA] += omega_tsum * focal_sigmoid<true>(p.z[7][ow + wo], tw, &d);
           oo[k] = omega_tsum * d;
-          if (oo[k] != 0.f) atomicAdd(o.dbias[7] + w + k, static_cast<double>(oo[k]));
+          if (!DET && oo[k] != 0.f) atomicAdd(o.dbias[7] + w + k, static_cast<double>(oo[k]));
+        }
+        if constexpr (DET) {              // outside the per-lane branches: every live lane of the warp takes part
+#pragma unroll
+          for (int t = 0; t < NB; ++t) det_bias_add(wacc + b5 + t * p.n_omega + w + k, bt[t][k], lm);
+          det_bias_add(wacc + b6 + w + k, rr[k], lm);
+          det_bias_add(wacc + b7 + w + k, oo[k], lm);
         }
       }
 #pragma unroll
@@ -537,6 +591,16 @@ __global__ void __launch_bounds__(256) loss_kernel_v2_p8(const LossParams p, con
     if (lane == 0) red[i][warp] = v;
   }
   __syncthreads();
+  if constexpr (DET) {
+    const int n = loss_elems(true, p.n_omega);
+    if (threadIdx.x < 18) {
+      double v = 0.0;
+      for (int w = 0; w < 8; ++w) v += red[threadIdx.x][w];
+      o.ws[det_slot_index(blockIdx.x, n, threadIdx.x)] = v;
+    }
+    for (int c = threadIdx.x; c < 19 + 8 * p.n_omega; c += 256) o.ws[det_slot_index(blockIdx.x, n, 18 + c)] = bacc[c] + bacc[kBiasCh + c];
+    return;
+  }
   if (threadIdx.x < 18) {
     double v = 0.0;
     for (int w = 0; w < 8; ++w) v += red[threadIdx.x][w];
@@ -544,18 +608,26 @@ __global__ void __launch_bounds__(256) loss_kernel_v2_p8(const LossParams p, con
   }
 }
 
-template <bool BWD, bool SUMS>
-static int launch_loss(const LossParams& p, cudaStream_t st) {
+static bool is_v2(const LossParams& p) { return p.c_type == 14 && p.c_charge == 3 && p.c_hs == 2 && p.n_btype == 6 && p.n_omega >= 4; }
+
+// blocks of the loss launches: the v2 kernels (and loss_kernel_v2_p8) stride over 64-pixel tiles, the generic one does not
+static unsigned loss_blocks(const LossParams& p) {
   const long long total = static_cast<long long>(p.N) * p.HW;
-  if (p.c_type == 14 && p.c_charge == 3 && p.c_hs == 2 && p.n_btype == 6 && p.n_omega >= 4) {
-    long long tiles = (total + kPx - 1) / kPx;
-    const long long cap = 148ll * 8 * 4;
-    const unsigned blocks = static_cast<unsigned>(tiles < cap ? tiles : cap);
-    loss_kernel_v2<BWD, SUMS><<<blocks, 256, 0, st>>>(p);
+  if (is_v2(p)) {
+    const long long tiles = (total + kPx - 1) / kPx, cap = 148ll * 8 * 4;
+    return static_cast<unsigned>(tiles < cap ? tiles : cap);
+  }
+  return static_cast<unsigned>((total + kLossThreads - 1) / kLossThreads);
+}
+
+template <bool BWD, bool SUMS, bool DET = false>
+static int launch_loss(const LossParams& p, cudaStream_t st, double* ws = nullptr) {
+  const unsigned blocks = loss_blocks(p);
+  if (is_v2(p)) {
+    loss_kernel_v2<BWD, SUMS, DET><<<blocks, 256, 0, st>>>(p, ws);
     return launch_check("loss_kernel_v2");
   }
-  const unsigned blocks = static_cast<unsigned>((total + kLossThreads - 1) / kLossThreads);
-  loss_kernel<BWD, SUMS><<<blocks, kLossThreads, 0, st>>>(p);
+  loss_kernel<BWD, SUMS, DET><<<blocks, kLossThreads, 0, st>>>(p, ws);
   return launch_check("loss_kernel");
 }
 
@@ -596,6 +668,10 @@ extern "C" int abc_loss_partials(const AbcLossDesc* d, void* stream) {
   for (int i = 0; fused && i < 8; ++i) fused = d->dlogits[i] != nullptr;
   if (int rc = fill(d, &p, fused, true)) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (d->ws) {                   // deterministic: block totals to slots, summed in block order
+    if (int rc = fused ? launch_loss<true, true, true>(p, st, d->ws) : launch_loss<false, true, true>(p, st, d->ws)) return rc;
+    return det_reduce(d->ws, static_cast<int>(loss_blocks(p)), 16, det_out1(p.sums, 16), 0, st);
+  }
   ABC_CUDA(cudaMemsetAsync(p.sums, 0, 16 * sizeof(double), st));
   return fused ? launch_loss<true, true>(p, st) : launch_loss<false, true>(p, st);
 }
@@ -627,11 +703,36 @@ extern "C" int abc_loss_partials_p8(const AbcLossDesc* d, const AbcLossP8Out* ou
     o.dz[k] = static_cast<uint4*>(out->dz[k]);
     o.planes[k] = out->planes[k];
     o.dbias[k] = out->dbias[k];
-    ABC_CUDA(cudaMemsetAsync(out->dbias[k], 0, chans[k] * sizeof(double), st));
+    if (!d->ws) ABC_CUDA(cudaMemsetAsync(out->dbias[k], 0, chans[k] * sizeof(double), st));
+  }
+  const unsigned blocks = loss_blocks(p);
+  if (d->ws) {                   // deterministic: sums and bias gradients per block to slots, summed in block order
+    ABC_REQUIRE(p.n_omega <= kLossMaxOmegaDet, "abc_loss_partials_p8: deterministic mode supports n_omega <= %d", kLossMaxOmegaDet);
+    o.ws = d->ws;
+    loss_kernel_v2_p8<true><<<blocks, 256, 0, st>>>(p, o);
+    if (int rc = launch_check("loss_kernel_v2_p8")) return rc;
+    DetOut r{};
+    const int order[9] = {-1, 0, 4, 1, 2, 3, 5, 6, 7};            // the slot layout of loss_elems(true, n_omega)
+    int end = 0;
+    for (int i = 0; i < 9; ++i) {
+      end += order[i] < 0 ? 16 : chans[order[i]];
+      r.ptr[i] = order[i] < 0 ? static_cast<void*>(p.sums) : static_cast<void*>(o.dbias[order[i]]);
+      r.end[i] = end;
+    }
+    r.count = 9;
+    return det_reduce(d->ws, static_cast<int>(blocks), loss_elems(true, p.n_omega), r, 0, st);
   }
   ABC_CUDA(cudaMemsetAsync(p.sums, 0, 16 * sizeof(double), st));
-  const long long total = static_cast<long long>(p.N) * p.HW;
-  const long long tiles = (total + kPx - 1) / kPx, cap = 148ll * 8 * 4;
-  loss_kernel_v2_p8<<<static_cast<unsigned>(tiles < cap ? tiles : cap), 256, 0, st>>>(p, o);
+  loss_kernel_v2_p8<<<blocks, 256, 0, st>>>(p, o);
   return launch_check("loss_kernel_v2_p8");
+}
+
+// Workspace of the deterministic loss passes (AbcLossDesc.ws): abc_loss_partials (p8 = 0) or abc_loss_partials_p8 (p8 = 1).
+extern "C" size_t abc_loss_workspace_bytes(const AbcLossDesc* d, int p8) {
+  using namespace abc;
+  if (!d || d->N <= 0 || d->H <= 0 || d->W <= 0) return 0;
+  LossParams p{};
+  p.N = d->N; p.HW = d->H * d->W;
+  p.c_type = d->c_type; p.c_charge = d->c_charge; p.c_hs = d->c_hs; p.n_omega = d->n_omega; p.n_btype = d->n_btype;
+  return det_ws_bytes(loss_blocks(p), loss_elems(p8 != 0, d->n_omega), sizeof(double));
 }

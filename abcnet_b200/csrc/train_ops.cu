@@ -12,6 +12,7 @@
 
 #include "bn_launch.cuh"
 #include "common.cuh"
+#include "det_slots.cuh"
 #include "p8_device.cuh"
 
 namespace abc {
@@ -70,15 +71,26 @@ __device__ __forceinline__ double block_sum(F v, double (*red)[8]) {
   return t;
 }
 
-// block-wide sum of 16 per-thread fp32 partials (8 channels x 2 statistics) -> fp64 atomics
+// block-wide sum of 16 per-thread fp32 partials (8 channels x 2 statistics) -> fp64 atomics, or (DET) the block's slot of
+// ws [slots][2 C] (the C first statistics, then the C second ones; C = 8 gridDim.y)
+template <bool DET>
 __device__ __forceinline__ void block_reduce16(const float* a, const float* b, double* __restrict__ ga, double* __restrict__ gb,
-                                               int c0, double (*red)[8]) {
+                                               int c0, double (*red)[8], double* __restrict__ ws) {
   const double t = block_sum<16>([&](int i) { return i < 8 ? a[i] : b[i - 8]; }, red);
-  if (threadIdx.x < 16) atomicAdd((threadIdx.x < 8 ? ga : gb) + c0 + (threadIdx.x & 7), t);
+  if (threadIdx.x < 16) {
+    if constexpr (DET) {
+      const int C = gridDim.y * 8;
+      ws[det_slot_index(bn_slot(blockIdx.x, blockIdx.z, gridDim.x), 2 * C, (threadIdx.x < 8 ? 0 : C) + c0 + (threadIdx.x & 7))] = t;
+    } else {
+      atomicAdd((threadIdx.x < 8 ? ga : gb) + c0 + (threadIdx.x & 7), t);
+    }
+  }
 }
 
 // ------------------------------------------------------------------------------------------- statistics
-__global__ void __launch_bounds__(kBnThreads) bn_stats_kernel(P8View z, int HW, double* __restrict__ sum, double* __restrict__ sumsq) {
+template <bool DET>
+__global__ void __launch_bounds__(kBnThreads) bn_stats_kernel(P8View z, int HW, double* __restrict__ sum, double* __restrict__ sumsq,
+                                                              double* __restrict__ ws) {
   const int plane = blockIdx.y, n = blockIdx.z;
   const uint4* __restrict__ zb = z.ptr + (static_cast<size_t>(n) * z.planes + z.plane_off + plane) * HW;
   float s[8], q[8];
@@ -107,7 +119,7 @@ __global__ void __launch_bounds__(kBnThreads) bn_stats_kernel(P8View z, int HW, 
     }
   }
   __shared__ double red[16][8];
-  block_reduce16(s, q, sum, sumsq, plane * 8, red);
+  block_reduce16<DET>(s, q, sum, sumsq, plane * 8, red, ws);
 }
 
 __global__ void bn_finalize_kernel(const double* __restrict__ sum, const double* __restrict__ sumsq, int C, double count,
@@ -230,6 +242,7 @@ struct BnActBwdParams {
   double count;
   const float* gscale;      // [C] or null: per-channel factor on dA / dP (everything downstream is linear in g)
   const unsigned char* drop_mask;   // the mask bytes bn_act wrote (null: regenerate the mask from the counter-based hash)
+  double* ws;               // deterministic reduce: [slots][2 C] block sums (det_slots.cuh)
 };
 
 // Gradient g wrt the BatchNorm output for one pixel (8 channels): g = dA * act'(pre) * dropout scale.
@@ -279,7 +292,7 @@ __device__ __forceinline__ void bwd_block4(const BnActBwdParams& p, const float 
 }
 
 // reduce: s1 = sum g, s2 = sum g * xhat (xhat = (z - mean) * invstd, accumulated as sum g*z and combined per block)
-template <bool POOL, int MINB = 2>
+template <bool POOL, int MINB = 2, bool DET = false>
 __global__ void __launch_bounds__(kBnThreads, MINB) bn_act_bwd_reduce_kernel(const BnActBwdParams p) {
   const int plane = blockIdx.y, n = blockIdx.z;
   const int HW = p.H * p.W;
@@ -371,7 +384,7 @@ __global__ void __launch_bounds__(kBnThreads, MINB) bn_act_bwd_reduce_kernel(con
 #pragma unroll
   for (int i = 0; i < 8; ++i) s2[i] = istd[i] * (t2[i] - mean[i] * s1[i]);
   __shared__ double red[16][8];
-  block_reduce16(s1, s2, p.s1, p.s2, plane * 8, red);
+  block_reduce16<DET>(s1, s2, p.s1, p.s2, plane * 8, red, p.ws);
 }
 
 // apply: dz = scale * (g - s1/M - xhat * s2/M) = scale * g + cb * z + ca  with per-channel constants ca, cb
@@ -492,9 +505,10 @@ __global__ void __launch_bounds__(256) nchw_to_p8_kernel(const float* __restrict
 
 // fp32 NCHW -> bf16 P8 with an optional device-side scale, zero-filled padding planes and per-channel sums of the scaled
 // values (the bias gradient of the 1x1 head convolutions): one pass over the loss gradient instead of three.
+template <bool DET>
 __global__ void __launch_bounds__(kBnThreads) nchw_to_p8_ex_kernel(const float* __restrict__ src, uint4* __restrict__ dst, int C,
                                                                    int HW, int dst_planes, const float* __restrict__ scale,
-                                                                   double* __restrict__ dbias) {
+                                                                   double* __restrict__ dbias, double* __restrict__ ws) {
   const int plane = blockIdx.y, n = blockIdx.z;
   const float sc = scale ? *scale : 1.f;
   const float* __restrict__ sb = src + (static_cast<size_t>(n) * C + plane * 8) * HW;
@@ -515,16 +529,22 @@ __global__ void __launch_bounds__(kBnThreads) nchw_to_p8_ex_kernel(const float* 
   if (dbias != nullptr && nvalid > 0) {      // block-uniform condition
     __shared__ double red[8][8];
     const double t = block_sum<8>([&](int i) { return s[i]; }, red);
-    if (threadIdx.x < nvalid) atomicAdd(dbias + plane * 8 + threadIdx.x, t);
+    if (threadIdx.x < nvalid) {
+      if constexpr (DET) ws[det_slot_index(bn_slot(blockIdx.x, blockIdx.z, gridDim.x), C, plane * 8 + threadIdx.x)] = t;   // ws [slots][C]
+      else atomicAdd(dbias + plane * 8 + threadIdx.x, t);
+    }
   }
 }
 
 // dW[16][9], db-free: gradient of the first 1 -> 16 convolution (no dgrad: the image needs no gradient)
 // img_cstride: channels of the image tensor (1 for the binary stem); img points at the channel to differentiate.
 // dw_costride: floats between consecutive output channels in dw ([16][cin][9]: cin * 9).
-template <typename T>
+// DET: the 8 warp totals go to fixed shared slots, summed in warp order, and the block total is stored to slot blockIdx.x of
+// ws [blocks][16 * dw_costride] (ws offset like dw) instead of the shared- and global-memory atomics.
+template <typename T, bool DET = false>
 __global__ void __launch_bounds__(256) conv_c1_wgrad_kernel(const T* __restrict__ img, P8View dz, int N, int H, int W,
-                                                            float* __restrict__ dw, int img_cstride, int dw_costride) {
+                                                            float* __restrict__ dw, int img_cstride, int dw_costride,
+                                                            float* __restrict__ ws) {
   __shared__ float acc[144];
   if (threadIdx.x < 144) acc[threadIdx.x] = 0.f;
   __syncthreads();
@@ -553,6 +573,24 @@ __global__ void __launch_bounds__(256) conv_c1_wgrad_kernel(const T* __restrict_
 #pragma unroll
       for (int k = 0; k < 9; ++k) loc[co * 9 + k] = fmaf(g[co], t[k], loc[co * 9 + k]);
   }
+  if constexpr (DET) {
+    __shared__ float part[8][144];
+#pragma unroll
+    for (int i = 0; i < 144; ++i) {
+      float v = loc[i];
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+      if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5][i] = v;
+    }
+    __syncthreads();
+    if (threadIdx.x < 144) {
+      float t = 0.f;
+#pragma unroll
+      for (int w = 0; w < 8; ++w) t += part[w][threadIdx.x];
+      ws[static_cast<size_t>(blockIdx.x) * 16 * dw_costride + (threadIdx.x / 9) * dw_costride + threadIdx.x % 9] = t;
+    }
+    return;
+  }
 #pragma unroll
   for (int i = 0; i < 144; ++i) {
     float v = loc[i];
@@ -569,9 +607,9 @@ __global__ void __launch_bounds__(256) conv_c1_wgrad_kernel(const T* __restrict_
 // 32 lanes together gather the 3 x 3 x 16 neighbourhood of dz: slot s = lane + 32 j -> (tap = s / 16, channel = s % 16), so 16
 // consecutive lanes read the 32 contiguous bytes of one pixel. Work is proportional to the ink count (0.84 M of 16.8 M pixels
 // per 64-image batch) instead of 144 FMAs for every pixel; a dense image degrades gracefully to the cost of the dense kernel.
-template <typename T>
+template <typename T, bool DET = false>
 __global__ void __launch_bounds__(256) conv_c1_wgrad_sparse_kernel(const T* __restrict__ img, P8View dz, int N, int H, int W,
-                                                                   float* __restrict__ dw) {
+                                                                   float* __restrict__ dw, float* __restrict__ ws) {
   __shared__ float acc[144];
   if (threadIdx.x < 144) acc[threadIdx.x] = 0.f;
   __syncthreads();
@@ -612,6 +650,22 @@ __global__ void __launch_bounds__(256) conv_c1_wgrad_sparse_kernel(const T* __re
       }
     }
   }
+  if constexpr (DET) {                    // as in conv_c1_wgrad_kernel: warp slots in shared memory, block slots in ws [blocks][144]
+    __shared__ float part[8][144];
+#pragma unroll
+    for (int j = 0; j < 5; ++j) {
+      const int sl = lane + 32 * j;
+      if (sl < 144) part[threadIdx.x >> 5][(sl & 15) * 9 + (sl >> 4)] = loc[j];
+    }
+    __syncthreads();
+    if (threadIdx.x < 144) {
+      float t = 0.f;
+#pragma unroll
+      for (int w = 0; w < 8; ++w) t += part[w][threadIdx.x];
+      ws[static_cast<size_t>(blockIdx.x) * 144 + threadIdx.x] = t;
+    }
+    return;
+  }
 #pragma unroll
   for (int j = 0; j < 5; ++j) {
     const int sl = lane + 32 * j;
@@ -647,19 +701,41 @@ static int p8_check(const void* ptr, int planes, int plane_off, int cplanes, con
   return ABC_OK;
 }
 
-extern "C" int abc_bn_stats(const void* z, int N, int H, int W, int planes, int plane_off, int C, double* sum, double* sumsq,
-                            void* stream) {
+// ws == nullptr: fp64 atomics; else the deterministic slots (abc_bn_stats_workspace_bytes) and their fixed-order sum
+static int bn_stats_launch(const void* z, int N, int H, int W, int planes, int plane_off, int C, double* sum, double* sumsq,
+                           double* ws, void* stream) {
   if (int rc = device_check()) return rc;
   ABC_REQUIRE(C >= 8 && C % 8 == 0 && N > 0 && N <= 65535 && H > 0 && W > 0 && sum && sumsq, "abc_bn_stats: bad arguments");
   ABC_REQUIRE(static_cast<long long>(H) * W < (1ll << 30), "abc_bn_stats: image too large");
   if (int rc = p8_check(z, planes, plane_off, C / 8, "abc_bn_stats")) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  ABC_CUDA(cudaMemsetAsync(sum, 0, C * sizeof(double), st));
-  ABC_CUDA(cudaMemsetAsync(sumsq, 0, C * sizeof(double), st));
   P8View v{static_cast<const uint4*>(z), planes, plane_off};
   const BnLaunch l = bn_launch_config(BnPass::kStats, N, C / 8, H, W);
-  bn_stats_kernel<<<l.grid, l.block, 0, st>>>(v, H * W, sum, sumsq);
+  if (ws) {
+    bn_stats_kernel<true><<<l.grid, l.block, 0, st>>>(v, H * W, sum, sumsq, ws);
+    if (int rc = launch_check("bn_stats_kernel")) return rc;
+    return det_reduce(ws, bn_slots(l), 2 * C, det_out2(sum, sumsq, C), 0, st);
+  }
+  ABC_CUDA(cudaMemsetAsync(sum, 0, C * sizeof(double), st));
+  ABC_CUDA(cudaMemsetAsync(sumsq, 0, C * sizeof(double), st));
+  bn_stats_kernel<false><<<l.grid, l.block, 0, st>>>(v, H * W, sum, sumsq, nullptr);
   return launch_check("bn_stats_kernel");
+}
+
+extern "C" int abc_bn_stats(const void* z, int N, int H, int W, int planes, int plane_off, int C, double* sum, double* sumsq,
+                            void* stream) {
+  return bn_stats_launch(z, N, H, W, planes, plane_off, C, sum, sumsq, nullptr, stream);
+}
+
+extern "C" int abc_bn_stats_det(const void* z, int N, int H, int W, int planes, int plane_off, int C, double* sum, double* sumsq,
+                                double* ws, void* stream) {
+  ABC_REQUIRE(ws != nullptr, "abc_bn_stats_det: null workspace");
+  return bn_stats_launch(z, N, H, W, planes, plane_off, C, sum, sumsq, ws, stream);
+}
+
+extern "C" size_t abc_bn_stats_workspace_bytes(int N, int H, int W, int C) {
+  if (N <= 0 || H <= 0 || W <= 0 || C < 8) return 0;
+  return det_ws_bytes(bn_slots(bn_launch_config(BnPass::kStats, N, C / 8, H, W)), 2ll * C, sizeof(double));
 }
 
 extern "C" int abc_bn_finalize(const double* sum, const double* sumsq, int C, double count, const float* gamma, const float* beta,
@@ -730,24 +806,37 @@ extern "C" int abc_bn_act_backward(const AbcBnActBwdDesc* d, void* stream) {
   p.gscale = d->gscale;
   p.drop_mask = static_cast<const unsigned char*>(d->drop_mask);
   ABC_REQUIRE((reinterpret_cast<uintptr_t>(d->gscale) & 15) == 0, "abc_bn_act_backward: gscale must be 16-byte aligned");
-  ABC_CUDA(cudaMemsetAsync(d->s1, 0, d->C * sizeof(double), st));
-  ABC_CUDA(cudaMemsetAsync(d->s2, 0, d->C * sizeof(double), st));
   const BnLaunch l = bn_launch_config(d->dP ? BnPass::kPool : BnPass::kPixels, d->N, cp, d->H, d->W);
-  if (d->dP) {
-    bn_act_bwd_reduce_kernel<true><<<l.grid, l.block, 0, st>>>(p);
+  p.ws = d->ws;
+  // resident blocks per SM (register cap) of the two passes: ABCNET_BN_MINB = <reduce digit><apply digit>, read once
+  static const int minb = [] { const char* e = getenv("ABCNET_BN_MINB"); return e ? atoi(e) : 34; }();
+  if (d->ws) {               // deterministic: block sums to slots, fixed-order sum into s1 / s2, then the same apply pass
+    if (d->dP) bn_act_bwd_reduce_kernel<true, 2, true><<<l.grid, l.block, 0, st>>>(p);
+    else bn_act_bwd_reduce_kernel<false, 3, true><<<l.grid, l.block, 0, st>>>(p);
     if (int rc = launch_check("bn_act_bwd_reduce_kernel")) return rc;
-    bn_act_bwd_apply_kernel<true><<<l.grid, l.block, 0, st>>>(p);
+    if (int rc = det_reduce(d->ws, bn_slots(l), 2 * d->C, det_out2(d->s1, d->s2, d->C), 0, st)) return rc;
   } else {
-    // resident blocks per SM (register cap) of the two passes: ABCNET_BN_MINB = <reduce digit><apply digit>, read once
-    static const int minb = [] { const char* e = getenv("ABCNET_BN_MINB"); return e ? atoi(e) : 34; }();
-    if (minb / 10 == 4) bn_act_bwd_reduce_kernel<false, 4><<<l.grid, l.block, 0, st>>>(p);
+    ABC_CUDA(cudaMemsetAsync(d->s1, 0, d->C * sizeof(double), st));
+    ABC_CUDA(cudaMemsetAsync(d->s2, 0, d->C * sizeof(double), st));
+    if (d->dP) bn_act_bwd_reduce_kernel<true><<<l.grid, l.block, 0, st>>>(p);
+    else if (minb / 10 == 4) bn_act_bwd_reduce_kernel<false, 4><<<l.grid, l.block, 0, st>>>(p);
     else bn_act_bwd_reduce_kernel<false, 3><<<l.grid, l.block, 0, st>>>(p);
     if (int rc = launch_check("bn_act_bwd_reduce_kernel")) return rc;
+  }
+  if (d->dP) {
+    bn_act_bwd_apply_kernel<true><<<l.grid, l.block, 0, st>>>(p);
+  } else {
     if (minb % 10 == 4) bn_act_bwd_apply_kernel<false, 4><<<l.grid, l.block, 0, st>>>(p);
     else if (minb % 10 == 3) bn_act_bwd_apply_kernel<false, 3><<<l.grid, l.block, 0, st>>>(p);
     else bn_act_bwd_apply_kernel<false, 2><<<l.grid, l.block, 0, st>>>(p);
   }
   return launch_check("bn_act_bwd_apply_kernel");
+}
+
+extern "C" size_t abc_bn_act_backward_workspace_bytes(const AbcBnActBwdDesc* d) {
+  if (!d || d->N <= 0 || d->H <= 0 || d->W <= 0 || d->C < 8) return 0;
+  const BnLaunch l = bn_launch_config(d->dP ? BnPass::kPool : BnPass::kPixels, d->N, d->C / 8, d->H, d->W);
+  return det_ws_bytes(bn_slots(l), 2ll * d->C, sizeof(double));
 }
 
 extern "C" int abc_nchw_to_p8(const float* src, void* dst, int N, int C, int H, int W, void* stream) {
@@ -760,17 +849,38 @@ extern "C" int abc_nchw_to_p8(const float* src, void* dst, int N, int C, int H, 
   return launch_check("nchw_to_p8_kernel");
 }
 
-extern "C" int abc_nchw_to_p8_ex(const float* src, void* dst, int N, int C, int H, int W, int dst_planes, const float* scale,
-                                 double* dbias, void* stream) {
+static int nchw_to_p8_ex_launch(const float* src, void* dst, int N, int C, int H, int W, int dst_planes, const float* scale,
+                                double* dbias, double* ws, void* stream) {
   if (int rc = device_check()) return rc;
   ABC_REQUIRE(src && dst && N > 0 && N <= 65535 && C > 0 && H > 0 && W > 0, "abc_nchw_to_p8_ex: bad arguments");
   ABC_REQUIRE(dst_planes >= (C + 7) / 8 && dst_planes <= 65535, "abc_nchw_to_p8_ex: dst_planes=%d too small for C=%d", dst_planes, C);
   ABC_REQUIRE((reinterpret_cast<uintptr_t>(dst) & 15) == 0, "abc_nchw_to_p8_ex: dst must be 16-byte aligned");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (dbias) ABC_CUDA(cudaMemsetAsync(dbias, 0, C * sizeof(double), st));
   const BnLaunch l = bn_launch_config(BnPass::kPixels, N, dst_planes, H, W);
-  nchw_to_p8_ex_kernel<<<l.grid, l.block, 0, st>>>(src, static_cast<uint4*>(dst), C, H * W, dst_planes, scale, dbias);
+  if (ws && dbias) {
+    nchw_to_p8_ex_kernel<true><<<l.grid, l.block, 0, st>>>(src, static_cast<uint4*>(dst), C, H * W, dst_planes, scale, dbias, ws);
+    if (int rc = launch_check("nchw_to_p8_ex_kernel")) return rc;
+    return det_reduce(ws, bn_slots(l), C, det_out1(dbias, C), 0, st);
+  }
+  if (dbias) ABC_CUDA(cudaMemsetAsync(dbias, 0, C * sizeof(double), st));
+  nchw_to_p8_ex_kernel<false><<<l.grid, l.block, 0, st>>>(src, static_cast<uint4*>(dst), C, H * W, dst_planes, scale, dbias, nullptr);
   return launch_check("nchw_to_p8_ex_kernel");
+}
+
+extern "C" int abc_nchw_to_p8_ex(const float* src, void* dst, int N, int C, int H, int W, int dst_planes, const float* scale,
+                                 double* dbias, void* stream) {
+  return nchw_to_p8_ex_launch(src, dst, N, C, H, W, dst_planes, scale, dbias, nullptr, stream);
+}
+
+extern "C" int abc_nchw_to_p8_ex_det(const float* src, void* dst, int N, int C, int H, int W, int dst_planes, const float* scale,
+                                     double* dbias, double* ws, void* stream) {
+  ABC_REQUIRE(ws != nullptr, "abc_nchw_to_p8_ex_det: null workspace");
+  return nchw_to_p8_ex_launch(src, dst, N, C, H, W, dst_planes, scale, dbias, ws, stream);
+}
+
+extern "C" size_t abc_nchw_to_p8_ex_workspace_bytes(int N, int C, int H, int W, int dst_planes) {
+  if (N <= 0 || C <= 0 || H <= 0 || W <= 0 || dst_planes <= 0) return 0;
+  return det_ws_bytes(bn_slots(bn_launch_config(BnPass::kPixels, N, dst_planes, H, W)), C, sizeof(double));
 }
 
 extern "C" int abc_channel_sum(const void* x, int N, int H, int W, int planes, int plane_off, int C, double* sum, double* sumsq_scratch,
@@ -778,45 +888,99 @@ extern "C" int abc_channel_sum(const void* x, int N, int H, int W, int planes, i
   return abc_bn_stats(x, N, H, W, planes, plane_off, C, sum, sumsq_scratch, stream);
 }
 
-extern "C" int abc_conv3x3_c1_wgrad(const void* img, int img_is_u8, const void* dz, int dz_planes, int dz_plane_off, int N, int H, int W,
-                                    float* dw, void* stream) {
+extern "C" int abc_channel_sum_det(const void* x, int N, int H, int W, int planes, int plane_off, int C, double* sum, double* sumsq_scratch,
+                                   double* ws, void* stream) {
+  return abc_bn_stats_det(x, N, H, W, planes, plane_off, C, sum, sumsq_scratch, ws, stream);
+}
+
+// ws == nullptr: atomics into the zeroed dw; else per-block slots (abc_conv3x3_wgrad_workspace_bytes) summed into dw in block order
+static int c1_wgrad_launch(const void* img, int img_is_u8, const void* dz, int dz_planes, int dz_plane_off, int N, int H, int W,
+                           float* dw, float* ws, void* stream) {
   if (int rc = device_check()) return rc;
   ABC_REQUIRE(img && dw && N > 0 && H > 0 && W > 0, "abc_conv3x3_c1_wgrad: bad arguments");
   if (int rc = p8_check(dz, dz_planes, dz_plane_off, 2, "abc_conv3x3_c1_wgrad(dz)")) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  ABC_CUDA(cudaMemsetAsync(dw, 0, 144 * sizeof(float), st));
+  if (!ws) ABC_CUDA(cudaMemsetAsync(dw, 0, 144 * sizeof(float), st));
   P8View v{static_cast<const uint4*>(dz), dz_planes, dz_plane_off};
   static const bool dense = getenv("ABCNET_C1_WGRAD_DENSE") != nullptr;      // the 144-FMA-per-pixel kernel (kept for comparison)
   if (!dense) {
-    const int blocks = 148 * 8;
+    const int blocks = kC1WgradBlocksSparse;
+    if (ws) {
+      if (img_is_u8)
+        conv_c1_wgrad_sparse_kernel<uint8_t, true><<<blocks, 256, 0, st>>>(static_cast<const uint8_t*>(img), v, N, H, W, dw, ws);
+      else
+        conv_c1_wgrad_sparse_kernel<float, true><<<blocks, 256, 0, st>>>(static_cast<const float*>(img), v, N, H, W, dw, ws);
+      if (int rc = launch_check("conv_c1_wgrad_sparse_kernel")) return rc;
+      return det_reduce(ws, blocks, 144, det_out1(dw, 144), 0, st);
+    }
     if (img_is_u8)
-      conv_c1_wgrad_sparse_kernel<uint8_t><<<blocks, 256, 0, st>>>(static_cast<const uint8_t*>(img), v, N, H, W, dw);
+      conv_c1_wgrad_sparse_kernel<uint8_t><<<blocks, 256, 0, st>>>(static_cast<const uint8_t*>(img), v, N, H, W, dw, nullptr);
     else
-      conv_c1_wgrad_sparse_kernel<float><<<blocks, 256, 0, st>>>(static_cast<const float*>(img), v, N, H, W, dw);
+      conv_c1_wgrad_sparse_kernel<float><<<blocks, 256, 0, st>>>(static_cast<const float*>(img), v, N, H, W, dw, nullptr);
     return launch_check("conv_c1_wgrad_sparse_kernel");
   }
-  const int blocks = 148 * 4;
+  const int blocks = kC1WgradBlocksDense;
+  if (ws) {
+    if (img_is_u8)
+      conv_c1_wgrad_kernel<uint8_t, true><<<blocks, 256, 0, st>>>(static_cast<const uint8_t*>(img), v, N, H, W, dw, 1, 9, ws);
+    else
+      conv_c1_wgrad_kernel<float, true><<<blocks, 256, 0, st>>>(static_cast<const float*>(img), v, N, H, W, dw, 1, 9, ws);
+    if (int rc = launch_check("conv_c1_wgrad_kernel")) return rc;
+    return det_reduce(ws, blocks, 144, det_out1(dw, 144), 0, st);
+  }
   if (img_is_u8)
-    conv_c1_wgrad_kernel<uint8_t><<<blocks, 256, 0, st>>>(static_cast<const uint8_t*>(img), v, N, H, W, dw, 1, 9);
+    conv_c1_wgrad_kernel<uint8_t><<<blocks, 256, 0, st>>>(static_cast<const uint8_t*>(img), v, N, H, W, dw, 1, 9, nullptr);
   else
-    conv_c1_wgrad_kernel<float><<<blocks, 256, 0, st>>>(static_cast<const float*>(img), v, N, H, W, dw, 1, 9);
+    conv_c1_wgrad_kernel<float><<<blocks, 256, 0, st>>>(static_cast<const float*>(img), v, N, H, W, dw, 1, 9, nullptr);
   return launch_check("conv_c1_wgrad_kernel");
 }
 
-// Weight gradient of the general stem (abc_conv3x3_cn): dw fp32 [16][cin][9], one pass over dz per input channel.
-extern "C" int abc_conv3x3_cn_wgrad(const float* img, int cin, const void* dz, int dz_planes, int dz_plane_off, int N, int H, int W,
+extern "C" int abc_conv3x3_c1_wgrad(const void* img, int img_is_u8, const void* dz, int dz_planes, int dz_plane_off, int N, int H, int W,
                                     float* dw, void* stream) {
+  return c1_wgrad_launch(img, img_is_u8, dz, dz_planes, dz_plane_off, N, H, W, dw, nullptr, stream);
+}
+
+extern "C" int abc_conv3x3_c1_wgrad_det(const void* img, int img_is_u8, const void* dz, int dz_planes, int dz_plane_off, int N, int H,
+                                        int W, float* dw, float* ws, void* stream) {
+  ABC_REQUIRE(ws != nullptr, "abc_conv3x3_c1_wgrad_det: null workspace");
+  return c1_wgrad_launch(img, img_is_u8, dz, dz_planes, dz_plane_off, N, H, W, dw, ws, stream);
+}
+
+// Weight gradient of the general stem (abc_conv3x3_cn): dw fp32 [16][cin][9], one pass over dz per input channel.
+static int cn_wgrad_launch(const float* img, int cin, const void* dz, int dz_planes, int dz_plane_off, int N, int H, int W,
+                           float* dw, float* ws, void* stream) {
   if (int rc = device_check()) return rc;
   ABC_REQUIRE(img && dw && N > 0 && H > 0 && W > 0 && cin >= 1 && cin <= 8, "abc_conv3x3_cn_wgrad: bad arguments");
   if (int rc = p8_check(dz, dz_planes, dz_plane_off, 2, "abc_conv3x3_cn_wgrad(dz)")) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  ABC_CUDA(cudaMemsetAsync(dw, 0, static_cast<size_t>(144) * cin * sizeof(float), st));
+  if (!ws) ABC_CUDA(cudaMemsetAsync(dw, 0, static_cast<size_t>(144) * cin * sizeof(float), st));
   P8View v{static_cast<const uint4*>(dz), dz_planes, dz_plane_off};
   for (int ci = 0; ci < cin; ++ci) {
-    conv_c1_wgrad_kernel<float><<<148 * 4, 256, 0, st>>>(img + static_cast<size_t>(ci) * H * W, v, N, H, W, dw + ci * 9, cin, cin * 9);
+    const float* x = img + static_cast<size_t>(ci) * H * W;
+    if (ws) conv_c1_wgrad_kernel<float, true><<<kC1WgradBlocksDense, 256, 0, st>>>(x, v, N, H, W, dw + ci * 9, cin, cin * 9, ws + ci * 9);
+    else conv_c1_wgrad_kernel<float><<<kC1WgradBlocksDense, 256, 0, st>>>(x, v, N, H, W, dw + ci * 9, cin, cin * 9, nullptr);
     if (int rc = launch_check("conv_c1_wgrad_kernel")) return rc;
   }
-  return ABC_OK;
+  return ws ? det_reduce(ws, kC1WgradBlocksDense, 144 * cin, det_out1(dw, 144 * cin), 0, st) : ABC_OK;
+}
+
+extern "C" int abc_conv3x3_cn_wgrad(const float* img, int cin, const void* dz, int dz_planes, int dz_plane_off, int N, int H, int W,
+                                    float* dw, void* stream) {
+  return cn_wgrad_launch(img, cin, dz, dz_planes, dz_plane_off, N, H, W, dw, nullptr, stream);
+}
+
+extern "C" int abc_conv3x3_cn_wgrad_det(const float* img, int cin, const void* dz, int dz_planes, int dz_plane_off, int N, int H, int W,
+                                        float* dw, float* ws, void* stream) {
+  ABC_REQUIRE(ws != nullptr, "abc_conv3x3_cn_wgrad_det: null workspace");
+  return cn_wgrad_launch(img, cin, dz, dz_planes, dz_plane_off, N, H, W, dw, ws, stream);
+}
+
+// Workspace of abc_conv3x3_c1_wgrad_det (cin = 1, either kernel) and abc_conv3x3_cn_wgrad_det.
+extern "C" size_t abc_conv3x3_wgrad_workspace_bytes(int cin) {
+  if (cin < 1) return 0;
+  const size_t dense = det_ws_bytes(kC1WgradBlocksDense, 144ll * cin, sizeof(float));
+  const size_t sparse = det_ws_bytes(kC1WgradBlocksSparse, 144, sizeof(float));
+  return dense > sparse ? dense : sparse;
 }
 
 extern "C" int abc_deinterleave2(const void* src, int src_planes, int src_plane_off, int C, void* dst, int N, int H, int W, void* stream) {

@@ -10,11 +10,13 @@
 //
 // Each CTA owns one (co tile, ci tile, tap group) and a strided subset of the pixel tiles; it accumulates
 // taps_per_cta x [128 x n_tile] fp32 blocks in TMEM (taps_per_cta * n_tile <= 512 columns) over all its tiles and adds
-// them to the global fp32 gradient with atomicAdd at the end (split-K over CTAs).
+// them to the global fp32 gradient with atomicAdd at the end (split-K over CTAs). The deterministic variant (DET) stores the
+// block to the CTA's split-K slot of a workspace instead, and det_reduce adds the slots to the gradient in slot order.
 #include <cuda.h>
 #include <cuda_bf16.h>
 
 #include "common.cuh"
+#include "det_slots.cuh"
 #include "ptx_sm100.cuh"
 
 namespace abc {
@@ -42,8 +44,10 @@ struct WgradParams {
   int tap_dy[9], tap_dx[9];
   int tap_col[9];          // row-box mode: accumulator column block of tap t = (dx + 1) * 3 + (dy + 1)
   float* dw;               // [ntaps][cout][cin] fp32, accumulated with atomicAdd
+  float* ws;               // DET: [gridDim.x][ntaps][cout][cin] fp32 split-K slots (det_slots.cuh)
 };
 
+template <bool DET = false>
 __global__ void __launch_bounds__(kWgThreads, 1)
 wgrad_kernel(const __grid_constant__ CUtensorMap tmap_dz, const __grid_constant__ CUtensorMap tmap_in, const WgradParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -177,7 +181,8 @@ wgrad_kernel(const __grid_constant__ CUtensorMap tmap_dz, const __grid_constant_
     mbar_wait(bar_done, 0);
     tc_fence_after();
     for (int t = 0; t < ntap; ++t) {
-      float* dst = p.dw + (static_cast<size_t>(tap0 + t) * p.cout + co) * p.cin + ci_t * p.n_tile;
+      const size_t off = (static_cast<size_t>(tap0 + t) * p.cout + co) * p.cin + ci_t * p.n_tile;
+      float* dst = DET ? p.ws + det_slot_index(blockIdx.x, p.ntaps * p.cout * p.cin, 0) + off : p.dw + off;
       const uint32_t taddr = tmem_base + (p.fold == 2 ? p.tap_col[tap0 + t] : t) * p.n_tile + (static_cast<uint32_t>(q * 32) << 16);
       for (int c0 = 0; c0 < p.n_tile; c0 += 16) {
         uint32_t raw[16];
@@ -186,7 +191,10 @@ wgrad_kernel(const __grid_constant__ CUtensorMap tmap_dz, const __grid_constant_
         if (co < p.cout) {
 #pragma unroll
           for (int i = 0; i < 16; ++i)
-            if (ci_t * p.n_tile + c0 + i < p.cin) atomicAdd(dst + c0 + i, __uint_as_float(raw[i]));
+            if (ci_t * p.n_tile + c0 + i < p.cin) {
+              if constexpr (DET) dst[c0 + i] = __uint_as_float(raw[i]);
+              else atomicAdd(dst + c0 + i, __uint_as_float(raw[i]));
+            }
         }
       }
     }
@@ -227,11 +235,8 @@ static int make_map(CUtensorMap* m, const void* base, int W, int H, int planes, 
   return ABC_OK;
 }
 
-}  // namespace abc
-
-extern "C" int abc_conv_wgrad(const AbcWgradDesc* d, void* stream) {
-  using namespace abc;
-  if (int rc = device_check()) return rc;
+// Launch parameters of abc_conv_wgrad (everything but the tensor maps): grid, shared memory, kernel parameters.
+static int wgrad_setup(const AbcWgradDesc* d, WgradParams& p, dim3& grid, uint32_t& smem_launch) {
   ABC_REQUIRE(d && d->dz && d->in && d->dw, "abc_conv_wgrad: null argument");
   ABC_REQUIRE(d->N > 0 && d->H > 0 && d->W > 0, "abc_conv_wgrad: bad geometry");
   ABC_REQUIRE(d->cout >= 8 && d->cout % 8 == 0 && d->cin >= 16 && d->cin % 16 == 0, "abc_conv_wgrad: cout %% 8, cin %% 16 (cout=%d cin=%d)",
@@ -244,7 +249,7 @@ extern "C" int abc_conv_wgrad(const AbcWgradDesc* d, void* stream) {
     ABC_REQUIRE(d->tap_dy[t] >= -1 && d->tap_dy[t] <= 1 && d->tap_dx[t] >= -1 && d->tap_dx[t] <= 1, "abc_conv_wgrad: tap offset");
     if (d->tap_dy[t] || d->tap_dx[t]) halo = 1;
   }
-  WgradParams p{};
+  p = WgradParams{};
   p.N = d->N; p.H = d->H; p.W = d->W;
   p.tiles_x = (d->W + 7) / 8; p.tiles_y = (d->H + 15) / 16;
   const int64_t tiles = static_cast<int64_t>(d->N) * p.tiles_x * p.tiles_y;
@@ -308,20 +313,48 @@ extern "C" int abc_conv_wgrad(const AbcWgradDesc* d, void* stream) {
   if (p.stages > kWgStages) p.stages = kWgStages;
   ABC_REQUIRE(p.stages >= 2, "abc_conv_wgrad: shared memory budget exceeded");
   const uint32_t smem_bytes = kWgHeader + p.stages * p.a_stage_bytes;
+  const int gy = p.n_co_tiles * p.n_ci_tiles * p.tap_groups;
+  grid = dim3(wgrad_grid_x(sm_count(), gy, p.num_tiles), gy);
+  smem_launch = smem_bytes < 120 * 1024 ? 120 * 1024 : smem_bytes;   // 1 CTA / SM (owns all TMEM columns)
+  return ABC_OK;
+}
 
+}  // namespace abc
+
+extern "C" int abc_conv_wgrad(const AbcWgradDesc* d, void* stream) {
+  using namespace abc;
+  if (int rc = device_check()) return rc;
+  WgradParams p;
+  dim3 grid;
+  uint32_t smem_launch;
+  if (int rc = wgrad_setup(d, p, grid, smem_launch)) return rc;
+  const int rows = 16 + 2 * p.halo, cols = 8 + 2 * p.halo;
   CUtensorMap map_dz, map_in;
   if (int rc = make_map(&map_dz, d->dz, d->W, d->H, d->dz_planes, d->N, 8, 16, p.m_planes)) return rc;
   if (int rc = make_map(&map_in, d->in, d->W, d->H, d->in_planes, d->N, p.fold == 2 ? 10 : (p.fold ? 8 : cols), p.fold ? 16 : rows, p.n_tile / 8))
     return rc;
   static PerDeviceOnce attr_once;
-  ABC_CUDA(attr_once.run([] { return cudaFuncSetAttribute(wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448); }));
-  const int gy = p.n_co_tiles * p.n_ci_tiles * p.tap_groups;
-  int sms = sm_count();
-  if (sms <= 0) sms = 148;
-  int gx = sms / gy;
-  if (gx < 1) gx = 1;
-  if (gx > p.num_tiles) gx = p.num_tiles;
-  const uint32_t smem_launch = smem_bytes < 120 * 1024 ? 120 * 1024 : smem_bytes;   // 1 CTA / SM (owns all TMEM columns)
-  wgrad_kernel<<<dim3(gx, gy), kWgThreads, smem_launch, static_cast<cudaStream_t>(stream)>>>(map_dz, map_in, p);
+  ABC_CUDA(attr_once.run([] {
+    if (cudaError_t e = cudaFuncSetAttribute(wgrad_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448)) return e;
+    return cudaFuncSetAttribute(wgrad_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
+  }));
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (d->ws) {        // deterministic: every CTA stores its block to slot blockIdx.x, then dw += the slots in slot order
+    p.ws = d->ws;
+    wgrad_kernel<true><<<grid, kWgThreads, smem_launch, st>>>(map_dz, map_in, p);
+    if (int rc = launch_check("wgrad_kernel")) return rc;
+    const int n = d->ntaps * d->cout * d->cin;
+    return det_reduce(d->ws, static_cast<int>(grid.x), n, det_out1(d->dw, n), 1, st);
+  }
+  wgrad_kernel<false><<<grid, kWgThreads, smem_launch, st>>>(map_dz, map_in, p);
   return launch_check("wgrad_kernel");
+}
+
+extern "C" size_t abc_conv_wgrad_workspace_bytes(const AbcWgradDesc* d) {
+  using namespace abc;
+  WgradParams p;
+  dim3 grid;
+  uint32_t smem_launch;
+  if (wgrad_setup(d, p, grid, smem_launch) != ABC_OK) return 0;
+  return det_ws_bytes(grid.x, static_cast<long long>(d->ntaps) * d->cout * d->cin, sizeof(float));
 }

@@ -39,6 +39,15 @@ def _desc(logits, targets, type_w, sums, scale, dlogits):
     return d
 
 
+def _det_ws(d, p8, dev):
+    """Under torch.use_deterministic_algorithms: a workspace for the fixed-order sums of the loss pass (AbcLossDesc.ws)."""
+    if not torch.are_deterministic_algorithms_enabled():
+        return None
+    ws = torch.empty(lib.abc_loss_workspace_bytes(C.byref(d), p8), dtype=torch.uint8, device=dev)
+    d.ws = ws.data_ptr()
+    return ws
+
+
 _IDX_CACHE = {}
 
 
@@ -79,8 +88,9 @@ def loss_forward_backward(s, type_w, targets, logits, scaled=True):
     dev = logits[0].device
     sums = torch.empty(16, dtype=torch.float64, device=dev)
     dlogits = [torch.empty_like(z) for z in logits]
-    check(lib.abc_loss_partials(C.byref(_desc(logits, targets, type_w, sums, None, None if scaled else dlogits)), st),
-          "abc_loss_partials")
+    d = _desc(logits, targets, type_w, sums, None, None if scaled else dlogits)
+    ws = _det_ws(d, 0, dev)  # noqa: F841  (alive until the call is enqueued)
+    check(lib.abc_loss_partials(C.byref(d), st), "abc_loss_partials")
     total, parts, ds, scale, h2l = _weighting(sums, s, dev)
     head_scale = None
     if scaled:
@@ -145,8 +155,9 @@ def loss_forward_p8(s, type_w, targets, logits, dz_p8, dbias):
             raise ValueError(f"dbias[{i}]: fp64 [{z.shape[1]}] required")
         out.dz[i], out.planes[i], out.dbias[i] = g.data_ptr(), g.shape[1], b.data_ptr()
     sums = torch.empty(16, dtype=torch.float64, device=dev)
-    check(lib.abc_loss_partials_p8(C.byref(_desc(logits, targets, type_w, sums, None, None)), C.byref(out), _lib.current_stream_ptr()),
-          "abc_loss_partials_p8")
+    d = _desc(logits, targets, type_w, sums, None, None)
+    ws = _det_ws(d, 1, dev)  # noqa: F841  (alive until the call is enqueued)
+    check(lib.abc_loss_partials_p8(C.byref(d), C.byref(out), _lib.current_stream_ptr()), "abc_loss_partials_p8")
     total, parts, ds, scale, h2l = _weighting(sums, s, dev)
     return total, parts, ds, scale[h2l]
 

@@ -60,6 +60,12 @@ def _st():
     return _lib.current_stream_ptr()
 
 
+def deterministic():
+    """torch.use_deterministic_algorithms(True) (warn_only too): every reduction of the training step then runs in a fixed
+    order (per-block slots of a workspace summed by one small kernel instead of atomics), read when the work is enqueued."""
+    return torch.are_deterministic_algorithms_enabled()
+
+
 def _n_tile(cout):
     c16 = (cout + 15) // 16 * 16
     if c16 <= 128:
@@ -166,8 +172,9 @@ def can_fuse_stats(pk, dst):
 
 
 def conv(pk, src, in_plane_off, dst, out_plane_off=0, act=0, out_mode=0, out_scale=(1, 0, 1, 0), pool=None, pool_plane_off=0,
-         stats=None):
-    """stats: (sum, sumsq) fp64 [cout] tensors -> fused BatchNorm statistics of the output (AbcConvDesc.stat_sum / stat_sq)."""
+         stats=None, ws=None):
+    """stats: (sum, sumsq) fp64 [cout] tensors -> fused BatchNorm statistics of the output (AbcConvDesc.stat_sum / stat_sq).
+    ws: ``nbytes -> tensor`` (TrainEngine.det_ws): the statistics are summed in a fixed order (AbcConvDesc.stat_ws)."""
     d = AbcConvDesc()
     N, in_planes, H, W, _ = src.shape
     d.in_, d.N, d.H, d.W = src.data_ptr(), N, H, W
@@ -196,12 +203,14 @@ def conv(pk, src, in_plane_off, dst, out_plane_off=0, act=0, out_mode=0, out_sca
         d.pool_out, d.pool_planes, d.pool_plane_off = pool.data_ptr(), pool.shape[1], pool_plane_off
     if stats is not None:
         d.stat_sum, d.stat_sq = stats[0].data_ptr(), stats[1].data_ptr()
+        if ws is not None:
+            d.stat_ws = ws(lib.abc_conv_stat_workspace_bytes(C.byref(d))).data_ptr()
     with _timed(f"conv {pk.cin}->{pk.cout} t{len(pk.taps)} @{H}x{W} nt{pk.n_tile}"):
         check(lib.abc_conv_igemm(C.byref(d), _st()), "abc_conv_igemm")
 
 
-def wgrad(dz, dz_off, cout, a, a_off, cin, taps):
-    """-> fp32 [ntaps, cout, cin]"""
+def wgrad(dz, dz_off, cout, a, a_off, cin, taps, ws=None):
+    """-> fp32 [ntaps, cout, cin]; ws as in conv(): fixed-order split-K sum (AbcWgradDesc.ws)."""
     N, _, H, W, _ = a.shape
     dw = torch.zeros((len(taps), cout, cin), dtype=torch.float32, device=a.device)
     d = AbcWgradDesc()
@@ -212,6 +221,8 @@ def wgrad(dz, dz_off, cout, a, a_off, cin, taps):
         d.tap_dy[i], d.tap_dx[i] = dy, dx
     d.dw = dw.data_ptr()
     d.row_boxes = 1 if os.environ.get("ABCNET_WGRAD_ROWBOX") else 0
+    if ws is not None:
+        d.ws = ws(lib.abc_conv_wgrad_workspace_bytes(C.byref(d))).data_ptr()
     with _timed(f"wgrad {cin}->{cout} t{len(taps)} @{H}x{W}"):
         check(lib.abc_conv_wgrad(C.byref(d), _st()), "abc_conv_wgrad")
     return dw
@@ -224,7 +235,7 @@ def phase_taps(parity, crop_first):
     return [(0, 0), (2, -1)] if parity == 0 else [(1, 0)]
 
 
-def upconv_backward(du, du_off, cout, x, w, crop_first, eng=None, key=None):
+def upconv_backward(du, du_off, cout, x, w, crop_first, eng=None, key=None, ws=None):
     """Backward of the up-sampling convolution. du: P8 gradient of the cropped output (planes [du_off, du_off+cout/8) of a
     [N, planes, 2H, 2W, 8] buffer); x: P8 input [N, cin/8, H, W, 8]; w: [cin, cout, 3, 3] fp32.
     Returns (dx P8 [N, cin/8, H, W, 8], dw fp32 [cin, cout, 3, 3])."""
@@ -247,7 +258,7 @@ def upconv_backward(du, du_off, cout, x, w, crop_first, eng=None, key=None):
                     fwd_taps.append((ky, kx, dy, dx))
             segments.append((t0, len(taps) - t0))
             phase = 2 * py + px
-            g = wgrad(dph, phase * (cout // 8), cout, x, 0, cin, [(dy, dx) for (_, _, dy, dx) in fwd_taps])
+            g = wgrad(dph, phase * (cout // 8), cout, x, 0, cin, [(dy, dx) for (_, _, dy, dx) in fwd_taps], ws=ws)
             for i, (ky, kx, _, _) in enumerate(fwd_taps):
                 dw[:, :, ky, kx] = g[i].t()
     if eng is None:
@@ -318,9 +329,22 @@ class TrainEngine:
     def buf(self, key, shape, dtype=torch.bfloat16, zero=False):
         t = self.bufs.get(key)
         if t is None or tuple(t.shape) != tuple(shape) or t.dtype != dtype:
-            t = (torch.zeros if zero else torch.empty)(shape, dtype=dtype, device=self.m.s.device)
+            # deterministic mode: torch fills torch.empty with NaN there, and a region no kernel writes (padding / halo planes)
+            # would turn into NaN * 0 in the gradients; zeroed once, such regions stay zero
+            t = (torch.zeros if zero or deterministic() else torch.empty)(shape, dtype=dtype, device=self.m.s.device)
             self.bufs[key] = t
         return t
+
+    def det_ws(self, nbytes):
+        """The workspace of the deterministic reductions: one buffer shared by all of them (they run in stream order, each
+        producer followed by its reduction), grown to the largest request -- reached in the warm-up before a graph capture."""
+        t = self.bufs.get("det:ws")
+        if t is None or t.numel() < nbytes:
+            t = self.bufs["det:ws"] = torch.empty(max(int(nbytes), 256), dtype=torch.uint8, device=self.m.s.device)
+        return t
+
+    def _ws(self):
+        return self.det_ws if deterministic() else None
 
     # ------------------------------------------------------------------ layer helpers
     def _stat_bufs(self, key, Cc):
@@ -332,7 +356,11 @@ class TrainEngine:
         dev = z.device
         gamma, beta, rmean, rvar = bn_params
         s, q = self._stat_bufs(key, Cc)
-        if not have_stats:
+        if not have_stats and deterministic():
+            ws = self.det_ws(lib.abc_bn_stats_workspace_bytes(N, H, W, Cc))
+            check(lib.abc_bn_stats_det(z.data_ptr(), N, H, W, z.shape[1], z_off, Cc, s.data_ptr(), q.data_ptr(), ws.data_ptr(), _st()),
+                  "abc_bn_stats_det")
+        elif not have_stats:
             check(lib.abc_bn_stats(z.data_ptr(), N, H, W, z.shape[1], z_off, Cc, s.data_ptr(), q.data_ptr(), _st()), "abc_bn_stats")
         st = [self.buf(key + f".st{i}", (Cc,), torch.float32) for i in range(4)]
         check(lib.abc_bn_finalize(s.data_ptr(), q.data_ptr(), Cc, float(N * H * W), gamma.data_ptr(), beta.data_ptr(), 1e-5, 0.1,
@@ -377,6 +405,8 @@ class TrainEngine:
         d.gscale = gscale.data_ptr() if gscale is not None else None
         if drop_p > 0 and key in self._mask_keys:                      # the keep bits the forward pass of this step stored
             d.drop_mask = self.bufs[key + ".mask"].data_ptr()
+        if deterministic():
+            d.ws = self.det_ws(lib.abc_bn_act_backward_workspace_bytes(C.byref(d))).data_ptr()
         check(lib.abc_bn_act_backward(C.byref(d), _st()), "abc_bn_act_backward")
         return s1, s2
 
@@ -503,7 +533,7 @@ class TrainEngine:
                     return Packed(mats, self._w(cv.bias), TAPS3, fold=js or row_fold_for(cin, cout), fold_swap=bool(js))
                 pk = self._pk(u["name"], make)
                 fused_stats = fuse and can_fuse_stats(pk, z)
-                conv(pk, src, u["src_off"], z, stats=self._stat_bufs("bn:" + u["name"], cout) if fused_stats else None)
+                conv(pk, src, u["src_off"], z, stats=self._stat_bufs("bn:" + u["name"], cout) if fused_stats else None, ws=self._ws())
             dst = self._tensor(u["dst"], B, H, W, (B, cout // 8, h, w, 8)) if u["keep"] or u["dst"][0] == "cat" else None
             pool = self._tensor(u["pool"], B, H, W) if u["pool"] else None
             bn = u["bn"]
@@ -525,7 +555,7 @@ class TrainEngine:
                           n_tile=256 if ((128 * nh) % 256 == 0 and os.environ.get("ABCNET_TRAIN_HEADS_NT256")) else 128)
         pk_h1 = self._pk("heads.conv1", make_h1)
         h1_stats = fuse and can_fuse_stats(pk_h1, zh)
-        conv(pk_h1, trunk, 0, zh, stats=self._stat_bufs("bn:heads", 128 * nh) if h1_stats else None)
+        conv(pk_h1, trunk, 0, zh, stats=self._stat_bufs("bn:heads", 128 * nh) if h1_stats else None, ws=self._ws())
         gam = torch.cat([om.bn.weight.detach() for om in m.out_modules]).float().contiguous()
         bet = torch.cat([om.bn.bias.detach() for om in m.out_modules]).float().contiguous()
         rme = torch.cat([om.bn.running_mean for om in m.out_modules]).float().contiguous()
@@ -572,6 +602,7 @@ class TrainEngine:
         m, sv = self.m, self.saved
         B, H, W = sv["B"], sv["H"], sv["W"]
         H4, W4 = H // 4, W // 4
+        ws = self._ws()
         dev = sv["x"].device
         hd = sv["heads"]
         nh = len(m.heads)
@@ -591,11 +622,16 @@ class TrainEngine:
                     g = torch.zeros((B, h_, H4, W4), dtype=torch.float32, device=dev)
                 g = g.contiguous().float()
                 # one pass: (optional per-head loss scale) * dlogits -> bf16 P8 with zero K padding, + conv2 bias gradient
-                check(lib.abc_nchw_to_p8_ex(g.data_ptr(), dl.data_ptr(), B, h_, H4, W4, c16 // 8,
-                                            head_scale[i:i + 1].data_ptr() if head_scale is not None else None, db.data_ptr(), _st()),
-                      "abc_nchw_to_p8_ex")
+                sc = head_scale[i:i + 1].data_ptr() if head_scale is not None else None
+                if ws is not None:
+                    w_ = ws(lib.abc_nchw_to_p8_ex_workspace_bytes(B, h_, H4, W4, c16 // 8))
+                    check(lib.abc_nchw_to_p8_ex_det(g.data_ptr(), dl.data_ptr(), B, h_, H4, W4, c16 // 8, sc, db.data_ptr(), w_.data_ptr(),
+                                                    _st()), "abc_nchw_to_p8_ex_det")
+                else:
+                    check(lib.abc_nchw_to_p8_ex(g.data_ptr(), dl.data_ptr(), B, h_, H4, W4, c16 // 8, sc, db.data_ptr(), _st()),
+                          "abc_nchw_to_p8_ex")
             c8 = (h_ + 7) // 8 * 8
-            dw2 = wgrad(dl, 0, c8, hd["hid"], 16 * i, 128, [(0, 0)])[0][:h_]
+            dw2 = wgrad(dl, 0, c8, hd["hid"], 16 * i, 128, [(0, 0)], ws=ws)[0][:h_]
             dbf = db.float()
             if p8 is not None:                                    # the factor the loss kernel left out (linear in the gradient)
                 dw2 = dw2 * head_scale[i]
@@ -610,7 +646,7 @@ class TrainEngine:
         dzh = self.buf("g:zheads", (B, 16 * nh, H4, W4, 8))
         gscale = head_scale.float().view(-1, 1).expand(-1, 128).reshape(-1).contiguous() if p8 is not None else None    # per hidden channel
         s1, s2 = self._bn_backward("bn:heads", hd["z"], 128 * nh, hd["st"], 2, dhid, 0, None, dzh, hd["p_drop"], sv["seed"], gscale=gscale)
-        dw1 = wgrad(dzh, 0, 128 * nh, hd["trunk"], 0, 128, TAPS3)            # [9][128*nh][128]
+        dw1 = wgrad(dzh, 0, 128 * nh, hd["trunk"], 0, 128, TAPS3, ws=ws)     # [9][128*nh][128]
         for i, om in enumerate(m.out_modules):
             sl = slice(128 * i, 128 * (i + 1))
             sink(om.conv1.weight, dw1[:, sl].permute(1, 2, 0).reshape(128, 128, 3, 3))
@@ -631,12 +667,17 @@ class TrainEngine:
                 xin = self._tensor(u["src"], B, H, W, (B, u["cin"] // 8, h, w, 8))
                 wt = u["up"].weight.detach().float()
                 dx, dwu = upconv_backward(gcat, u["dst_off"], u["cout"], xin, wt, m.crop_first,
-                                          eng=self if self.arena is not None else None, key=(u["name"] + ".dgrad", u["up"].weight))
+                                          eng=self if self.arena is not None else None, key=(u["name"] + ".dgrad", u["up"].weight), ws=ws)
                 sink(u["up"].weight, dwu)
                 sm = self.buf("up.sum", (u["cout"],), torch.float64)
                 sq = self.buf("up.sq", (u["cout"],), torch.float64)
-                check(lib.abc_channel_sum(gcat.data_ptr(), B, 2 * h, 2 * w, gcat.shape[1], u["dst_off"], u["cout"], sm.data_ptr(),
-                                          sq.data_ptr(), _st()), "abc_channel_sum")
+                if ws is not None:
+                    w_ = ws(lib.abc_bn_stats_workspace_bytes(B, 2 * h, 2 * w, u["cout"]))
+                    check(lib.abc_channel_sum_det(gcat.data_ptr(), B, 2 * h, 2 * w, gcat.shape[1], u["dst_off"], u["cout"], sm.data_ptr(),
+                                                  sq.data_ptr(), w_.data_ptr(), _st()), "abc_channel_sum_det")
+                else:
+                    check(lib.abc_channel_sum(gcat.data_ptr(), B, 2 * h, 2 * w, gcat.shape[1], u["dst_off"], u["cout"], sm.data_ptr(),
+                                              sq.data_ptr(), _st()), "abc_channel_sum")
                 sink(u["up"].bias, sm.float())
                 gsrc = self._tensor(u["src"], B, H, W, (B, u["cin"] // 8, h, w, 8), grad=True)
                 gsrc.copy_(dx)
@@ -654,7 +695,15 @@ class TrainEngine:
             sink(u["conv"].bias, torch.zeros(cout, device=dev))
             if u.get("first"):
                 dwf = torch.zeros(144 * m.n_channels, dtype=torch.float32, device=dev)
-                if m.n_channels == 1:
+                if ws is not None:
+                    w_ = ws(lib.abc_conv3x3_wgrad_workspace_bytes(m.n_channels))
+                    if m.n_channels == 1:
+                        check(lib.abc_conv3x3_c1_wgrad_det(sv["x"].data_ptr(), 1 if sv["u8"] else 0, dz.data_ptr(), 2, 0, B, h, w, dwf.data_ptr(),
+                                                           w_.data_ptr(), _st()), "abc_conv3x3_c1_wgrad_det")
+                    else:
+                        check(lib.abc_conv3x3_cn_wgrad_det(sv["x"].data_ptr(), m.n_channels, dz.data_ptr(), 2, 0, B, h, w, dwf.data_ptr(),
+                                                           w_.data_ptr(), _st()), "abc_conv3x3_cn_wgrad_det")
+                elif m.n_channels == 1:
                     check(lib.abc_conv3x3_c1_wgrad(sv["x"].data_ptr(), 1 if sv["u8"] else 0, dz.data_ptr(), 2, 0, B, h, w, dwf.data_ptr(), _st()),
                           "abc_conv3x3_c1_wgrad")
                 else:
@@ -663,7 +712,7 @@ class TrainEngine:
                 sink(u["conv"].weight, dwf.reshape(16, m.n_channels, 3, 3))
                 continue
             src = self._tensor(u["src"], B, H, W, (B, cin // 8, h, w, 8))
-            dwt = wgrad(dz, 0, cout, src, u["src_off"], cin, TAPS3)               # [9][cout][cin]
+            dwt = wgrad(dz, 0, cout, src, u["src_off"], cin, TAPS3, ws=ws)        # [9][cout][cin]
             sink(u["conv"].weight, dwt.permute(1, 2, 0).reshape(cout, cin, 3, 3))
             gsrc = self._tensor(u["src"], B, H, W, (B, cin // 8, h, w, 8), grad=True)
             def make_d(cv=u["conv"], cin=cin, cout=cout):

@@ -47,6 +47,7 @@ class TrainStep:
         self.loss = torch.zeros((), dtype=torch.float64, device=dev)
         self.parts = torch.zeros(8, dtype=torch.float64, device=dev)
         self._opt_in_graph = optimizer is not None and bool(optimizer.defaults.get("capturable", False))
+        self._det = None                                   # torch.are_deterministic_algorithms_enabled() when the graph was captured
 
     # ------------------------------------------------------------------ the enqueued work
     def _sink(self, p, g):
@@ -90,6 +91,8 @@ class TrainStep:
         if not self.use_graph:
             self._enqueue(x, targets, True)
             return self.loss.clone()
+        if self.graph is not None and self._det != torch.are_deterministic_algorithms_enabled():
+            self.graph = None                              # the other reduction mode is a different set of kernels: re-capture
         if self.graph is not None and (x.shape != self._x.shape or x.dtype != self._x.dtype):
             # e.g. the last, partial batch of a DataLoader without drop_last (the reference's loaders, train.py:43-46): run
             # it eagerly through the same kernels; the graph of the regular batch shape stays valid (its buffers are keyed
@@ -113,6 +116,7 @@ class TrainStep:
         return self.loss.clone()                           # a fresh tensor per step: callers may collect the returned losses
 
     def _capture(self, x, targets):
+        self._det = torch.are_deterministic_algorithms_enabled()
         # static input buffers; the first batch is also used for the warm-up iterations (parameters are restored after)
         self._x = x.clone()
         self._tg = [t.clone() for t in targets]

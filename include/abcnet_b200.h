@@ -20,6 +20,7 @@
 #ifndef ABCNET_B200_H_
 #define ABCNET_B200_H_
 
+#include <stddef.h>
 #include <stdint.h>
 
 #ifdef __cplusplus
@@ -163,9 +164,14 @@ typedef struct AbcConvDesc {
    * "decision-stable" inference mode (UNet(..., act_dtype="fp16")): fewer threshold / NMS / omega ties flip against the fp32
    * reference. Outputs saturate at +-65504. Inference only (no fused statistics, no cta_pair). */
   int act_fp16;
+  /* Optional (NULL = fp64 atomics): workspace of abc_conv_stat_workspace_bytes(desc) bytes for the fused statistics. Each
+   * epilogue owner stores its partial sums to a slot of its own and a second kernel sums the slots in a fixed order, so that
+   * stat_sum / stat_sq are bit-reproducible (torch.use_deterministic_algorithms). */
+  double* stat_ws;
 } AbcConvDesc;
 
 ABC_API int abc_conv_igemm(const AbcConvDesc* desc, void* stream);
+ABC_API size_t abc_conv_stat_workspace_bytes(const AbcConvDesc* desc);
 /* Bytes of packed weights for a layer (host-side helper for allocation). */
 ABC_API int64_t abc_conv_wpack_bytes(int cin, int cout, int ntaps, int n_tile);
 
@@ -331,6 +337,8 @@ typedef struct AbcLossDesc {
   double* sums;             /* [16] device: numerators 0..7, denominators 8..15 (order of AbcLossIndex) */
   const float* scale;       /* [8] device: dL/dnum_k = u_k / denom_k (backward pass only) */
   float* dlogits[8];        /* backward pass only */
+  double* ws;               /* optional (NULL = fp64 atomics): abc_loss_workspace_bytes(desc, p8) bytes; the sums (and, in
+                               abc_loss_partials_p8, the bias gradients) are then added in a fixed order: bit-reproducible */
 } AbcLossDesc;
 enum AbcLossIndex { ABC_L_ATOM = 0, ABC_L_BOND, ABC_L_TYPE, ABC_L_CHARGE, ABC_L_BTYPE, ABC_L_RHO, ABC_L_OMEGA, ABC_L_HS };
 ABC_API int abc_loss_partials(const AbcLossDesc* desc, void* stream);
@@ -348,6 +356,8 @@ typedef struct AbcLossP8Out {
   double* dbias[8];
 } AbcLossP8Out;
 ABC_API int abc_loss_partials_p8(const AbcLossDesc* desc, const AbcLossP8Out* out, void* stream);
+/* Workspace of the deterministic mode of abc_loss_partials (p8 = 0) or abc_loss_partials_p8 (p8 = 1; n_omega <= 64). */
+ABC_API size_t abc_loss_workspace_bytes(const AbcLossDesc* desc, int p8);
 
 /* ---------------------------------------------------------------------------------------------------
  * Training-mode building blocks (autograd of src/unet.py as used by src/train.py:94,139-140).
@@ -391,8 +401,23 @@ typedef struct AbcBnActBwdDesc {
   const float* gscale;                             /* [C] device or NULL: dA is multiplied by gscale[c] first (a per-channel
                                                       factor the producer of dA left out, e.g. the per-loss scale of the heads) */
   const void* drop_mask;                           /* the bytes abc_bn_act stored (AbcBnActDesc.drop_mask) or NULL = regenerate */
+  double* ws;                                      /* optional (NULL = fp64 atomics): abc_bn_act_backward_workspace_bytes(desc)
+                                                      bytes; s1 / s2 are then summed in a fixed order (bit-reproducible) */
 } AbcBnActBwdDesc;
 ABC_API int abc_bn_act_backward(const AbcBnActBwdDesc* desc, void* stream);
+ABC_API size_t abc_bn_act_backward_workspace_bytes(const AbcBnActBwdDesc* desc);
+/* Deterministic forms of abc_bn_stats / abc_channel_sum / abc_nchw_to_p8_ex (torch.use_deterministic_algorithms): the
+ * per-block sums are stored to slots of the caller's workspace `ws` and summed in a fixed order instead of added with fp64
+ * atomics, so the results are bit-reproducible for a given device and shape. ws: the bytes the *_workspace_bytes queries
+ * return. */
+ABC_API int abc_bn_stats_det(const void* z, int N, int H, int W, int planes, int plane_off, int C, double* sum, double* sumsq,
+                             double* ws, void* stream);
+ABC_API int abc_channel_sum_det(const void* x, int N, int H, int W, int planes, int plane_off, int C, double* sum, double* scratch,
+                                double* ws, void* stream);
+ABC_API size_t abc_bn_stats_workspace_bytes(int N, int H, int W, int C);    /* also abc_channel_sum_det */
+ABC_API int abc_nchw_to_p8_ex_det(const float* src, void* dst, int N, int C, int H, int W, int dst_planes, const float* scale,
+                                  double* dbias, double* ws, void* stream);
+ABC_API size_t abc_nchw_to_p8_ex_workspace_bytes(int N, int C, int H, int W, int dst_planes);
 /* fp32 NCHW -> bf16 P8 with zero-padded channels (dlogits -> tensor-core operand). */
 ABC_API int abc_nchw_to_p8(const float* src, void* dst, int N, int C, int H, int W, void* stream);
 /* Same in one pass with: a device-side scalar scale (NULL = 1), dst_planes >= ceil(C/8) planes written (padding planes
@@ -442,7 +467,9 @@ ABC_API int abc_adam_chunk_elems(void);
 ABC_API int abc_adam_step(const void* p_ptrs, const void* g_ptrs, const void* m_ptrs, const void* v_ptrs, const int64_t* sizes,
                           const int32_t* chunks, int n_chunks, const float* hyper, float* step_dev, void* stream);
 /* Weight gradient of a convolution on tcgen05 tensor cores (cuDNN backward-filter of the reference's autograd):
- * dw[tap][co][ci] (fp32, caller-zeroed, accumulated with atomicAdd) = sum_pixels dz[co](y, x) * in[ci](y + dy, x + dx). */
+ * dw[tap][co][ci] (fp32, caller-zeroed, accumulated with atomicAdd) = sum_pixels dz[co](y, x) * in[ci](y + dy, x + dx).
+ * With ws (abc_conv_wgrad_workspace_bytes(desc) bytes) every split-K CTA stores its block to a slot of its own and the
+ * slots are added to dw in slot order: bit-reproducible for a given device and shape. */
 typedef struct AbcWgradDesc {
   const void* dz; int dz_planes, dz_plane_off; int cout;    /* P8 bf16 gradient of the conv output */
   const void* in; int in_planes, in_plane_off; int cin;     /* P8 bf16 conv input */
@@ -452,8 +479,10 @@ typedef struct AbcWgradDesc {
   int row_boxes;   /* 0 (default) / 1: tap-folded launches (cin <= 32, the plain 3x3 tap set) load three row-shifted 16 x 10 boxes and
                       take the dx taps as operand start offsets instead of loading nine shifted 16 x 8 boxes: half the L2 ->
                       shared-memory traffic, three MMAs per K step instead of one; same result, measured equally fast */
+  float* ws;       /* optional, NULL = atomics: deterministic split-K workspace */
 } AbcWgradDesc;
 ABC_API int abc_conv_wgrad(const AbcWgradDesc* desc, void* stream);
+ABC_API size_t abc_conv_wgrad_workspace_bytes(const AbcWgradDesc* desc);
 /* First convolution without folded BN / activation (training mode): z = conv(img) + b. */
 ABC_API int abc_conv3x3_c1_raw(const void* img, int img_is_u8, const float* w, const float* b, void* out, int N, int H, int W,
                                int out_planes, int out_plane_off, void* stream);
@@ -463,6 +492,13 @@ ABC_API int abc_conv3x3_c1_wgrad(const void* img, int img_is_u8, const void* dz,
 /* Same for the general stem: dw fp32 [16][cin][9] (zeroed by the call). */
 ABC_API int abc_conv3x3_cn_wgrad(const float* img, int cin, const void* dz, int dz_planes, int dz_plane_off, int N, int H, int W,
                                  float* dw, void* stream);
+/* Deterministic forms of the two (per-block slots of ws, summed in block order; dw is written, not accumulated) and their
+ * workspace (cin = 1 for abc_conv3x3_c1_wgrad_det). */
+ABC_API int abc_conv3x3_c1_wgrad_det(const void* img, int img_is_u8, const void* dz, int dz_planes, int dz_plane_off, int N, int H,
+                                     int W, float* dw, float* ws, void* stream);
+ABC_API int abc_conv3x3_cn_wgrad_det(const float* img, int cin, const void* dz, int dz_planes, int dz_plane_off, int N, int H, int W,
+                                     float* dw, float* ws, void* stream);
+ABC_API size_t abc_conv3x3_wgrad_workspace_bytes(int cin);
 
 /* ---------------------------------------------------------------------------------------------------
  * Whole-network inference (SURVEY.md section 8b: abc_unet_forward_infer) -- UNet.forward of src/unet.py:100-119 in eval mode
